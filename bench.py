@@ -281,6 +281,15 @@ def library_bar(dev, frames):
 
 
 # ----------------------------------------------------------------------------------------------
+def dump_outputs(directory, arrays):
+    """--dump-outputs: every array as <directory>/<name>.npy in float32, so that two builds can be compared
+    output for output (the inputs and weights are seeded: the same arguments give the same inputs)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def _timed(fn, steps, warmup, world, dist, dev, local, after=None):
     """warm-up, barrier, CUDA-event timing of `steps` calls (+ `after()` once, inside the timed region),
     max over ranks -> (total ms, clocks)."""
@@ -624,6 +633,9 @@ def run_infer(args, dev, world, rank, local, dist):
     total_ms, clocks = _timed(step, K, args.warmup, world, dist, dev, local, after=final_gather)
     ms_per_step = total_ms / K
     value = world * frames * K / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # the later measurements below reuse `outs`: the last timed step's logits are written now
+        dump_outputs(args.dump_outputs, {"logits": outs[K - 1].view(WINDOWS, LENGTH, 7)})
 
     # ---- the gathered logits are what the other rank computed: rank 0 recomputes rank 1's last step
     gather_verified = None
@@ -775,7 +787,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-library-bar", action="store_true")
     ap.add_argument("--no-sub-records", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the per-frame logits of the last timed step (rank 0, "
+                         f"{WINDOWS} x {LENGTH} x 7) as DIR/logits.npy (float32); --workload infer only")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "infer"):
+        ap.error("--dump-outputs is implemented for --impl b200 --workload infer")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
