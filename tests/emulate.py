@@ -10,13 +10,65 @@ import torch.nn.functional as F
 
 
 def _r(x, on):
-    return x.to(torch.bfloat16).float() if on else x
+    return x.to(torch.bfloat16).to(x.dtype) if on else x
 
 
 def border_class_map(H, W):
     r = torch.ones(H, dtype=torch.long); r[0] = 0; r[-1] = 2
     c = torch.ones(W, dtype=torch.long); c[0] = 0; c[-1] = 2
     return r.view(-1, 1) * 3 + c.view(1, -1)          # [H, W]
+
+
+def ir50_unit(u, h, round_t=True, envelope=False):
+    """One IR-50 residual unit from its packed weights, computed in h's dtype and on h's device.
+
+    h: the unit's input [N, cin, H, W] (NCHW; bf16 values as the previous unit stored them).  Returns (y, E):
+    y is the unit's output before its final bf16 rounding.  conv1's output t is rounded to bf16 where the
+    kernels round it (round_t).  E (envelope=True) is a rounding-ambiguity envelope: conv2(A, |w2|) with
+    A = |bf16(prelu(z + d)) - bf16(prelu(z - d))|, d = 2^-14 |z| + 1e-6 rms(z), z = conv1's pre-activation.
+    It bounds how far a correct kernel's output can move because its fp32 z (summed in another order)
+    rounds t to the other neighbouring bf16 value.  E is None without envelope."""
+    cin, depth, stride = u["cin"], u["depth"], u["stride"]
+    w1 = u["w1"].to(h.dtype).view(depth, 3, 3, cin).permute(0, 3, 1, 2)
+    cls = border_class_map(h.shape[2], h.shape[3]).to(h.device)
+    z = F.conv2d(h, w1, None, 1, 1) + u["bias1"].to(h.dtype)[cls].permute(2, 0, 1).unsqueeze(0)   # [9,depth] by class
+    al = u["alpha"].to(h.dtype).view(1, -1, 1, 1)
+
+    def prelu(v):
+        return torch.where(v >= 0, v, v * al)
+
+    t = _r(prelu(z), round_t)
+    w2 = u["w2"].to(h.dtype)
+    w2m = w2[:, :9 * depth].view(depth, 3, 3, depth).permute(0, 3, 1, 2)
+    y = F.conv2d(t, w2m, None, stride, 1)
+    if u["has_proj"]:
+        y = y + F.conv2d(h, w2[:, 9 * depth:].view(depth, cin, 1, 1), None, stride)
+    else:
+        y = y + h
+    y = y + u["bias2"].to(h.dtype).view(1, -1, 1, 1)
+    E = None
+    if envelope:
+        d = 2.0 ** -14 * z.abs() + 1e-6 * z.pow(2).mean().sqrt()
+        A = (_r(prelu(z + d), True) - _r(prelu(z - d), True)).abs()
+        E = F.conv2d(A, w2m.abs(), None, stride, 1)
+    return y, E
+
+
+# Per-element acceptance bound of a bf16 kernel output against a high-precision reference of the same op:
+#   |got - ref| <= (1 + BF16_SLACK) 2^-8 |ref| + E + C_RMS rms(ref)
+# 2^-8 |ref| is the round-to-nearest step to bf16 (pack_bf16x2); E covers intermediate roundings (ir50_unit),
+# C_RMS rms(ref) the fp32 accumulation of a different summation order.
+C_RMS = 1e-4
+BF16_SLACK = 2.0 ** -5
+
+
+def bound_ratio(got, ref, E=None, c=C_RMS):
+    """Elementwise |got - ref| / bound (<= 1 passes), computed in ref's dtype; a NaN in got counts as inf."""
+    got = got.to(ref.dtype)
+    bound = (1 + BF16_SLACK) * 2.0 ** -8 * ref.abs() + c * ref.pow(2).mean().sqrt()
+    if E is not None:
+        bound = bound + E
+    return torch.nan_to_num((got - ref).abs() / bound, nan=float("inf"))
 
 
 def ir50_packed(pk, x, round_act=True, upto=None):
@@ -28,21 +80,8 @@ def ir50_packed(pk, x, round_act=True, upto=None):
     h = _r(torch.where(h >= 0, h, h * a), round_act)
     taps = {-1: h.permute(0, 2, 3, 1).contiguous()}
     for i, u in enumerate(pk["units"]):
-        cin, depth, stride = u["cin"], u["depth"], u["stride"]
-        w1 = u["w1"].float().view(depth, 3, 3, cin).permute(0, 3, 1, 2)
-        t = F.conv2d(h, w1, None, 1, 1)
-        cls = border_class_map(h.shape[2], h.shape[3])
-        t = t + u["bias1"][cls].permute(2, 0, 1).unsqueeze(0)        # [9,depth] indexed by class map
-        al = u["alpha"].view(1, -1, 1, 1)
-        t = _r(torch.where(t >= 0, t, t * al), round_act)
-        w2 = u["w2"].float()
-        w2m = w2[:, :9 * depth].view(depth, 3, 3, depth).permute(0, 3, 1, 2)
-        y = F.conv2d(t, w2m, None, stride, 1)
-        if u["has_proj"]:
-            y = y + F.conv2d(h, w2[:, 9 * depth:].view(depth, cin, 1, 1), None, stride)
-        else:
-            y = y + h
-        h = _r(y + u["bias2"].view(1, -1, 1, 1), round_act)
+        y, _ = ir50_unit(u, h, round_t=round_act)
+        h = _r(y, round_act)
         taps[i] = h.permute(0, 2, 3, 1).contiguous()
         if upto is not None and i == upto:
             return None, taps

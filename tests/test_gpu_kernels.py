@@ -1,9 +1,10 @@
 """GPU parity tests, kernel by kernel, through the C-ABI (libcer_b200.so).
 
-Each CUDA kernel is compared with a plain fp32 PyTorch computation of the same op on the CPU
-(F.conv2d etc. on the bf16-rounded operands the kernel sees), so a failure points at one kernel.
-Tolerances: bf16 outputs -> error relative to the tensor's max <= 1e-2 (one bf16 ulp is 2^-8 of
-the value); fp32 head kernels -> 1e-4 absolute.
+Each CUDA kernel is compared with a plain PyTorch computation of the same op (F.conv2d etc. on the
+bf16-rounded operands the kernel sees), so a failure points at one kernel.  Single convolutions: fp64
+reference on the device, the kernel instantiation that ran pinned by name (cer_conv_last_variant), and
+the per-element bound of tests/emulate.py (bound_ratio: one bf16 rounding plus 1e-4 of the rms) for bf16
+outputs, 1e-4 of the rms for fp32 outputs.  Other kernels: fp32 references, 1e-4 absolute for fp32 heads.
 """
 import numpy as np
 import pytest
@@ -29,75 +30,107 @@ def _rel_err(a, b):
     return ((a - b).abs().max() / b.abs().max().clamp_min(1e-6)).item()
 
 
-def _conv_case(dev, n, H, cin, cout, ksize, stride, classes, prelu, residual, fp32, seed, n_alloc=None):
+def _conv_case(dev, n, H, W, cin, cout, ksize, stride, classes, prelu, residual, fp32, seed, n_alloc=None):
+    """Runs one conv through cer_conv_forward -> (output, fp64 reference NHWC, name of the kernel that ran)."""
+    from feature_vs_text_compound_emotion_b200 import _capi
     from feature_vs_text_compound_emotion_b200.engine import conv_forward
     g = torch.Generator().manual_seed(seed)
     pad = 1 if ksize == 3 else 0
     n_alloc = n_alloc or n
-    x = torch.randn(n_alloc, H, H, cin, generator=g).to(torch.bfloat16)
-    w = (torch.randn(cout, ksize, ksize, cin, generator=g) * (ksize * ksize * cin) ** -0.5).to(torch.bfloat16)
-    bias = 0.5 * torch.randn(classes, cout, generator=g)
-    alpha = (0.25 + 0.1 * torch.randn(cout, generator=g)) if prelu else None
-    Ho = (H + 2 * pad - ksize) // stride + 1
-    res = torch.randn(n, Ho, Ho, cout, generator=g).to(torch.bfloat16) if residual else None
-    # fp32 reference on the same bf16-rounded operands
-    y = F.conv2d(x[:n].float().permute(0, 3, 1, 2), w.float().permute(0, 3, 1, 2), None, stride, pad)
+    x = torch.randn(n_alloc, H, W, cin, generator=g).to(torch.bfloat16).to(dev)
+    w = (torch.randn(cout, ksize, ksize, cin, generator=g) * (ksize * ksize * cin) ** -0.5).to(torch.bfloat16).to(dev)
+    bias = (0.5 * torch.randn(classes, cout, generator=g)).to(dev)
+    alpha = (0.25 + 0.1 * torch.randn(cout, generator=g)).to(dev) if prelu else None
+    Ho, Wo = (H + 2 * pad - ksize) // stride + 1, (W + 2 * pad - ksize) // stride + 1
+    res = torch.randn(n, Ho, Wo, cout, generator=g).to(torch.bfloat16).to(dev) if residual else None
+    # fp64 reference on the same bf16-rounded operands
+    y = F.conv2d(x[:n].double().permute(0, 3, 1, 2), w.double().permute(0, 3, 1, 2), None, stride, pad)
     if classes == 9:
-        y = y + bias[emulate.border_class_map(Ho, Ho)].permute(2, 0, 1).unsqueeze(0)
+        y = y + bias.double()[emulate.border_class_map(Ho, Wo).to(dev)].permute(2, 0, 1).unsqueeze(0)
     else:
-        y = y + bias.view(1, -1, 1, 1)
+        y = y + bias.double().view(1, -1, 1, 1)
     if prelu:
-        y = torch.where(y >= 0, y, y * alpha.view(1, -1, 1, 1))
+        y = torch.where(y >= 0, y, y * alpha.double().view(1, -1, 1, 1))
     y = y.permute(0, 2, 3, 1)
     if residual:
-        y = y + res.float()
-    out = conv_forward(x.to(dev), w.reshape(cout, -1).to(dev), bias.to(dev), ksize, stride, pad,
-                       alpha=None if alpha is None else alpha.to(dev), res=None if res is None else res.to(dev),
-                       out_fp32=fp32, n_frames=n)
+        y = y + res.double()
+    out = conv_forward(x, w.reshape(cout, -1), bias, ksize, stride, pad, alpha=alpha, res=res, out_fp32=fp32, n_frames=n)
     torch.cuda.synchronize()
-    return _rel_err(out, y), out, y
+    return out, y, _capi.lib().cer_conv_last_variant().decode()
 
 
-# (n, H, cin, cout, ksize, stride, classes, prelu, residual, fp32)
+def _assert_conv_within_bound(out, ref, fp32):
+    if fp32:
+        err = (out.double() - ref).abs().max().item()
+        assert err <= emulate.C_RMS * ref.pow(2).mean().sqrt().item(), f"max abs error {err}"
+    else:
+        worst = emulate.bound_ratio(out, ref).max().item()
+        assert worst <= 1.0, f"worst ratio to the bound {worst}"
+
+
+# (n, H, W, cin, cout, ksize, stride, classes, prelu, residual, fp32, kernel instantiation it selects)
 CONV_CASES = [
-    (3, 10, 256, 256, 3, 1, 9, True, False, False),     # stage-3 conv1 (the 50.7% class), ragged M = 300
-    (3, 10, 256, 256, 3, 1, 1, False, True, False),     # stage-3 conv2 + residual
-    (2, 40, 64, 64, 3, 1, 9, True, False, False),       # stage-1 conv1, BN = 64
-    (2, 40, 64, 128, 3, 1, 9, True, False, False),      # widening conv1
-    (2, 40, 128, 128, 3, 2, 1, False, False, False),    # stride-2 conv2
-    (5, 20, 128, 128, 3, 1, 1, False, True, False),     # stage 2
-    (7, 5, 512, 512, 3, 1, 9, True, False, False),      # stage 4: 25 px/frame, tiles span frames, 2 n-tiles
-    (4, 10, 256, 512, 3, 1, 9, True, False, False),     # widening to 512
-    (4, 10, 512, 512, 3, 2, 1, False, False, False),    # stride-2 at 10x10 -> 5x5
-    (3, 40, 64, 128, 1, 2, 1, False, False, False),     # 1x1 stride-2 projection alone
-    (130, 1, 12800, 512, 1, 1, 1, False, False, True),  # the FC head as a 1x1 conv, fp32 out, 2 m-tiles
-    (1, 5, 512, 512, 3, 1, 9, True, True, False),       # a single frame (tiny tensor: driver-quirk path)
-    (48, 40, 64, 64, 3, 1, 9, True, False, False),      # 600 tiles >= 4 waves: weights-resident variant, BN = 64
-    (48, 40, 64, 64, 3, 1, 1, False, True, False),      # same with residual epilogue
-    (48, 40, 64, 128, 3, 1, 9, True, False, False),     # weights-resident variant, BN = 128
-    (49, 40, 64, 64, 3, 1, 9, True, False, False),      # strip kernel, odd frame count: the last tile is half empty
-    (49, 40, 64, 64, 3, 1, 1, False, True, False),      # same with residual
-    (21, 56, 64, 64, 3, 1, 9, True, False, False),      # strip kernel on a 56-row map: tiles cross strips and frames mid-tile
-    (800, 10, 256, 256, 3, 1, 9, True, False, False),   # 625 tiles (odd): CTA-pair (cta_group::2) variant, ragged last pair
-    (800, 10, 256, 256, 3, 1, 1, False, True, False),   # CTA-pair variant with residual epilogue
-    (200, 20, 128, 128, 3, 1, 9, True, False, False),   # CTA-pair variant, BN = 128
-    (1530, 5, 512, 512, 3, 1, 9, True, False, False),   # CTA-pair variant, two n-tiles, tiles span frames
+    (3, 10, 10, 256, 256, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,1>"),     # stage-3 conv1, ragged M = 300
+    (3, 10, 10, 256, 256, 3, 1, 1, False, True, False, "conv_igemm_kernel<64,8,0,0>"),      # stage-3 conv2 + residual, BN narrowed
+    (2, 40, 40, 64, 64, 3, 1, 9, True, False, False, "conv_igemm_kernel<64,8,0,0>"),        # stage-1 conv1, too few tiles for halo
+    (2, 40, 40, 64, 128, 3, 1, 9, True, False, False, "conv_igemm_kernel<128,6,0,0>"),      # widening conv1
+    (2, 40, 40, 128, 128, 3, 2, 1, False, False, False, "conv_igemm_kernel<64,8,0,0>"),     # stride-2 conv2
+    (5, 20, 20, 128, 128, 3, 1, 1, False, True, False, "conv_igemm_kernel<64,8,0,0>"),      # stage 2
+    (7, 5, 5, 512, 512, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,1>"),       # stage 4: 25 px/frame, tiles span frames, 2 n-tiles
+    (4, 10, 10, 256, 512, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,1>"),     # widening to 512
+    (4, 10, 10, 512, 512, 3, 2, 1, False, False, False, "conv_igemm_kernel<128,6,0,1>"),    # stride-2 at 10x10 -> 5x5
+    (3, 40, 40, 64, 128, 1, 2, 1, False, False, False, "conv_igemm_kernel<64,8,0,0>"),      # 1x1 stride-2 projection alone
+    (130, 1, 1, 12800, 512, 1, 1, 1, False, False, True, "conv_igemm_kernel<128,6,0,0>"),   # the FC head as a 1x1 conv, fp32 out, 2 m-tiles
+    (1, 5, 5, 512, 512, 3, 1, 9, True, True, False, "conv_igemm_kernel<256,4,0,1>"),        # a single frame (tiny tensor: driver-quirk path)
+    (48, 40, 40, 64, 64, 3, 1, 9, True, False, False, "conv_strip_kernel"),                 # 600 tiles >= 2 waves
+    (48, 40, 40, 64, 64, 3, 1, 1, False, True, False, "conv_strip_kernel"),                 # same with residual epilogue
+    (48, 40, 40, 64, 128, 3, 1, 9, True, False, False, "conv_halo_kernel<128>"),            # Cout = 128
+    (49, 40, 40, 64, 64, 3, 1, 9, True, False, False, "conv_strip_kernel"),                 # odd frame count: the last tile is half empty
+    (49, 40, 40, 64, 64, 3, 1, 1, False, True, False, "conv_strip_kernel"),                 # same with residual
+    (21, 56, 56, 64, 64, 3, 1, 9, True, False, False, "conv_strip_kernel"),                 # 56-row map: tiles cross strips and frames mid-tile
+    (800, 10, 10, 256, 256, 3, 1, 9, True, False, False, "conv_igemm2_kernel<256,6>"),      # 625 tiles (odd): ragged last CTA pair
+    (800, 10, 10, 256, 256, 3, 1, 1, False, True, False, "conv_igemm2_kernel<256,6>"),      # CTA pair with residual epilogue
+    (200, 20, 20, 128, 128, 3, 1, 9, True, False, False, "conv_igemm2_bres_kernel<128,4,18>"),  # CTA pair, weights resident
+    (1530, 5, 5, 512, 512, 3, 1, 9, True, False, False, "conv_igemm2_kernel<256,6>"),       # CTA pair, two n-tiles, tiles span frames
+    (198, 12, 16, 64, 64, 3, 1, 9, True, False, False, "conv_halo_kernel<64>"),             # H % 8 != 0: no strip; ragged 16-row band
+    (190, 20, 20, 64, 64, 3, 1, 9, True, False, False, "conv_igemm_kernel<64,9,1,1>"),      # W % 8 != 0: no halo; weights resident
+    (190, 20, 20, 64, 128, 3, 1, 9, True, False, False, "conv_igemm_kernel<128,4,1,0>"),    # same, Cout = 128
+    (95, 10, 10, 64, 256, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,0>"),     # 9 k-steps: not a multiple of 4
+    (3, 5, 5, 512, 64, 3, 1, 9, True, False, False, "conv_igemm_kernel<64,8,0,1>"),         # 72 k-steps, BN = 64
+    (758, 10, 10, 256, 128, 3, 1, 9, True, False, False, "conv_igemm2_kernel<128,6>"),      # CTA pair, 36 k-steps, BN = 128
+    (7, 6, 10, 256, 256, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,1>"),      # non-square map, 9-class bias
 ]
 
 
-@pytest.mark.parametrize("case", CONV_CASES, ids=lambda c: "n%d_h%d_%dto%d_k%ds%d_c%d%s%s%s" % (
-    c[0], c[1], c[2], c[3], c[4], c[5], c[6], "_prelu" if c[7] else "", "_res" if c[8] else "", "_f32" if c[9] else ""))
+def _conv_id(c):
+    hw = "h%d" % c[1] if c[1] == c[2] else "h%dw%d" % (c[1], c[2])
+    return "n%d_%s_%dto%d_k%ds%d_c%d%s%s%s" % (c[0], hw, c[3], c[4], c[5], c[6], c[7], "_prelu" if c[8] else "",
+                                              "_res" if c[9] else "", "_f32" if c[10] else "")
+
+
+@pytest.mark.parametrize("case", CONV_CASES, ids=_conv_id)
 def test_conv_igemm_matches_conv2d(case):
     dev = _dev()
-    err, out, ref = _conv_case(dev, *case, seed=11)
-    assert err < 1e-2, f"relative error {err}"
+    *shape, variant = case
+    out, ref, ran = _conv_case(dev, *shape, seed=11)
+    assert ran == variant
+    _assert_conv_within_bound(out, ref, shape[-1])
+
+
+# (n_alloc, case): the tensor-map extent holds more frames than the pass computes (the plan's layout)
+PADDED_CASES = [
+    (11, (3, 10, 10, 256, 256, 3, 1, 9, True, False, False, "conv_igemm_kernel<256,4,0,1>")),
+    (806, (799, 10, 10, 256, 256, 3, 1, 9, True, False, False, "conv_igemm2_kernel<256,6>")),    # ragged last CTA pair
+]
 
 
 def test_conv_igemm_padded_allocation_matches():
-    """Same layer with the tensor-map extent larger than the valid frames (the plan's layout)."""
+    """Same layers with the tensor-map extent larger than the valid frames (the plan's layout)."""
     dev = _dev()
-    err, _, _ = _conv_case(dev, 3, 10, 256, 256, 3, 1, 9, True, False, False, seed=12, n_alloc=11)
-    assert err < 1e-2
+    for n_alloc, (*shape, variant) in PADDED_CASES:
+        out, ref, ran = _conv_case(dev, *shape, seed=12, n_alloc=n_alloc)
+        assert ran == variant
+        _assert_conv_within_bound(out, ref, shape[-1])
 
 
 def test_stem_and_units_progressively():
