@@ -24,6 +24,10 @@ class IrUnit(C.Structure):
                 ("w2", C.c_void_p), ("bias2", C.c_void_p)]
 
 
+class IrSe(C.Structure):
+    _fields_ = [("hidden", C.c_int32), ("reserved", C.c_int32), ("fc1", C.c_void_p), ("fc2", C.c_void_p)]
+
+
 class Ir50Weights(C.Structure):
     _fields_ = [("in_h", C.c_int32), ("in_w", C.c_int32),
                 ("stem_w", C.c_void_p), ("stem_bias", C.c_void_p), ("stem_alpha", C.c_void_p),
@@ -97,6 +101,9 @@ SIGNATURES = {
     "cer_check_device": (C.c_int, []),
     "cer_ir50_workspace_bytes": (C.c_size_t, [C.POINTER(Ir50Weights), C.c_int64]),
     "cer_ir50_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(Ir50Weights), C.c_int64, C.c_void_p, C.c_size_t]),
+    "cer_ir50_workspace_bytes_se": (C.c_size_t, [C.POINTER(Ir50Weights), C.POINTER(IrSe), C.c_int64]),
+    "cer_ir50_create_se": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(Ir50Weights), C.POINTER(IrSe), C.c_int64, C.c_void_p,
+                                     C.c_size_t]),
     "cer_ir50_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "cer_ir50_debug_activation": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
     "cer_ir50_op_variant": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_char_p, C.c_int32]),

@@ -9,7 +9,7 @@ int set_error(int code, const std::string& msg) {
 }  // namespace cer
 
 extern "C" const char* cer_last_error(void) { return cer::g_last_error.c_str(); }
-extern "C" int cer_version(void) { return 100; }
+extern "C" int cer_version(void) { return 101; }
 
 extern "C" int cer_check_device(void) {
   int dev = 0;

@@ -26,6 +26,7 @@ struct ConvGeom {
   const void* weight; const float* bias; int bias_classes; const float* alpha;
   const __nv_bfloat16* res; void* dst; int Cout; int out_fp32;
   int pool;        // 1: fuse MaxPool2d(2,2) into the epilogue (dst is the pooled tensor); see conv_can_pool()
+  int wld;         // elements per weight row (0: the conv's K); a conv over a column slice of a wider weight matrix
 };
 
 int load_driver_entry_points();

@@ -1,6 +1,6 @@
-// IR-50 frame encoder plan: stem kernel, tcgen05 implicit-GEMM residual units, FC head, L2 norm.
-// C-ABI: cer_ir50_* in include/cer_b200.h.  Reference semantics: models/arcface_model.py:44-60,
-// :120-151 and models/backbone.py:99-103 (see DESIGN.md for the BN folding algebra).
+// IR frame encoder plan (IR-50/100/152, plain or with SE units): stem kernel, tcgen05 implicit-GEMM residual
+// units, SE tails (se.cu), FC head, L2 norm.  C-ABI: cer_ir50_* in include/cer_b200.h.  Reference semantics:
+// models/arcface_model.py:23-84, :120-151 and models/backbone.py:99-103 (see DESIGN.md for the BN folding algebra).
 #include <cuda_runtime.h>
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -18,6 +18,7 @@
 #include "stem_tc.cuh"
 #include "conv_strip.cuh"
 #include "conv_raster.cuh"
+#include "se.h"
 #include <cstdlib>
 
 namespace cer {
@@ -196,10 +197,10 @@ static int make_im2col_map(CUtensorMap* map, const void* base, int N, int H, int
   return CER_OK;
 }
 
-// Packed weights [Cout][K] bf16, box = 64 (k) x BN (cout), 128B swizzle.
-static int make_weight_map(CUtensorMap* map, const void* base, int Cout, int K, int BN) {
+// Packed weights [Cout][K] bf16 (rows of ld >= K elements; 0: ld = K), box = 64 (k) x BN (cout), 128B swizzle.
+static int make_weight_map(CUtensorMap* map, const void* base, int Cout, int K, int BN, int ld = 0) {
   cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)Cout};
-  cuuint64_t strides[1] = {(cuuint64_t)K * 2};
+  cuuint64_t strides[1] = {(cuuint64_t)(ld > 0 ? ld : K) * 2};
   cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)BN};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box,
@@ -351,9 +352,9 @@ int build_conv_op(ConvOp* op, const ConvGeom& g, int n_cap, bool host_tables) {
     p.tmap_a2 = p.tmap_a;
   }
   const int ktot = g.ksize * g.ksize * g.Cin + g.Cin2;
-  rc = make_weight_map(&p.tmap_b, g.weight, g.Cout, ktot, op->bn);
+  rc = make_weight_map(&p.tmap_b, g.weight, g.Cout, ktot, op->bn, g.wld);
   if (rc) return rc;
-  rc = make_weight_map(&op->tmap_b_half, g.weight, g.Cout, ktot, op->bn / 2);
+  rc = make_weight_map(&op->tmap_b_half, g.weight, g.Cout, ktot, op->bn / 2, g.wld);
   if (rc) return rc;
   p.Hout = Hout; p.Wout = Wout; p.Cout = g.Cout;
   p.cin_chunks = g.Cin / kBlockK;
@@ -736,6 +737,17 @@ struct cer_ir50 {
   std::vector<ActInfo> unit_out;    // where each unit's output lives
   ActInfo stem_out;
   CUtensorMap stem_out_map;         // stem output [pixels][64] bf16 for the TMA store of stem_tc_kernel
+  // IR-SE units (cer_ir50_create_se): conv2 stores the pre-gate r; the projection conv (ops[proj_op], after the FC)
+  // writes the shortcut into the conv1 buffer; then squeeze-excite into `gate` and r * gate + shortcut over r.
+  struct SeTail {
+    int on, hidden;
+    const float* fc1; const float* fc2;
+    int proj_op;                    // -1: identity shortcut read from the unit input at stride sc_stride
+    const __nv_bfloat16* sc; int sc_h, sc_w, sc_stride;
+    __nv_bfloat16* r; int Ho, Wo, C;
+  };
+  std::vector<SeTail> se;           // per unit (all off for an IR plan)
+  float* gate;                      // [cap][512] fp32, SE plans only
 };
 
 static const int kPadFrames = 8;   // a 128-pixel tile may run at most 127 pixels (<= 6 frames of 5x5) past the end
@@ -767,7 +779,8 @@ static int build_raster_stage(cer_ir50* p) {
     int h = H, w2 = W;
     for (int i = 0; i < n_units; ++i) {
       const cer_ir_unit& u = p->units[i];
-      ok[i] = raster_unit_ok(h, w2, u.cin, u.depth, u.stride, u.has_proj);
+      // an SE unit runs on the im2col kernels; its tail stores dense NHWC, so the unit after it cannot start a run
+      ok[i] = raster_unit_ok(h, w2, u.cin, u.depth, u.stride, u.has_proj) && !p->se[i].on && !(i > 0 && p->se[i - 1].on);
       // the tensor a run starts from must be storable as a padded raster: by an im2col kernel (Cin >= 128: never
       // the halo / strip kernels), not by the stem
       if (ok[i] && (i == 0 || (!ok[i - 1] && p->units[i - 1].depth < 128))) ok[i] = 0;
@@ -809,9 +822,26 @@ static bool raster_pass(const cer_ir50* p, int frames) {
   return p->raster_hw > 0 && ((long long)frames * p->raster_hw + kBlockM - 1) / kBlockM >= 4LL * p->num_sms;
 }
 
-// one conv op of a pass (op = 0 .. 2U-1 unit convs, 2U = FC)
+// the SE tail of unit i after its conv2: projection conv (transition units), squeeze-excite, scale + shortcut
+static int launch_se_tail(cer_ir50* p, int i, int frames, cudaStream_t st) {
+  const cer_ir50::SeTail& s = p->se[i];
+  if (s.proj_op >= 0) {
+    int rc = launch_conv(p->ops[s.proj_op], frames, p->num_sms, st);
+    if (rc) return rc;
+  }
+  int rc = launch_se_squeeze(s.r, s.fc1, s.fc2, p->gate, frames, s.Ho * s.Wo, s.C, s.hidden, st);
+  if (rc) return rc;
+  return launch_se_scale(s.r, p->gate, s.sc, frames, s.Ho, s.Wo, s.C, s.sc_h, s.sc_w, s.sc_stride, p->num_sms, st);
+}
+
+// one op of a pass (op = 0 .. 2U-1 unit convs, 2U = FC); the conv2 op of an SE unit includes the unit's SE tail
 static int launch_plan_op(cer_ir50* p, int op, int frames, bool rast, cudaStream_t st) {
   const int n_units = (int)p->units.size();
+  if (op < 2 * n_units && (op & 1) && p->se[op >> 1].on) {
+    int rc = launch_conv(p->ops[op], frames, p->num_sms, st);
+    if (rc) return rc;
+    return launch_se_tail(p, op >> 1, frames, st);
+  }
   if (!rast || op >= 2 * n_units) return launch_conv(p->ops[op], frames, p->num_sms, st);
   const cer_ir50::RasterOp& r = p->rops[op];
   if (r.rast_ok) return launch_raster(r.kp, frames, p->num_sms, st);
@@ -824,15 +854,27 @@ static int launch_plan_op(cer_ir50* p, int op, int frames, bool rast, cudaStream
   return launch_conv(p->ops[op], frames, p->num_sms, st, kp.Wout + 1);
 }
 
-extern "C" size_t cer_ir50_workspace_bytes(const cer_ir50_weights* w, int64_t frames_per_pass) {
+static const int kSeMaxC = 512;     // gate buffer row: the widest unit
+static size_t gate_bytes(int64_t frames_per_pass) { return ((size_t)frames_per_pass * kSeMaxC * 4 + 1023) & ~size_t(1023); }
+
+extern "C" size_t cer_ir50_workspace_bytes_se(const cer_ir50_weights* w, const cer_ir_se* se, int64_t frames_per_pass) {
   if (!w || frames_per_pass <= 0) return 0;
   const size_t act = ((max_act_bytes_per_frame(w) * (frames_per_pass + kPadFrames)) + 1023) & ~size_t(1023);
   const size_t fc = (((size_t)frames_per_pass + kPadFrames) * w->emb_dim * 4 + 1023) & ~size_t(1023);
-  return 3 * act + fc + 1024;
+  return 3 * act + fc + 1024 + (se ? gate_bytes(frames_per_pass) : 0);
+}
+
+extern "C" size_t cer_ir50_workspace_bytes(const cer_ir50_weights* w, int64_t frames_per_pass) {
+  return cer_ir50_workspace_bytes_se(w, nullptr, frames_per_pass);
 }
 
 extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_t frames_per_pass,
                                void* workspace_dev, size_t workspace_bytes) {
+  return cer_ir50_create_se(out, w, nullptr, frames_per_pass, workspace_dev, workspace_bytes);
+}
+
+extern "C" int cer_ir50_create_se(cer_ir50** out, const cer_ir50_weights* w, const cer_ir_se* se, int64_t frames_per_pass,
+                                  void* workspace_dev, size_t workspace_bytes) {
   if (!out || !w || !workspace_dev || frames_per_pass <= 0 || w->n_units <= 0 || !w->units)
     return set_error(CER_ERR_INVALID, "cer_ir50_create: null/invalid argument");
   if (frames_per_pass + kPadFrames > (1 << 24)) return set_error(CER_ERR_INVALID, "frames_per_pass too large");
@@ -840,8 +882,15 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
   if (rc) return rc;
   rc = load_driver_entry_points();
   if (rc) return rc;
-  if (workspace_bytes < cer_ir50_workspace_bytes(w, frames_per_pass))
+  if (workspace_bytes < cer_ir50_workspace_bytes_se(w, se, frames_per_pass))
     return set_error(CER_ERR_WORKSPACE, "cer_ir50_create: workspace too small");
+  if (se) {
+    for (int i = 0; i < w->n_units; ++i) {
+      const int d = w->units[i].depth;
+      if (!se[i].fc1 || !se[i].fc2 || se[i].hidden <= 0 || se[i].hidden > 64 || d > kSeMaxC || 256 % (d / 8))
+        return set_error(CER_ERR_INVALID, "cer_ir50_create_se: SE unit needs fc1/fc2, 0 < hidden <= 64, depth in {64,128,256,512}");
+    }
+  }
   if (reinterpret_cast<uintptr_t>(workspace_dev) % 256) return set_error(CER_ERR_INVALID, "workspace must be 256B aligned");
 
   cer_ir50* p = new cer_ir50();
@@ -857,6 +906,10 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace_dev) + 1023) & ~uintptr_t(1023));
   for (int i = 0; i < 3; ++i) p->buf[i] = base + i * p->act_bytes;
   p->fc_out = reinterpret_cast<float*>(base + 3 * p->act_bytes);
+  const size_t fc_bytes = ((size_t)p->n_cap * w->emb_dim * 4 + 1023) & ~size_t(1023);
+  p->gate = se ? reinterpret_cast<float*>(base + 3 * p->act_bytes + fc_bytes) : nullptr;
+  p->se.assign(w->n_units, cer_ir50::SeTail{});
+  std::vector<int> proj_units;
 
   int H = w->in_h, W = w->in_w;
   int cur = 0, tb = 1, nxt = 2;
@@ -867,9 +920,11 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
   for (int i = 0; i < w->n_units; ++i) {
     const cer_ir_unit& u = p->units[i];
     if (u.cin != C) { delete p; return set_error(CER_ERR_INVALID, "unit cin does not match previous depth"); }
-    if (!u.has_proj && (u.stride != 1 || u.cin != u.depth)) {
+    const bool is_se = se != nullptr;
+    if (!u.has_proj && (u.cin != u.depth || (u.stride != 1 && !is_se))) {
       delete p;
-      return set_error(CER_ERR_INVALID, "identity shortcut needs stride 1 and cin == depth (MaxPool(1,2) shortcut unsupported)");
+      return set_error(CER_ERR_INVALID,
+                       "identity shortcut needs cin == depth and stride 1 (pass a MaxPool(1,2) shortcut as identity columns)");
     }
     ConvGeom g1{};
     g1.src = p->buf[cur]; g1.H = H; g1.W = W; g1.Cin = u.cin; g1.ksize = 3; g1.stride = 1; g1.pad = 1;
@@ -882,7 +937,10 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
 
     ConvGeom g2{};
     g2.src = p->buf[tb]; g2.H = H; g2.W = W; g2.Cin = u.depth; g2.ksize = 3; g2.stride = u.stride; g2.pad = 1;
-    if (u.has_proj) {
+    if (is_se) {
+      // r = conv2 + BN shift only: the gate scales r, the shortcut is added after it (launch_se_tail)
+      if (u.has_proj) { g2.wld = 9 * u.depth + u.cin; proj_units.push_back(i); }
+    } else if (u.has_proj) {
       g2.src2 = p->buf[cur]; g2.H2 = H; g2.W2 = W; g2.Cin2 = u.cin; g2.stride2 = u.stride;
     } else {
       g2.res = reinterpret_cast<const __nv_bfloat16*>(p->buf[cur]);
@@ -894,9 +952,20 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
     if (rc) { delete p; return rc; }
     p->ops.push_back(op2);
 
+    const int Hin = H, Win = W;
     H = (H - 1) / u.stride + 1;
     W = (W - 1) / u.stride + 1;
     C = u.depth;
+    if (is_se) {
+      cer_ir50::SeTail& t = p->se[i];
+      t.on = 1; t.hidden = se[i].hidden; t.fc1 = se[i].fc1; t.fc2 = se[i].fc2; t.proj_op = -1;
+      t.r = reinterpret_cast<__nv_bfloat16*>(p->buf[nxt]); t.Ho = H; t.Wo = W; t.C = C;
+      if (u.has_proj) {      // the projection output lands in the conv1 buffer, which conv2 has consumed
+        t.sc = reinterpret_cast<const __nv_bfloat16*>(p->buf[tb]); t.sc_h = H; t.sc_w = W; t.sc_stride = 1;
+      } else {
+        t.sc = reinterpret_cast<const __nv_bfloat16*>(p->buf[cur]); t.sc_h = Hin; t.sc_w = Win; t.sc_stride = u.stride;
+      }
+    }
     p->unit_out.push_back({p->buf[nxt], H, W, C});
     std::swap(cur, nxt);
   }
@@ -911,6 +980,22 @@ extern "C" int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_
   rc = build_conv_op(&opf, gf, p->n_cap, true);
   if (rc) { delete p; return rc; }
   p->ops.push_back(opf);
+  // projection convs of the SE transition units: op indices after the FC; K = the w2 columns after 9*depth, BN folded,
+  // output into the conv1 buffer (smaller than conv1's output: stride 2, same depth)
+  for (int i : proj_units) {
+    const cer_ir_unit& u = p->units[i];
+    const cer_ir50::ActInfo& x = i == 0 ? p->stem_out : p->unit_out[i - 1];
+    ConvGeom gp{};
+    gp.src = x.ptr; gp.H = x.H; gp.W = x.W; gp.Cin = u.cin; gp.ksize = 1; gp.stride = u.stride; gp.pad = 0;
+    gp.weight = static_cast<const __nv_bfloat16*>(u.w2) + 9 * u.depth; gp.wld = 9 * u.depth + u.cin;
+    gp.bias = u.bias2 + u.depth; gp.bias_classes = 1; gp.alpha = nullptr;
+    gp.dst = const_cast<__nv_bfloat16*>(p->se[i].sc); gp.Cout = u.depth; gp.out_fp32 = 0;
+    ConvOp opp;
+    rc = build_conv_op(&opp, gp, p->n_cap, true);
+    if (rc) { delete p; return rc; }
+    p->se[i].proj_op = (int)p->ops.size();
+    p->ops.push_back(opp);
+  }
   *out = p;
   return CER_OK;
 }
@@ -993,7 +1078,7 @@ extern "C" const char* cer_conv_last_variant(void) { return conv_last_variant();
 // (conv1, conv2 of unit 0, ...), 2U + 1 = FC.  The activation buffers must hold a previous forward of the
 // same frames (every op then reads the same data it reads in a real pass).
 extern "C" int cer_ir50_run_ops(cer_ir50* p, const float* x, int64_t frames, int32_t first_op, int32_t last_op, void* stream) {
-  const int n_conv = p ? (int)p->ops.size() : 0;
+  const int n_conv = p ? 2 * (int)p->units.size() + 1 : 0;     // unit convs + FC (projection convs run inside conv2 ops)
   if (!p || frames <= 0 || frames > p->cap || first_op < 0 || last_op < first_op || last_op > n_conv || (first_op == 0 && !x))
     return set_error(CER_ERR_INVALID, "cer_ir50_run_ops: bad argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1015,6 +1100,7 @@ extern "C" int64_t cer_ir50_launches(const cer_ir50* p, int64_t n_frames) {
   for (int64_t f0 = 0; f0 < n_frames; f0 += p->cap) {
     const int frames = (int)std::min<int64_t>(p->cap, n_frames - f0);
     total += 1 + 2 * (int64_t)p->units.size() + 2;
+    for (const cer_ir50::SeTail& t : p->se) total += t.on ? 2 + (t.proj_op >= 0) : 0;   // squeeze, scale (+ projection)
     if (raster_pass(p, frames))
       for (const cer_ir50::RasterOp& r : p->rops) total += (!r.rast_ok && r.out_padded) ? 1 : 0;   // raster_zero_pads_kernel
   }

@@ -11,7 +11,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import _capi
-from ._capi import FusionWeights, Ir50Weights, IrUnit, TcnBlock, VggConv, VggFc, VggishWeights, check, lib
+from ._capi import FusionWeights, Ir50Weights, IrSe, IrUnit, TcnBlock, VggConv, VggFc, VggishWeights, check, lib
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -19,8 +19,9 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
 
 
 class Ir50Engine:
-    """IR-50 frame encoder plan (cer_ir50_*).  ``frames_per_pass`` bounds the workspace: inputs
-    longer than that are processed in passes inside one C call."""
+    """IR frame encoder plan (cer_ir50_*): IR-50/100/152, plain or IR-SE (packed units carrying "se" weights run
+    through cer_ir50_create_se).  ``frames_per_pass`` bounds the workspace: inputs longer than that are
+    processed in passes inside one C call."""
 
     def __init__(self, packed: dict, device: torch.device, frames_per_pass: int = 512):
         _capi.require_gpu()
@@ -42,10 +43,21 @@ class Ir50Engine:
         self._w = Ir50Weights(packed["in_hw"], packed["in_hw"], put(packed["stem_w"]), put(packed["stem_bias"]),
                               put(packed["stem_alpha"]), len(units), self._units, packed["fc_in"], packed["emb_dim"],
                               put(packed["fc_w"]), put(packed["fc_bias"]))
+        self.se = "se" in units[0]
+        if any(("se" in u) != self.se for u in units):
+            raise ValueError("either every unit or no unit carries SE weights")
+        self._se = None
+        if self.se:
+            self._se = (IrSe * len(units))()
+            for i, u in enumerate(units):
+                self._se[i] = IrSe(u["se"]["fc1"].shape[0], 0, put(u["se"]["fc1"]), put(u["se"]["fc2"]))
         self.emb_dim = packed["emb_dim"]
         self.in_hw = packed["in_hw"]
         self.unit_shapes = []
-        self.conv_ops = []            # per conv op in plan order: geometry and algorithmic FLOPs per frame (bench accounting)
+        # per conv op in plan order (conv1, conv2 per unit, the FC, then the SE plan's projection convs): geometry and
+        # algorithmic FLOPs per frame (bench accounting; identity columns of a MaxPool(1, 2) shortcut are not counted)
+        self.conv_ops = []
+        proj_ops = []
         hw = self.in_hw
         for u in units:
             hin = hw
@@ -54,16 +66,22 @@ class Ir50Engine:
             self.conv_ops.append({"cin": u["cin"], "cout": u["depth"], "h_in": hin, "h_out": hin, "stride": 1, "proj_cin": 0,
                                   "flop": 2.0 * hin * hin * u["depth"] * 9 * u["cin"]})
             kproj = u["cin"] if u["has_proj"] else 0
+            if self.se and kproj:
+                proj_ops.append({"cin": u["cin"], "cout": u["depth"], "h_in": hin, "h_out": hw, "stride": u["stride"],
+                                 "proj_cin": 0, "flop": 2.0 * hw * hw * u["depth"] * kproj})
+                kproj = 0
+            kflop = 0 if u.get("identity_sc") else kproj
             self.conv_ops.append({"cin": u["depth"], "cout": u["depth"], "h_in": hin, "h_out": hw, "stride": u["stride"],
-                                  "proj_cin": kproj, "flop": 2.0 * hw * hw * u["depth"] * (9 * u["depth"] + kproj)})
+                                  "proj_cin": kproj, "flop": 2.0 * hw * hw * u["depth"] * (9 * u["depth"] + kflop)})
         self.conv_ops.append({"cin": packed["fc_in"], "cout": packed["emb_dim"], "h_in": 1, "h_out": 1, "stride": 1, "proj_cin": 0,
                               "flop": 2.0 * packed["fc_in"] * packed["emb_dim"]})
+        self.conv_ops += proj_ops
         with torch.cuda.device(self.device):
-            nbytes = lib().cer_ir50_workspace_bytes(C.byref(self._w), self.frames_per_pass)
+            nbytes = lib().cer_ir50_workspace_bytes_se(C.byref(self._w), self._se, self.frames_per_pass)
             self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
             h = C.c_void_p()
-            check(lib().cer_ir50_create(C.byref(h), C.byref(self._w), self.frames_per_pass, self._ws.data_ptr(), nbytes),
-                  "cer_ir50_create")
+            check(lib().cer_ir50_create_se(C.byref(h), C.byref(self._w), self._se, self.frames_per_pass, self._ws.data_ptr(),
+                                           nbytes), "cer_ir50_create_se")
         self._h = h
 
     def forward(self, x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -98,10 +116,11 @@ class Ir50Engine:
 
     @property
     def n_conv_ops(self) -> int:
-        return 2 * len(self.unit_shapes) + 1
+        return len(self.conv_ops)
 
     def op_variant(self, op_index: int, n_frames: int) -> str:
-        """Kernel instantiation the plan launches for conv op ``op_index`` (conv1, conv2 of each unit, then the FC)."""
+        """Kernel instantiation the plan launches for conv op ``op_index`` (conv1, conv2 of each unit, the FC, then
+        the SE plan's projection convs)."""
         buf = C.create_string_buffer(96)
         check(lib().cer_ir50_op_variant(self._h, op_index, n_frames, buf, 96), "cer_ir50_op_variant")
         return buf.value.decode()

@@ -114,6 +114,27 @@ class bottleneck_IR(nn.Module):
                                        nn.BatchNorm2d(depth))
 
 
+class SEModule(nn.Module):
+    """Parameter layout of models/arcface_model.py:23-41: fc1 / fc2 1x1 convs without bias (the gate
+    sigmoid(fc2(relu(fc1(mean_hw(x))))) runs in se.cu)."""
+
+    def __init__(self, channels: int, reduction: int):
+        super().__init__()
+        self.avg_pool = nn.AdaptiveAvgPool2d(1)
+        self.fc1 = nn.Conv2d(channels, channels // reduction, kernel_size=1, padding=0, bias=False)
+        self.relu = nn.ReLU(inplace=True)
+        self.fc2 = nn.Conv2d(channels // reduction, channels, kernel_size=1, padding=0, bias=False)
+        self.sigmoid = nn.Sigmoid()
+
+
+class bottleneck_IR_SE(bottleneck_IR):
+    """Parameter layout of models/arcface_model.py:63-84: bottleneck_IR plus res_layer.5 = SEModule(depth, 16)."""
+
+    def __init__(self, in_channel: int, depth: int, stride: int):
+        super().__init__(in_channel, depth, stride)
+        self.res_layer.append(SEModule(depth, 16))
+
+
 def get_blocks(num_layers: int):
     """Unit table of models/arcface_model.py:95-117 as (in_channel, depth, stride) triples."""
     def stage(cin, depth, n, stride=2):
@@ -137,21 +158,24 @@ class Backbone(_PackedModule):
     The CUDA plan is built for the spatial size the output_layer expects (H = 8*sqrt(fc_in/512));
     as in the reference, a mismatching input size is an error."""
 
-    frames_per_pass = 2400      # frames per pass of the plan (workspace ~1.25 MB per frame)
+    frames_per_pass = 2400      # frames per pass of IR-50 / IR-SE-50 plans (workspace ~1.25 MB per 40 px frame)
+    # IR-100 / IR-152 (total stride 16, 112 px inputs for the 7x7 head): ~4.8 MB of workspace per frame; 512 frames
+    # give stage 4 (7 x 7 px per frame) about 200 output tiles of 128 px x 256 channels, more than the 148 SMs
+    deep_frames_per_pass = 512
 
     def __init__(self, num_layers, drop_ratio, input_channels=3, mode='ir'):
         super().__init__()
         assert num_layers in [50, 100, 152], 'num_layers should be 50,100, or 152'
         assert mode in ['ir', 'ir_se'], 'mode should be ir or ir_se'
-        if mode != 'ir':
-            raise NotImplementedError("mode 'ir_se' is not on the LFAN path (never selected: backbone.py:73)")
         if input_channels != 3:
             raise NotImplementedError("the stem kernel is built for 3 input channels (RGB face crops)")
+        unit_module = bottleneck_IR if mode == 'ir' else bottleneck_IR_SE
         self.input_layer = nn.Sequential(nn.Conv2d(input_channels, 64, (3, 3), 1, 1, bias=False),
                                          nn.BatchNorm2d(64), nn.PReLU(64))
         self.output_layer = _output_layer(512, 7, drop_ratio)
-        self.body = nn.Sequential(*[bottleneck_IR(c, d, s) for c, d, s in get_blocks(num_layers)])
+        self.body = nn.Sequential(*[unit_module(c, d, s) for c, d, s in get_blocks(num_layers)])
         self._strides = [s for _, _, s in get_blocks(num_layers)]
+        self._num_layers = num_layers
 
     def _build_engine(self) -> Ir50Engine:
         sd = {k: v.detach().cpu() for k, v in self.state_dict().items()}
@@ -160,12 +184,10 @@ class Backbone(_PackedModule):
             total_stride *= s
         fc_in = sd["output_layer.3.weight"].shape[1]
         spatial = int(round((fc_in / 512) ** 0.5))
-        pk = packing.pack_ir50(sd, prefix="", in_hw=spatial * total_stride)
         # the reference's strides are carried by the modules, not the state_dict
-        for u, s in zip(pk["units"], self._strides):
-            if u["stride"] != s:
-                raise NotImplementedError("a stride-2 unit with identity (MaxPool) shortcut is not built (IR-100/152 stage 1)")
-        return Ir50Engine(pk, self._device(), self.frames_per_pass)
+        pk = packing.pack_ir50(sd, prefix="", in_hw=spatial * total_stride, strides=self._strides)
+        fpp = self.frames_per_pass if self._num_layers == 50 else self.deep_frames_per_pass
+        return Ir50Engine(pk, self._device(), fpp)
 
     def engine(self) -> Ir50Engine:
         eng = self._fresh_engine()
@@ -178,8 +200,8 @@ class Backbone(_PackedModule):
 
 
 class VisualBackbone(_PackedModule):
-    """models/backbone.py:69-130: IR-50 with the 5x5 head (40x40 inputs) plus the unused
-    ``logits`` Linear that strict state_dict loading requires."""
+    """models/backbone.py:69-130: IR-50 (mode='ir') or IR-SE-50 (mode='ir_se') with the 5x5 head (40x40
+    inputs) plus the unused ``logits`` Linear that strict state_dict loading requires."""
 
     def __init__(self, input_channels=3, num_classes=8, use_pretrained=True, state_dict_path="", mode="ir",
                  embedding_dim=512):

@@ -15,6 +15,12 @@ Algebra (eval mode; reference lines in brackets):
   epilogue indexes it with the border class of each output pixel.  Exact, no extra activation.
 * The 1x1/stride-2 projection shortcut of the first unit of stages 2-4 is appended to conv2's K
   axis (its own BN scale folded in), so `res + shortcut` [:57-60] is one accumulation.
+* The MaxPool2d(1, 2) shortcut of a stride-2 unit with cin == depth (stage 1 of IR-100 / IR-152) is
+  packed the same way with identity columns, w2 = [w2 | I]: products by 1.0 are exact.
+* IR-SE units (bottleneck_IR_SE [:63-84], SEModule [:23-41]): the gate scales the residual branch
+  only, so the plan keeps the shortcut out of conv2 -- a projection keeps its columns in w2 but runs
+  as its own 1x1 conv, with its BN shift as a second bias row (bias2 [2][depth]); a stride-2
+  identity shortcut stays an identity (has_proj = 0).  fc1 / fc2 ship as fp32 matrices.
 * output_layer [backbone.py:99-103]: BN2d and BN1d are folded into the Linear, whose K axis is
   permuted from NCHW-flatten (c,h,w) [arcface_model.py:12-14] to the NHWC order the conv stack
   produces.
@@ -36,26 +42,31 @@ def _bn_affine(sd, p):
     return s, t
 
 
-def infer_units(sd: Dict[str, torch.Tensor], prefix: str):
-    """(cin, depth, stride) per unit, recovered from the state_dict itself: a unit has a projection
-    shortcut iff shortcut_layer.0.weight exists; in this family projection <=> stride 2
-    (arcface_model.py:87-102), except a stride-1 stage-1 first unit which has cin == depth."""
+def infer_units(sd: Dict[str, torch.Tensor], prefix: str, strides: Sequence[int] = None):
+    """(cin, depth, stride, proj) per unit, recovered from the state_dict itself: a unit has a projection
+    shortcut iff shortcut_layer.0.weight exists.  Without ``strides``, stride 2 is inferred from a projection
+    (IR-50, arcface_model.py:87-102); the MaxPool2d(1, 2) shortcut of IR-100 / IR-152 stage 1 leaves no key,
+    so those strides come from the modules (``strides``, one per unit)."""
     units = []
     i = 0
     while f"{prefix}body.{i}.res_layer.1.weight" in sd:
         w1 = sd[f"{prefix}body.{i}.res_layer.1.weight"]
         depth, cin = int(w1.shape[0]), int(w1.shape[1])
         proj = f"{prefix}body.{i}.shortcut_layer.0.weight" in sd
-        units.append((cin, depth, 2 if proj else 1, proj))
+        units.append((cin, depth, (2 if proj else 1) if strides is None else int(strides[i]), proj))
         i += 1
+    if strides is not None and len(strides) != len(units):
+        raise ValueError(f"{len(strides)} strides for {len(units)} units")
     return units
 
 
 def pack_ir50(sd: Dict[str, torch.Tensor], prefix: str = "backbone.", in_hw: int = 40,
-              operand_dtype: torch.dtype = torch.bfloat16) -> dict:
+              operand_dtype: torch.dtype = torch.bfloat16, strides: Sequence[int] = None) -> dict:
     """Returns {'stem_w','stem_bias','stem_alpha', 'units': [ {cin,depth,stride,has_proj,w1,bias1,alpha,w2,bias2} ],
     'fc_w','fc_bias','fc_in','emb_dim'} as CPU tensors (``operand_dtype`` for w1/w2/fc_w -- bf16 for the
-    kernels, fp32 only in tests of the algebra -- fp32 otherwise)."""
+    kernels, fp32 only in tests of the algebra -- fp32 otherwise).  ``strides``: the units' strides (see
+    infer_units).  A unit whose MaxPool2d(1, 2) shortcut became identity columns also has 'identity_sc': 1; an
+    IR-SE unit has 'se': {'fc1' [hidden][depth], 'fc2' [depth][hidden]} (fp32)."""
     p = prefix
     out = {}
     W = sd[p + "input_layer.0.weight"].double()                      # [64, 3, 3, 3] (co, ci, r, s)
@@ -67,8 +78,9 @@ def pack_ir50(sd: Dict[str, torch.Tensor], prefix: str = "backbone.", in_hw: int
 
     units = []
     hw = in_hw
-    for i, (cin, depth, stride, proj) in enumerate(infer_units(sd, p)):
+    for i, (cin, depth, stride, proj) in enumerate(infer_units(sd, p, strides)):
         u = f"{p}body.{i}."
+        se = u + "res_layer.5.fc1.weight" in sd
         s1, t1 = _bn_affine(sd, u + "res_layer.0")
         W1 = sd[u + "res_layer.1.weight"].double()                   # [depth, cin, 3, 3]
         w1 = (W1 * s1.view(1, -1, 1, 1)).permute(0, 2, 3, 1).reshape(depth, 9 * cin)     # K = (r, s, ci)
@@ -82,17 +94,29 @@ def pack_ir50(sd: Dict[str, torch.Tensor], prefix: str = "backbone.", in_hw: int
         W2 = sd[u + "res_layer.3.weight"].double()                   # [depth, depth, 3, 3]
         w2 = (W2 * s2.view(-1, 1, 1, 1)).permute(0, 2, 3, 1).reshape(depth, 9 * depth)
         bias2 = t2.clone()
+        identity_sc = not proj and not se and stride != 1
         if proj:
             ss, ts = _bn_affine(sd, u + "shortcut_layer.1")
             Wsc = sd[u + "shortcut_layer.0.weight"].double().reshape(depth, cin)
             w2 = torch.cat([w2, Wsc * ss.view(-1, 1)], dim=1)
-            bias2 = bias2 + ts
-        units.append({
-            "cin": cin, "depth": depth, "stride": stride, "has_proj": int(proj),
+            bias2 = torch.stack([bias2, ts]) if se else bias2 + ts
+        elif identity_sc:
+            if cin != depth:
+                raise ValueError(f"unit {i}: an identity shortcut needs cin == depth")
+            w2 = torch.cat([w2, torch.eye(depth, dtype=torch.float64)], dim=1)
+        unit = {
+            "cin": cin, "depth": depth, "stride": stride, "has_proj": int(proj or identity_sc),
             "w1": w1.to(operand_dtype).contiguous(), "bias1": bias1.float().contiguous(),
             "alpha": sd[u + "res_layer.2.weight"].float().contiguous(),
             "w2": w2.to(operand_dtype).contiguous(), "bias2": bias2.float().contiguous(),
-        })
+        }
+        if identity_sc:
+            unit["identity_sc"] = 1
+        if se:
+            fc1 = sd[u + "res_layer.5.fc1.weight"]
+            unit["se"] = {"fc1": fc1.reshape(fc1.shape[0], depth).float().contiguous(),
+                          "fc2": sd[u + "res_layer.5.fc2.weight"].reshape(depth, fc1.shape[0]).float().contiguous()}
+        units.append(unit)
         hw = (hw - 1) // stride + 1
     out["units"] = units
 

@@ -17,12 +17,25 @@ from typing import Dict, List, Sequence
 
 import torch
 
+from .modules import get_blocks
+
 # (in_channel, depth, stride) per residual unit of IR-50 as configured by the reference
 # (models/arcface_model.py:95-102: unit counts 3/4/14/3, first stage stride 1).
 IR50_UNITS = ([(64, 64, 1)] * 3
               + [(64, 128, 2)] + [(128, 128, 1)] * 3
               + [(128, 256, 2)] + [(256, 256, 1)] * 13
               + [(256, 512, 2)] + [(512, 512, 1)] * 2)
+
+
+def ir_units(num_layers: int):
+    """(in_channel, depth, stride) per unit of IR-50 / IR-100 / IR-152 (modules.get_blocks)."""
+    return get_blocks(num_layers)
+
+
+# SE weight gains: fc1 ~ U(+-SE_GAIN1 / sqrt(depth)), fc2 ~ U(+-SE_GAIN2 / sqrt(hidden)).  Larger than a default
+# init so that the gates differ across channels AND frames (a gate stuck near one value would hide a gate
+# applied to the wrong frame), without saturating them (which would hide a dropped gate).
+SE_GAIN1, SE_GAIN2 = 8.0, 4.0
 
 # configs.py:61-73 (tcn.channels) and models/model.py:388-393 (embedding_dim / encoder_dim)
 TCN_CHANNELS = {
@@ -55,10 +68,13 @@ def _conv(sd, key, cout, cin, k, g):
 
 
 def visual_backbone_state_dict(seed: int = 0, units=IR50_UNITS, num_classes: int = 8,
-                               spatial: int = 5) -> "OrderedDict[str, torch.Tensor]":
+                               spatial: int = 5, se: bool = False) -> "OrderedDict[str, torch.Tensor]":
     """``VisualBackbone.state_dict()`` layout (models/backbone.py:69-130): prefix ``backbone.``
-    for the IR-50 and the unused ``logits.*`` head that strict loading still requires."""
+    for the IR-50 and the unused ``logits.*`` head that strict loading still requires.  ``units``: any
+    get_blocks table (ir_units(100) ...); ``se``: IR-SE units (res_layer.5.fc{1,2}.weight, drawn from their own
+    generator, so every other tensor equals the se=False one)."""
     g = torch.Generator().manual_seed(seed)
+    gse = torch.Generator().manual_seed(seed + 104729)
     sd: "OrderedDict[str, torch.Tensor]" = OrderedDict()
     b = "backbone."
     _conv(sd, b + "input_layer.0.weight", 64, 3, 3, g)
@@ -74,6 +90,10 @@ def visual_backbone_state_dict(seed: int = 0, units=IR50_UNITS, num_classes: int
         sd[u + "res_layer.2.weight"] = 0.25 + 0.1 * torch.randn(depth, generator=g)
         _conv(sd, u + "res_layer.3.weight", depth, depth, 3, g)
         _bn(sd, u + "res_layer.4", depth, g)
+        if se:
+            hid = depth // 16
+            sd[u + "res_layer.5.fc1.weight"] = _uniform(gse, (hid, depth, 1, 1), SE_GAIN1 * depth ** -0.5)
+            sd[u + "res_layer.5.fc2.weight"] = _uniform(gse, (depth, hid, 1, 1), SE_GAIN2 * hid ** -0.5)
     c = units[-1][1]
     _bn(sd, b + "output_layer.0", c, g)
     fin = c * spatial * spatial

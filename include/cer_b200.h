@@ -45,6 +45,10 @@ int cer_check_device(void);
  * (arcface_model.py:44-60), the 5x5 output_layer (backbone.py:99-103) and l2_norm (:17-20).
  * Weights arrive pre-packed by feature_vs_text_compound_emotion_b200/packing.py:
  * ------------------------------------------------------------------------------------------ */
+/* A MaxPool2d(1, s) shortcut with s = 2 (cin == depth: the first unit of IR-100 / IR-152) is passed as a
+ * projection with identity columns: w2 = [w2 | I], bias2 unchanged, has_proj = 1.  Products by 1.0 are exact.
+ * In an IR-SE unit (cer_ir_se) a stride-2 identity shortcut is passed as is (has_proj = 0): the SE tail reads
+ * the strided input directly. */
 typedef struct cer_ir_unit {
   int32_t cin, depth, stride;   /* bottleneck_IR(in_channel, depth, stride)                        */
   int32_t has_proj;             /* 1: 1x1/stride conv+BN shortcut fused as extra K columns of w2   */
@@ -53,7 +57,17 @@ typedef struct cer_ir_unit {
   const float* alpha;           /* fp32 [depth]          res_layer.2 PReLU slopes                                   */
   const void* w2;               /* bf16 [depth][9*depth (+cin)]  res_layer.3 * BN scale (+ shortcut conv * its BN scale) */
   const float* bias2;           /* fp32 [depth]          res_layer.4 BN shift (+ shortcut BN shift)                 */
+                                /* IR-SE unit with has_proj: fp32 [2][depth], res_layer.4 shift then shortcut shift */
 } cer_ir_unit;
+
+/* SEModule(depth, 16) of an IR-SE unit (bottleneck_IR_SE, models/arcface_model.py:23-41, 63-84): res_layer.5.
+ * The unit computes r = BN(conv3x3(PReLU(conv3x3(BN(x))))), gate[n][c] = sigmoid(fc2 relu(fc1 mean_hw(r))) and
+ * out = r * gate + shortcut(x).  A projection shortcut runs as its own 1x1 conv (the w2 columns after 9*depth). */
+typedef struct cer_ir_se {
+  int32_t hidden, reserved;     /* hidden = depth / 16 (<= 64); reserved = 0                        */
+  const float* fc1;             /* fp32 [hidden][depth]  res_layer.5.fc1.weight                     */
+  const float* fc2;             /* fp32 [depth][hidden]  res_layer.5.fc2.weight                     */
+} cer_ir_se;
 
 typedef struct cer_ir50_weights {
   int32_t in_h, in_w;           /* 40, 40                                                          */
@@ -76,6 +90,12 @@ size_t cer_ir50_workspace_bytes(const cer_ir50_weights* w, int64_t frames_per_pa
  * workspace must stay valid and unmoved for the life of the plan. */
 int cer_ir50_create(cer_ir50** out, const cer_ir50_weights* w, int64_t frames_per_pass, void* workspace_dev,
                     size_t workspace_bytes);
+/* The same for an IR-SE backbone: `se` is a HOST array of n_units entries (device pointers inside); NULL gives
+ * exactly the plan of cer_ir50_workspace_bytes / cer_ir50_create.  The SE plan adds a [frames_per_pass][512] fp32
+ * gate buffer to the workspace and does not run the padded-raster stage. */
+size_t cer_ir50_workspace_bytes_se(const cer_ir50_weights* w, const cer_ir_se* se, int64_t frames_per_pass);
+int cer_ir50_create_se(cer_ir50** out, const cer_ir50_weights* w, const cer_ir_se* se, int64_t frames_per_pass,
+                       void* workspace_dev, size_t workspace_bytes);
 /* x_nchw_dev: fp32 [n_frames][3][in_h][in_w] in [-1,1]; emb_out_dev: fp32 [n_frames][emb_dim],
  * unit L2 norm per row.  Any n_frames >= 0 (processed in passes). */
 int cer_ir50_forward(cer_ir50* plan, const float* x_nchw_dev, int64_t n_frames, float* emb_out_dev, void* stream);
@@ -86,15 +106,18 @@ int cer_ir50_forward(cer_ir50* plan, const float* x_nchw_dev, int64_t n_frames, 
 int64_t cer_ir50_debug_activation(cer_ir50* plan, const float* x_nchw_dev, int64_t frames, int32_t unit_index,
                                   void* dst_dev, void* stream);
 /* Name of the kernel instantiation the plan launches for conv op `op_index` (0 .. 2*n_units - 1: conv1,
- * conv2 of each unit in order; 2*n_units: the FC) when a pass holds min(n_frames, frames_per_pass) frames,
+ * conv2 of each unit in order; 2*n_units: the FC; after it, in an SE plan, the projection convs of the IR-SE
+ * transition units in unit order) when a pass holds min(n_frames, frames_per_pass) frames,
  * e.g. "conv_igemm2_kernel<256,6>".  Writes a NUL-terminated string, returns its length or a negative status. */
 int cer_ir50_op_variant(const cer_ir50* plan, int32_t op_index, int64_t n_frames, char* buf, int32_t buflen);
 /* Profiling aid: launch ops [first_op, last_op] of one pass in plan order (0 = stem, 1 .. 2*n_units = unit
  * convs, 2*n_units + 1 = FC) on `frames` <= frames_per_pass frames.  The plan's activation buffers must hold
- * an earlier forward of the same frames.  x_nchw_dev is read by op 0 only. */
+ * an earlier forward of the same frames.  x_nchw_dev is read by op 0 only.  The conv2 op of an IR-SE unit also
+ * runs that unit's projection conv and SE tail, so the full range 0 .. 2*n_units + 1 is one forward pass. */
 int cer_ir50_run_ops(cer_ir50* plan, const float* x_nchw_dev, int64_t frames, int32_t first_op, int32_t last_op, void* stream);
 /* Number of kernel launches one forward of n_frames enqueues (for bench accounting; depends on the pass sizes:
- * a pass that runs the padded-raster stage adds one pad-zeroing launch). */
+ * a pass that runs the padded-raster stage adds one pad-zeroing launch; an IR-SE unit adds its squeeze and
+ * scale kernels and, for a transition unit, its projection conv). */
 int64_t cer_ir50_launches(const cer_ir50* plan, int64_t n_frames);
 void cer_ir50_destroy(cer_ir50* plan);
 
