@@ -127,6 +127,7 @@ SIGNATURES = {
                                            C.c_void_p, C.c_size_t, C.c_void_p]),
     "cer_fusion_head_forward": (C.c_int, [C.POINTER(FusionWeights), C.POINTER(C.c_void_p), C.c_int64, C.c_void_p,
                                           C.c_void_p, C.c_void_p]),
+    "cer_head_last_variant": (C.c_char_p, []),
     "cer_head_train_workspace_bytes": (C.c_size_t, [C.POINTER(HeadTrainSpec), C.c_int64, C.c_int64]),
     "cer_head_train_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(HeadTrainSpec), C.c_int64, C.c_int64, C.c_void_p,
                                         C.c_size_t]),

@@ -6,10 +6,13 @@ int set_error(int code, const std::string& msg) {
   g_last_error = msg;
   return code;
 }
+static thread_local const char* g_head_variant = "none";
+void set_head_variant(const char* name) { g_head_variant = name; }
 }  // namespace cer
 
 extern "C" const char* cer_last_error(void) { return cer::g_last_error.c_str(); }
-extern "C" int cer_version(void) { return 101; }
+extern "C" int cer_version(void) { return 102; }
+extern "C" const char* cer_head_last_variant(void) { return cer::g_head_variant; }
 
 extern "C" int cer_check_device(void) {
   int dev = 0;

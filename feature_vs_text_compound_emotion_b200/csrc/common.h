@@ -6,6 +6,7 @@
 
 namespace cer {
 int set_error(int code, const std::string& msg);   // records msg for cer_last_error(), returns code
+void set_head_variant(const char* name);           // records the kernel a head launch site ran (cer_head_last_variant)
 }
 
 #define CER_CUDA(expr)                                                                              \

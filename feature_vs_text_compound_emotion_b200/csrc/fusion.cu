@@ -27,6 +27,10 @@ constexpr int kFusThreads = kFusWarps * 32;
 constexpr int kMaxE = 128;      // modal_dim * n_modals
 constexpr int kMaxOut = 16;
 
+// The instantiations cer_fusion_head_forward can run, kFR = 4..8 (cer_head_last_variant reports the one a launch used).
+static const char* const kHeadVariantNames[] = {"fusion_head_kernel<4>", "fusion_head_kernel<5>", "fusion_head_kernel<6>",
+                                                "fusion_head_kernel<7>", "fusion_head_kernel<8>"};
+
 struct FusionDims {
   int M, E, D3, hd, H, n_out, din_total, dim[CER_MAX_MODALS], doff[CER_MAX_MODALS];
 };
@@ -406,6 +410,7 @@ extern "C" int cer_fusion_head_forward(const cer_fusion_weights* w, const float*
     static unsigned long long configured = 0;                                                                              \
     if (first_use_on_device(&configured))                                                                                  \
       CER_CUDA(cudaFuncSetAttribute(fusion_head_kernel<FR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxDyn));   \
+    set_head_variant(kHeadVariantNames[FR - kFRMin]);                                                                      \
     fusion_head_kernel<FR><<<grid, kFusThreads, smem, st>>>(*w, d, f[0], f[1], f[2], f[3], (long long)rows, logits, fused_out); \
   } break;
   switch (fr) {

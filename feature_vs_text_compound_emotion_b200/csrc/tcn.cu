@@ -33,6 +33,15 @@ constexpr float kLeaky = 0.01f;
 
 __device__ __forceinline__ float lrelu(float v) { return v >= 0.f ? v : v * kLeaky; }
 
+// The instantiations launch_tcn can run, COUT-major (cer_head_last_variant reports the one a launch used).
+static const char* const kHeadVariantNames[] = {
+  "tcn_block_kernel<32,1,5>", "tcn_block_kernel<32,2,5>", "tcn_block_kernel<32,4,5>", "tcn_block_kernel<32,8,5>",
+  "tcn_block_kernel<64,1,5>", "tcn_block_kernel<64,2,5>", "tcn_block_kernel<64,4,5>", "tcn_block_kernel<64,8,5>",
+  "tcn_block_kernel<128,1,5>", "tcn_block_kernel<128,2,5>", "tcn_block_kernel<128,4,5>", "tcn_block_kernel<128,8,5>",
+  "tcn_block_kernel<256,1,5>", "tcn_block_kernel<256,2,5>", "tcn_block_kernel<256,4,5>", "tcn_block_kernel<256,8,5>"};
+
+constexpr int log2_small(int v) { return v <= 1 ? 0 : 1 + log2_small(v / 2); }
+
 // COUT in {32,64,128,256}; DIL in {1,2,4,8}; KS = kernel size (5).
 template <int COUT, int DIL, int KS>
 struct TcnCfg {
@@ -221,6 +230,8 @@ static int launch_tcn(const cer_tcn_block& blk, const float* x, float* y, int B,
   if (first_use_on_device(&configured)) {
     CER_CUDA(cudaFuncSetAttribute(tcn_block_kernel<COUT, DIL, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
   }
+  static_assert(COUT >= 32 && COUT <= 256 && DIL <= 8, "kHeadVariantNames covers COUT 32..256, DIL 1..8");
+  set_head_variant(kHeadVariantNames[4 * log2_small(COUT / 32) + log2_small(DIL)]);
   dim3 grid((T + kTT - 1) / kTT, B);
   tcn_block_kernel<COUT, DIL, 5><<<grid, kTcnThreads, C::SMEM, st>>>(blk, x, y, T);
   CER_CUDA(cudaGetLastError());

@@ -13,7 +13,11 @@
 //   B tile (BN couts x 32 fp32)  : tiled TMA from the packed weight [C_out][k*C_in (+ C_in_ds)].
 //   The 1x1 downsample of launch 2 accumulates into a second TMEM accumulator (it is added AFTER
 //   conv2's LeakyReLU, so it cannot share conv2's accumulator).
-// One CTA = one 128 x BN tile (the head has only B*T/128 * C_out/BN <= ~80 tiles).
+// One CTA = one 128 x BN tile (the head has only B*T/128 * C_out/BN <= ~80 tiles).  BN = 64 when C_out is a
+// multiple of 64, else 32, so every C_out % 32 == 0 is covered by whole N tiles.
+// Causal halo limit: the A map is a rank-4 im2col map, whose bounding-box corners cuTensorMapEncodeIm2col
+// accepts only in [-128, 127]; the lower corner is -(k-1)d, so (k-1)d <= 128 (checked before any encode).
+// The full range holds on a B200: a k = 5, d = 32 block (halo 128) matches its fp64 reference.
 // Why TF32 and not bf16: SURVEY.md H4 -- argmax parity of the head is marginal in bf16
 // (99.7-99.8 %) and safe in TF32 (1.5e-3 max-abs logit error, 100 % agreement).
 #include <cuda_runtime.h>
@@ -58,6 +62,10 @@ constexpr int kTcBlockM = 128;
 constexpr int kTcBlockK = 32;         // 32 fp32 = 128 B = one swizzle row; 4 MMAs of K = 8 per k-step
 constexpr int kTcABytes = kTcBlockM * 128;
 constexpr float kLeakyTc = 0.01f;
+constexpr int kTcMaxHalo = 128;
+
+// The instantiations launch_tcn_tc can run (cer_head_last_variant reports the one a launch used).
+static const char* const kHeadVariantNames[] = {"tcn_igemm_kernel<64,8>", "tcn_igemm_kernel<32,8>"};
 
 template <int BN, int STAGES>
 struct TcnSmem {
@@ -246,6 +254,8 @@ static int launch_tcn_tc(const TcnKernelParams& p, int grid, cudaStream_t st) {
   if (first_use_on_device(&configured)) {
     CER_CUDA(cudaFuncSetAttribute(tcn_igemm_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
   }
+  static_assert((BN == 64 || BN == 32) && STAGES == 8, "kHeadVariantNames lists <64,8> and <32,8> only");
+  set_head_variant(kHeadVariantNames[BN == 64 ? 0 : 1]);
   tcn_igemm_kernel<BN, STAGES><<<grid, kTcThreads, L::kTotal, st>>>(p);
   CER_CUDA(cudaGetLastError());
   return CER_OK;
@@ -271,7 +281,7 @@ static int run_tcn_conv(const float* main_in, int c_main, const float* ds_x, int
   } else {
     p.tmap_a2 = p.tmap_a;
   }
-  const int bn = cout >= 64 ? 64 : 32;
+  const int bn = cout % 64 == 0 ? 64 : 32;
   rc = make_tiled2d_map_generic(&p.tmap_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, weight, cout, ktot, bn, kTcBlockK);
   if (rc) return rc;
   p.M = B * T; p.T = T; p.Cout = cout;
@@ -302,7 +312,9 @@ extern "C" int cer_tcn_block_tc_forward(const cer_tcn_block* blk, const float* x
   if (!blk || !x || !y || batch <= 0 || length <= 0) return set_error(CER_ERR_INVALID, "cer_tcn_block_tc_forward: bad argument");
   if (blk->c_in % 32 || blk->c_out % 32) return set_error(CER_ERR_INVALID, "tcn_tc: channels must be multiples of 32");
   if (blk->kernel_size < 1 || blk->kernel_size > 8) return set_error(CER_ERR_INVALID, "tcn_tc: kernel_size out of range");
-  if ((blk->kernel_size - 1) * blk->dilation > 65535) return set_error(CER_ERR_INVALID, "tcn_tc: dilation too large");
+  if ((blk->kernel_size - 1) * blk->dilation > kTcMaxHalo)
+    return set_error(CER_ERR_INVALID, "tcn_tc: causal halo (kernel_size-1)*dilation must be at most 128 "
+                                      "(rank-4 im2col bounding-box corner limit)");
   if (!blk->w1 || !blk->b1 || !blk->w2 || !blk->b2) return set_error(CER_ERR_INVALID, "tcn_tc: null weight");
   const bool has_ds = blk->wd != nullptr;     // here `wd` only flags that w2 carries the downsample columns
   if (!has_ds && blk->c_in != blk->c_out) return set_error(CER_ERR_INVALID, "tcn_tc: identity residual needs c_in == c_out");

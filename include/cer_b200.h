@@ -218,7 +218,8 @@ int cer_tcn_block_forward(const cer_tcn_block* blk, const float* x_dev, float* y
  * accumulate) -- the production path.  Same struct, different weight layout:
  *   w1: fp32 [c_out][k*c_in], K = (tap, ci);   w2: fp32 [c_out][k*c_out (+ c_in)] with the 1x1
  *   downsample weights appended as the last c_in columns (wd != NULL only flags their presence,
- *   bd is its bias).  Channels must be multiples of 32.  workspace holds conv1's output. */
+ *   bd is its bias).  Channels must be multiples of 32, the causal halo (kernel_size-1)*dilation at most 128
+ *   (the im2col tensor map's bounding-box corner range).  workspace holds conv1's output. */
 size_t cer_tcn_block_tc_workspace_bytes(const cer_tcn_block* blk, int64_t batch, int64_t length);
 int cer_tcn_block_tc_forward(const cer_tcn_block* blk, const float* x_dev, float* y_dev, int64_t batch, int64_t length,
                              void* workspace_dev, size_t workspace_bytes, void* stream);
@@ -259,6 +260,12 @@ int cer_modal_attention_forward(const float* const* qkv_dev, int64_t rows, int32
 
 int cer_fusion_head_forward(const cer_fusion_weights* w, const float* const* feats_dev, int64_t rows,
                             float* logits_dev, float* fused_out_dev /* [rows][E] or NULL */, void* stream);
+
+/* Name of the kernel instantiation the last head launch on this thread ran: one conv launch of
+ * cer_tcn_block_tc_forward (e.g. "tcn_igemm_kernel<64,8>"), cer_tcn_block_forward ("tcn_block_kernel<128,4,5>")
+ * or cer_fusion_head_forward ("fusion_head_kernel<5>").  "none" before the first launch; a call refused
+ * before launching leaves it unchanged. */
+const char* cer_head_last_variant(void);
 
 /* ------------------------------------------------------------------------------------------
  * Fusion-head training step (BASELINE config 4).   Replaces, for the trainable head of LFAN
