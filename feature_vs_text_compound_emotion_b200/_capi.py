@@ -180,7 +180,18 @@ SIGNATURES = {
     "cer_tanh_inplace": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),
     "cer_stitch_windows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64,
                                      C.c_void_p, C.c_void_p]),
+    "cer_stream_stage": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                   C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cer_stream_gather": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                    C.c_void_p]),
+    "cer_stream_average": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "cer_stream_retain": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
+                                    C.c_void_p, C.c_void_p]),
 }
+
+# int32 fields of cer_stream_entry, in order
+STREAM_ENTRY_FIELDS = ("sid", "slot", "lslot", "start", "t_now", "parity", "active", "reserved")
 
 _lib: Optional[C.CDLL] = None
 

@@ -440,6 +440,58 @@ int cer_stitch_windows(const float* win_logits_dev, const int32_t* win_start_dev
 int cer_video_vote(const float* logits_dev, int64_t length, int32_t n_cls, int32_t ignore_last_class, int32_t* out_dev,
                    void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Streaming LFAN head (streaming.StreamSession).   Advances n live streams by c frames per step
+ * through the unchanged TCN (cer_tcn_block_tc_forward) and fusion (cer_fusion_head_forward)
+ * kernels; these calls hold the per-stream state around them.  A step is a fixed sequence of
+ * launches: the host writes one table of n * n_slots entries ([n][n_slots], each stream's active
+ * windows first, in start order) and copies it to the device once.
+ *
+ * Per stream the session keeps, for a k = 5 LFAN (halo h_b = 4 * 2^b, ring rows R_b = 2 h_b):
+ *   TCN rings   n_slots * 2 * sum_b R_b * C_in_pad(b) floats per modality (two halves, see stream.cu)
+ *   logit ring  n_lslots * W * n_out floats     (the last W frames of each window's logits)
+ *   input ring  W * D_m floats per modality     (the last W frames of each block-0 input)
+ * With W = 300, H = 200, c <= 101 (n_slots = 2, n_lslots = 3), n_out = 7 and video / vggish / bert
+ * TCNs of 512 -> [512,256,256,128], 128 -> [32,32,32,32], 768 -> [512,256,256,128] this comes to
+ * 3.00 MB per stream (2.63 MB with synthetic.TCN_CHANNELS); the input rings are 1.69 MB of it.
+ * streaming.StreamSession.state_bytes() computes it for a given model.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct {
+  int32_t sid;      /* persistent stream slot: row of every ring */
+  int32_t slot;     /* TCN ring slot of the window: window index mod n_slots */
+  int32_t lslot;    /* logit ring slot of the window: window index mod n_lslots */
+  int32_t start;    /* first frame of the window, in the stream's own frames */
+  int32_t t_now;    /* frames of the stream before this step */
+  int32_t parity;   /* TCN ring half read this step; the other half is written */
+  int32_t active;   /* 0: padding entry (staged as zeros, nothing written back) */
+  int32_t reserved;
+} cer_stream_entry;
+
+/* One TemporalBlock's staged input: staged [n_entries][ring_rows + chunk][c_pad] fp32, rows of
+ * frames max(start, t_now - ring_rows) + r.  Chunk rows come from src: src_len == 0: the chunk
+ * input [n_entries / n_slots][chunk][src_dim] (channels zero-padded to c_pad); else the previous
+ * block's output [n_entries][src_len][src_dim] staged with src_ring_rows (src_len = src_ring_rows
+ * + chunk).  Earlier rows come from ring [streams][n_slots][2][ring_rows][c_pad], whose other half
+ * receives the last ring_rows rows. */
+int cer_stream_stage(const cer_stream_entry* table_dev, int32_t n_entries, int32_t n_slots, int32_t chunk,
+                     int32_t ring_rows, int32_t c_pad, const float* src_dev, int32_t src_dim, int32_t src_len,
+                     int32_t src_ring_rows, float* ring_dev, float* staged_dev, void* stream);
+/* The chunk rows of the last block's output [n_entries][src_ring_rows + chunk][dim] ->
+ * dst [n_entries][chunk][dim] (rows before a window's start, and inactive entries, are zero). */
+int cer_stream_gather(const cer_stream_entry* table_dev, int32_t n_entries, int32_t chunk, const float* src_dev,
+                      int32_t src_ring_rows, int32_t dim, float* dst_dev, void* stream);
+/* win_logits [n_streams * n_slots][chunk][n_out] -> out [n_streams][chunk][n_out]: per frame the
+ * mean over the windows covering it, summed in start order (the arithmetic of cer_stitch_windows);
+ * each window's logits also go to logit_ring [streams][n_lslots][window_length][n_out] at its
+ * window-relative row. */
+int cer_stream_average(const cer_stream_entry* table_dev, int32_t n_streams, int32_t n_slots, int32_t chunk,
+                       int32_t window_length, int32_t n_out, const float* win_logits_dev, float* out_dev,
+                       float* logit_ring_dev, int32_t n_lslots, void* stream);
+/* The chunk input src [n_streams][chunk][dim] -> ring [streams][window_length][dim] at row
+ * frame mod window_length. */
+int cer_stream_retain(const cer_stream_entry* table_dev, int32_t n_streams, int32_t n_slots, int32_t chunk,
+                      const float* src_dev, int32_t dim, int32_t window_length, float* ring_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
