@@ -51,6 +51,11 @@ class VggishWeights(C.Structure):
                 ("n_fcs", C.c_int32), ("fcs", C.POINTER(VggFc)), ("zeros", C.c_void_p)]
 
 
+class VggishStep(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("layer", C.c_int32), ("h", C.c_int32), ("w", C.c_int32), ("c", C.c_int32),
+                ("out_fp32", C.c_int32), ("pool_fused", C.c_int32)]
+
+
 class TcnBlock(C.Structure):
     _fields_ = [("c_in", C.c_int32), ("c_out", C.c_int32), ("kernel_size", C.c_int32), ("dilation", C.c_int32),
                 ("w1", C.c_void_p), ("b1", C.c_void_p), ("w2", C.c_void_p), ("b2", C.c_void_p),
@@ -119,6 +124,9 @@ SIGNATURES = {
     "cer_vggish_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "cer_vggish_launches": (C.c_int64, [C.c_void_p, C.c_int64]),
     "cer_vggish_destroy": (None, [C.c_void_p]),
+    "cer_vggish_steps": (C.c_int32, [C.c_void_p, C.POINTER(VggishStep), C.c_int32]),
+    "cer_vggish_debug_activation": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "cer_vggish_op_variant": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_char_p, C.c_int32]),
     "cer_tcn_block_workspace_bytes": (C.c_size_t, [C.POINTER(TcnBlock), C.c_int64, C.c_int64]),
     "cer_tcn_block_forward": (C.c_int, [C.POINTER(TcnBlock), C.c_void_p, C.c_void_p, C.c_int64, C.c_int64,
                                         C.c_void_p, C.c_size_t, C.c_void_p]),

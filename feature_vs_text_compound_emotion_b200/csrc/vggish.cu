@@ -7,6 +7,7 @@
 #include <cuda_bf16.h>
 #include <algorithm>
 #include <cstdint>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -136,7 +137,8 @@ struct cer_vggish {
   int n_cap;
   int num_sms;
   uint8_t* buf[2];
-  struct Step { int kind; ConvOp op; int H, W, C; const void* src; void* dst; };   // kind 0: conv/fc, 1: pool
+  // kind 0: conv/fc, 1: pool (H, W, C: its input); desc: what cer_vggish_steps reports
+  struct Step { int kind; ConvOp op; int H, W, C; const void* src; void* dst; cer_vggish_step desc; };
   std::vector<Step> steps;
   int emb_dim;
 };
@@ -208,6 +210,7 @@ extern "C" int cer_vggish_create(cer_vggish** out, const cer_vggish_weights* w, 
     s.kind = 0;
     rc = build_conv_op(&s.op, g, p->n_cap);
     if (rc) { delete p; return rc; }
+    s.desc = {0, i, fuse_pool ? H / 2 : H, fuse_pool ? W / 2 : W, c.cout, 0, fuse_pool ? 1 : 0};
     p->steps.push_back(s);
     cur ^= 1;
     C = c.cout;
@@ -217,6 +220,7 @@ extern "C" int cer_vggish_create(cer_vggish** out, const cer_vggish_weights* w, 
       if ((H & 1) || (W & 1) || (C % 8)) { delete p; return set_error(CER_ERR_INVALID, "vggish: pool needs even H, W and C % 8 == 0"); }
       cer_vggish::Step ps{};
       ps.kind = 1; ps.H = H; ps.W = W; ps.C = C; ps.src = p->buf[cur]; ps.dst = p->buf[cur ^ 1];
+      ps.desc = {1, i, H / 2, W / 2, C, 0, 0};
       p->steps.push_back(ps);
       cur ^= 1;
       H /= 2; W /= 2;
@@ -235,12 +239,45 @@ extern "C" int cer_vggish_create(cer_vggish** out, const cer_vggish_weights* w, 
     s.kind = 0;
     rc = build_conv_op(&s.op, g, p->n_cap);
     if (rc) { delete p; return rc; }
+    s.desc = {2, i, 1, 1, f.out_dim, last ? 1 : 0, 0};
     p->steps.push_back(s);
     cur ^= 1;
     dim = f.out_dim;
   }
   p->emb_dim = dim;
   *out = p;
+  return CER_OK;
+}
+
+// One pass of n <= cap patches: the stem, then steps 0 .. last_step.  The last FC writes straight into emb_out.
+static int run_pass(cer_vggish* p, const float* x, int n, int last_step, float* emb_out, cudaStream_t st) {
+  const int H = p->w.in_h, W = p->w.in_w;
+  const long long pix = (long long)n * (H / 2) * (W / 2);
+  const int blocks = (int)std::min<long long>((pix + 127) / 128, (long long)p->num_sms * 16);
+  vgg_stem_pool_kernel<<<blocks, 128, 0, st>>>(x, p->w.conv1_w, p->w.conv1_bias, reinterpret_cast<__nv_bfloat16*>(p->buf[0]),
+                                               n, H, W);
+  CER_CUDA(cudaGetLastError());
+  for (size_t i = 0; i < p->steps.size() && (int)i <= last_step; ++i) {
+    const cer_vggish::Step& s = p->steps[i];
+    if (s.kind == 0) {
+      if (i + 1 == p->steps.size()) {       // the last FC writes straight into the caller's output
+        ConvOp op = s.op;
+        op.kp.out = emb_out;
+        int rc = launch_conv(op, n, p->num_sms, st);
+        if (rc) return rc;
+      } else {
+        int rc = launch_conv(s.op, n, p->num_sms, st);
+        if (rc) return rc;
+      }
+    } else {
+      const int C8 = s.C / 8;
+      const long long total = (long long)n * (s.H / 2) * (s.W / 2) * C8;
+      const int pb = (int)std::min<long long>((total + 255) / 256, (long long)p->num_sms * 32);
+      maxpool2x2_kernel<<<pb, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(s.src), static_cast<__nv_bfloat16*>(s.dst),
+                                            total, s.H, s.W, C8);
+      CER_CUDA(cudaGetLastError());
+    }
+  }
   return CER_OK;
 }
 
@@ -253,34 +290,49 @@ extern "C" int cer_vggish_forward(cer_vggish* p, const float* x, int64_t n_patch
   const int H = p->w.in_h, W = p->w.in_w;
   for (int64_t f0 = 0; f0 < n_patches; f0 += p->cap) {
     const int n = (int)std::min<int64_t>(p->cap, n_patches - f0);
-    const long long pix = (long long)n * (H / 2) * (W / 2);
-    const int blocks = (int)std::min<long long>((pix + 127) / 128, (long long)p->num_sms * 16);
-    vgg_stem_pool_kernel<<<blocks, 128, 0, st>>>(x + f0 * H * W, p->w.conv1_w, p->w.conv1_bias,
-                                                 reinterpret_cast<__nv_bfloat16*>(p->buf[0]), n, H, W);
-    CER_CUDA(cudaGetLastError());
-    for (size_t i = 0; i < p->steps.size(); ++i) {
-      const cer_vggish::Step& s = p->steps[i];
-      if (s.kind == 0) {
-        if (i + 1 == p->steps.size()) {       // the last FC writes straight into the caller's output
-          ConvOp op = s.op;
-          op.kp.out = emb_out + f0 * p->emb_dim;
-          int rc = launch_conv(op, n, p->num_sms, st);
-          if (rc) return rc;
-        } else {
-          int rc = launch_conv(s.op, n, p->num_sms, st);
-          if (rc) return rc;
-        }
-      } else {
-        const int C8 = s.C / 8;
-        const long long total = (long long)n * (s.H / 2) * (s.W / 2) * C8;
-        const int pb = (int)std::min<long long>((total + 255) / 256, (long long)p->num_sms * 32);
-        maxpool2x2_kernel<<<pb, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(s.src), static_cast<__nv_bfloat16*>(s.dst),
-                                              total, s.H, s.W, C8);
-        CER_CUDA(cudaGetLastError());
-      }
-    }
+    int rc = run_pass(p, x + f0 * H * W, n, (int)p->steps.size() - 1, emb_out + f0 * p->emb_dim, st);
+    if (rc) return rc;
   }
   return CER_OK;
+}
+
+extern "C" int32_t cer_vggish_steps(const cer_vggish* p, cer_vggish_step* out, int32_t max_steps) {
+  if (!p || max_steps < 0 || (max_steps > 0 && !out)) return set_error(CER_ERR_INVALID, "cer_vggish_steps: bad argument");
+  for (int i = 0; i < (int)p->steps.size() && i < max_steps; ++i) out[i] = p->steps[i].desc;
+  return (int32_t)p->steps.size();
+}
+
+extern "C" int64_t cer_vggish_debug_activation(cer_vggish* p, const float* x, int64_t n_patches, int32_t step, void* dst_dev,
+                                               void* stream) {
+  if (!p || !x || !dst_dev || n_patches <= 0 || n_patches > p->cap || step < -1 || step >= (int)p->steps.size())
+    return set_error(CER_ERR_INVALID, "cer_vggish_debug_activation: bad argument");
+  if (reinterpret_cast<uintptr_t>(x) % 4 || reinterpret_cast<uintptr_t>(dst_dev) % 16)
+    return set_error(CER_ERR_INVALID, "cer_vggish_debug_activation: dst must be 16B aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool last = step + 1 == (int)p->steps.size();
+  int rc = run_pass(p, x, (int)n_patches, step, last ? static_cast<float*>(dst_dev) : nullptr, st);
+  if (rc) return rc;
+  if (last) return n_patches * p->emb_dim;
+  int64_t elems = n_patches * (p->w.in_h / 2) * (p->w.in_w / 2) * p->w.c1;
+  const void* src = p->buf[0];
+  if (step >= 0) {
+    const cer_vggish::Step& s = p->steps[step];
+    elems = n_patches * s.desc.h * s.desc.w * s.desc.c;
+    src = s.kind == 0 ? s.op.kp.out : s.dst;
+  }
+  CER_CUDA(cudaMemcpyAsync(dst_dev, src, (size_t)elems * 2, cudaMemcpyDeviceToDevice, st));
+  return elems;
+}
+
+extern "C" int cer_vggish_op_variant(const cer_vggish* p, int32_t step, int64_t n_patches, char* buf, int32_t buflen) {
+  if (!p || !buf || buflen <= 0 || step < -1 || step >= (int)p->steps.size() || n_patches <= 0)
+    return set_error(CER_ERR_INVALID, "cer_vggish_op_variant: bad argument");
+  const int n = (int)std::min<int64_t>(p->cap, n_patches);
+  const char* name = step < 0 ? "vgg_stem_pool_kernel"
+                     : p->steps[step].kind == 1 ? "maxpool2x2_kernel"
+                                                : conv_variant_name(p->steps[step].op, n, p->num_sms);
+  const int len = snprintf(buf, (size_t)buflen, "%s", name);
+  return len < buflen ? len : buflen - 1;
 }
 
 extern "C" int64_t cer_vggish_launches(const cer_vggish* p, int64_t n_patches) {

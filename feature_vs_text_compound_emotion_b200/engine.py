@@ -11,7 +11,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import _capi
-from ._capi import FusionWeights, Ir50Weights, IrSe, IrUnit, TcnBlock, VggConv, VggFc, VggishWeights, check, lib
+from ._capi import FusionWeights, Ir50Weights, IrSe, IrUnit, TcnBlock, VggConv, VggFc, VggishStep, VggishWeights, check, lib
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -173,6 +173,15 @@ class VggishEngine:
             check(lib().cer_vggish_create(C.byref(h), C.byref(self._w), self.patches_per_pass, self._ws.data_ptr(), nbytes),
                   "cer_vggish_create")
         self._h = h
+        n_steps = check(lib().cer_vggish_steps(h, None, 0), "cer_vggish_steps")
+        desc = (VggishStep * n_steps)()
+        check(lib().cer_vggish_steps(h, desc, n_steps), "cer_vggish_steps")
+        # per plan step after the stem (cer_vggish_step): kind "conv" / "pool" / "fc", the index into packed["convs"] or
+        # packed["fcs"] (a pool: of the conv it follows), the per-patch output shape and dtype, and whether a conv's
+        # epilogue applied the following max-pool
+        self.step_shapes = [{"kind": ("conv", "pool", "fc")[d.kind], "layer": d.layer, "shape": (d.h, d.w, d.c),
+                             "dtype": torch.float32 if d.out_fp32 else torch.bfloat16, "pool_fused": bool(d.pool_fused)}
+                            for d in desc]
 
     def forward(self, x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         if x.dim() != 3 or x.shape[1] != self.in_h or x.shape[2] != self.in_w:
@@ -190,6 +199,29 @@ class VggishEngine:
 
     def launches(self, n: int) -> int:
         return int(lib().cer_vggish_launches(self._h, n))
+
+    def debug_activation(self, x: torch.Tensor, step: int) -> torch.Tensor:
+        """Output [n, h, w, c] of plan step ``step`` (-1: the stem's pooled bf16 map) for one pass over x's n <=
+        patches_per_pass patches; shape and dtype as in step_shapes."""
+        x = x.contiguous()
+        n = x.shape[0]
+        if step < 0:
+            shape, dtype = (self.in_h // 2, self.in_w // 2, self._w.c1), torch.bfloat16
+        else:
+            shape, dtype = self.step_shapes[step]["shape"], self.step_shapes[step]["dtype"]
+        dst = torch.empty(n, *shape, dtype=dtype, device=self.device)
+        with torch.cuda.device(self.device):
+            r = lib().cer_vggish_debug_activation(self._h, x.data_ptr(), n, step, dst.data_ptr(),
+                                                  _capi.current_stream_ptr(self.device))
+        check(int(r), "cer_vggish_debug_activation")
+        return dst
+
+    def op_variant(self, step: int, n_patches: int) -> str:
+        """Kernel instantiation plan step ``step`` launches (-1: the stem) when a pass holds min(n_patches,
+        patches_per_pass) patches."""
+        buf = C.create_string_buffer(96)
+        check(lib().cer_vggish_op_variant(self._h, step, n_patches, buf, 96), "cer_vggish_op_variant")
+        return buf.value.decode()
 
     def __del__(self):
         h = getattr(self, "_h", None)

@@ -174,6 +174,27 @@ int cer_vggish_forward(cer_vggish* plan, const float* x_dev, int64_t n_patches, 
 int64_t cer_vggish_launches(const cer_vggish* plan, int64_t n_patches);
 void cer_vggish_destroy(cer_vggish* plan);
 
+/* One step of the plan after the stem, in launch order (tests / inspection). */
+typedef struct cer_vggish_step {
+  int32_t kind;                   /* 0: convs[layer] (3x3 + ReLU), 1: the separate MaxPool2d(2,2) after convs[layer], 2: fcs[layer] */
+  int32_t layer;
+  int32_t h, w, c;                /* per-patch output: bf16 NHWC [h][w][c]; an FC is [1][1][out_dim]                    */
+  int32_t out_fp32;               /* 1: fp32 output (the last FC)                                                       */
+  int32_t pool_fused;             /* 1: a conv whose epilogue applies the following MaxPool2d(2,2) (h, w are pooled)   */
+} cer_vggish_step;
+/* Copies the first min(max_steps, n) step descriptors to `out` and returns n, the number of steps. */
+int32_t cer_vggish_steps(const cer_vggish* plan, cer_vggish_step* out, int32_t max_steps);
+/* Debug/inspection: one pass over `n_patches` (<= patches_per_pass) patches -- the stem, then steps 0 .. step --
+ * and a copy of that step's output to dst_dev (16 B aligned).  step = -1 is the stem's pooled bf16
+ * [n][in_h/2][in_w/2][c1]; the last step (the fp32 FC) writes dst_dev directly.  At n_patches = patches_per_pass
+ * the launches are exactly those of that cer_vggish_forward pass.  Returns the element count or a negative status. */
+int64_t cer_vggish_debug_activation(cer_vggish* plan, const float* x_dev, int64_t n_patches, int32_t step, void* dst_dev,
+                                    void* stream);
+/* Name of the kernel instantiation step `step` launches when a pass holds min(n_patches, patches_per_pass) patches:
+ * "vgg_stem_pool_kernel" for step -1, "maxpool2x2_kernel" for a separate pool, else a conv variant such as
+ * "conv_igemm2_kernel<256,6>".  Writes a NUL-terminated string, returns its length or a negative status. */
+int cer_vggish_op_variant(const cer_vggish* plan, int32_t step, int64_t n_patches, char* buf, int32_t buflen);
+
 /* ------------------------------------------------------------------------------------------
  * Log-mel front end of the inline-VGGish modality.   Replaces log_mel_spectrogram /
  * stft_magnitude / periodic_hann / spectrogram_to_mel_matrix (abaw5_pre_processing/base/vggish/

@@ -71,6 +71,47 @@ def bound_ratio(got, ref, E=None, c=C_RMS):
     return torch.nan_to_num((got - ref).abs() / bound, nan=float("inf"))
 
 
+def vggish_stem(pk, x):
+    """VGGish features.0-2 from the packed fp32 weights, in x's dtype: x [N,H,W] -> maxpool2(relu(conv3x3(x) + b))
+    [N,64,H/2,W/2] (NCHW).  The fp32 weights and inputs are exact in fp64."""
+    w = pk["conv1_w"].to(x.device, x.dtype).view(3, 3, -1).permute(2, 0, 1).unsqueeze(1)     # [(r,s)][co] -> [co,1,r,s]
+    z = F.conv2d(x.unsqueeze(1), w, pk["conv1_bias"].to(x.device, x.dtype), 1, 1)
+    return F.max_pool2d(torch.relu(z), 2)
+
+
+def vggish_conv(c, h, pool):
+    """One packed VGGish conv in h's dtype: h [N,cin,H,W] (the bf16 values the previous step stored) ->
+    relu(conv3x3(h, w) + b), max-pooled 2x2 if `pool`.  One rounding (to bf16) follows the fp32 accumulation, so
+    the bound needs no envelope (E = 0); max commutes with that monotone rounding, and with ReLU every pooled value
+    bounds the other three of its window, so the pooled output keeps the same bound."""
+    cin, cout = c["cin"], c["cout"]
+    w = c["w"].to(h.device, h.dtype).view(cout, 3, 3, cin).permute(0, 3, 1, 2)
+    y = torch.relu(F.conv2d(h, w, c["bias"].to(h.device, h.dtype), 1, 1))
+    return F.max_pool2d(y, 2) if pool else y
+
+
+def vggish_fc(f, a):
+    """One packed VGGish FC in a's dtype: a [N,in_dim] (the NHWC flatten of the previous step) -> a w^T + b, ReLU if
+    f["relu"]."""
+    y = F.linear(a, f["w"].to(a.device, a.dtype), f["bias"].to(a.device, a.dtype))
+    return torch.relu(y) if f["relu"] else y
+
+
+# The last FC stores fp32: |got - ref| <= FC_DOT_C (|a| |w|^T + |b|), a bound on reordering an fp32 dot product.
+# 2^-14 is the ceiling at which one dropped 64-wide K chunk of a 4096-long dot product still fails it
+# (tests/test_vggish_parity_guards.py keeps both sides of that honest).
+FC_DOT_C = 2.0 ** -14
+
+
+def fc_dot_ratio(got, a, f, c=FC_DOT_C):
+    """Elementwise |got - vggish_fc(f, a)| / (c (|a| |w|^T + |b|)), computed in a's dtype; NaN counts as inf."""
+    w = f["w"].to(a.device, a.dtype)
+    b = f["bias"].to(a.device, a.dtype)
+    ref = vggish_fc(f, a)
+    bound = c * (a.abs() @ w.abs().t() + b.abs())
+    return torch.nan_to_num((got.to(a.dtype) - ref).abs() / bound, nan=float("inf"))
+
+
 def ir50_packed(pk, x, round_act=True, upto=None):
     """x: [N,3,H,W] fp32 -> (emb [N,512], dict of unit outputs NHWC)."""
     N, _, H, W = x.shape

@@ -120,6 +120,7 @@ def test_struct_sizes_match_header_layout():
     assert ctypes.sizeof(_capi.IrUnit) == 16 + 5 * 8
     assert ctypes.sizeof(_capi.TcnBlock) == 16 + 8 * 8
     assert ctypes.sizeof(_capi.Ir50Weights) == 8 + 3 * 8 + 8 + 8 + 8 + 2 * 8
+    assert ctypes.sizeof(_capi.VggishStep) == 7 * 4
 
 
 def test_alternative_head_layouts_equal_reference(golden_dir):

@@ -85,9 +85,12 @@ def _selectable_variants():
 def test_every_conv_variant_has_a_parity_case():
     from tests.test_gpu_ir50_layers import PLAN_CASES
     from tests.test_gpu_kernels import CONV_CASES, PADDED_CASES
+    from tests import test_gpu_vggish_layers as vgg
     pinned = {c[-1] for c in CONV_CASES} | {c[-1] for _, c in PADDED_CASES}
     for case in PLAN_CASES:
         pinned |= case["variants"]
+    for case in vgg.PLAN_CASES:
+        pinned |= {v for _, v, _ in case["variants"]} - {vgg.STEM, vgg.POOL}
     selectable = _selectable_variants()
     assert selectable == pinned, (f"without a parity case: {sorted(selectable - pinned)}; "
                                   f"not a kernel of ir50.cu: {sorted(pinned - selectable)}")
