@@ -171,6 +171,10 @@ SIGNATURES = {
     "cer_logmel_forward": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double,
                                      C.c_void_p, C.c_void_p]),
     "cer_frame_examples": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "cer_stream_logmel": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                    C.c_int32, C.c_double, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "cer_stream_examples": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                      C.c_void_p]),
     "cer_linear_forward": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                      C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_softmax_gate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
@@ -200,6 +204,9 @@ SIGNATURES = {
 
 # int32 fields of cer_stream_entry, in order
 STREAM_ENTRY_FIELDS = ("sid", "slot", "lslot", "start", "t_now", "parity", "active", "reserved")
+# cer_stream_audio_entry, in order (int32 x4, then int64 x3)
+STREAM_AUDIO_ENTRY_FIELDS = (("slot", "<i4"), ("first_row", "<i4"), ("n_rows", "<i4"), ("reserved", "<i4"),
+                             ("a0", "<i8"), ("src_off", "<i8"), ("n_new", "<i8"))
 
 _lib: Optional[C.CDLL] = None
 

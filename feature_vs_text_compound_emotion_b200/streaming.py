@@ -22,13 +22,16 @@ unchanged; csrc/stream.cu holds the per-stream state around them (DESIGN.md sect
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
+from fractions import Fraction
 from typing import Dict, List, Sequence, Tuple
 
 import numpy as np
 import torch
 
 from . import _capi
+from .packing import LOGMEL, logmel_tables
 from .windowing import gather_windows, preprocess_frames, window_starts
 
 
@@ -93,6 +96,93 @@ def step_table(streams: Sequence[Tuple[int, int, int]], chunk: int, window_lengt
 
 
 # ----------------------------------------------------------------------------------------------
+# Audio bookkeeping of a session opened with wave_fps (pure host logic; DESIGN.md section 5.17)
+# ----------------------------------------------------------------------------------------------
+def example_grid(fps: float) -> Tuple[int, float]:
+    """(log-mel rows per VGGish example, rows between example starts) at ``fps``: the expressions of
+    LogMelEngine.examples(wave, 0.96, 1 / fps), so that every start below is the offline one."""
+    rate = 1.0 / (LOGMEL["hop"] / LOGMEL["sample_rate"])
+    return int(round(0.96 * rate)), (1.0 / fps) * rate
+
+
+def example_start(t: int, fps: float) -> int:
+    """First log-mel row of frame t's example (Python round, as my_frame)."""
+    return round(example_grid(fps)[1] * t)
+
+
+def logmel_rows(n_samples: int) -> int:
+    """Complete STFT rows of ``n_samples`` samples (cer_logmel_num_frames)."""
+    win, hop = LOGMEL["win"], LOGMEL["hop"]
+    return 0 if n_samples < win else 1 + (n_samples - win) // hop
+
+
+def example_samples(t: int, fps: float) -> int:
+    """Samples after which frame t's example is complete: its last row, s_t + 95, needs hop * (s_t + 95) + win."""
+    rows = example_grid(fps)[0]
+    return LOGMEL["hop"] * (example_start(t, fps) + rows - 1) + LOGMEL["win"]
+
+
+def frames_ready(n_samples: int, fps: float) -> int:
+    """Number of leading frames whose example is complete after ``n_samples`` samples."""
+    rows, step = example_grid(fps)
+    if n_samples < example_samples(0, fps):
+        return 0
+    t = int((logmel_rows(n_samples) - rows) / step) + 1            # estimate, then settle on the exact count
+    while t > 0 and example_samples(t - 1, fps) > n_samples:
+        t -= 1
+    while example_samples(t, fps) <= n_samples:
+        t += 1
+    return t
+
+
+def stream_lag(fps: float) -> int:
+    """The fixed lag L of a wave stream: with audio in step with the video (floor(T * sr / fps) samples after T
+    frames), frame T - L's example is complete.  Its last sample is hop * (s + rows - 1) + win with
+    s <= hop_rows * (T - L) + 1/2, so L = ceil((hop * (rows - 1) + win + hop / 2 + 1) * fps / sr) suffices
+    (the + 1 covers the floor)."""
+    rows = example_grid(fps)[0]
+    need = LOGMEL["hop"] * (rows - 1) + LOGMEL["win"] + Fraction(LOGMEL["hop"], 2) + 1
+    return math.ceil(need * Fraction(fps) / LOGMEL["sample_rate"])
+
+
+def synced_samples(frames: int, fps: float) -> int:
+    """Samples of audio in step with ``frames`` video frames."""
+    return math.floor(frames * LOGMEL["sample_rate"] / fps)
+
+
+def released_upto(frames: int, n_samples: int, emitted: int, lag: int, fps: float) -> int:
+    """Frames released once a stream has ``frames`` frames and ``n_samples`` samples and had released ``emitted``:
+    frames [emitted, result) go through the head now."""
+    return max(emitted, min(frames - lag, frames_ready(n_samples, fps)))
+
+
+def n_examples_total(lm_rows: int, fps: float) -> int:
+    """Examples of a log-mel of ``lm_rows`` rows (LogMelEngine.examples' count); frames at or above it reuse the last."""
+    rows, step = example_grid(fps)
+    return 1 + int(math.floor((lm_rows - rows) / step)) if lm_rows >= rows else 0
+
+
+def flush_schedule(emitted: int, frames: int, max_chunk: int) -> List[Tuple[int, int]]:
+    """(first frame, count) of the head steps that release frames [emitted, frames), at most max_chunk each."""
+    return [(a, min(max_chunk, frames - a)) for a in range(emitted, frames, max_chunk)]
+
+
+def hold_rows(lag: int, max_chunk: int) -> int:
+    """Ring rows of held-back non-audio features: up to lag + 2 * max_chunk unreleased frames after a push, plus
+    the chunk being pushed, which is stored before the frames it releases are gathered."""
+    return lag + 3 * max_chunk
+
+
+def logmel_ring_rows(lag: int, max_chunk: int, fps: float) -> int:
+    """Log-mel ring rows per stream.  During a push the rows in use run from the example start of the oldest
+    unreleased frame (>= T - lag - 3 * max_chunk) to the rows of audio at most lag + max_chunk frames ahead of T:
+    fewer than (2 lag + 4 max_chunk) hop_rows rows.  close adds one second (100 rows) of padding and may reuse the
+    example before the oldest unreleased frame (one more frame)."""
+    step = example_grid(fps)[1]
+    return math.ceil((2 * lag + 4 * max_chunk + 1) * step) + LOGMEL["sample_rate"] // LOGMEL["hop"] + 1
+
+
+# ----------------------------------------------------------------------------------------------
 # Session
 # ----------------------------------------------------------------------------------------------
 class StreamSession:
@@ -101,10 +191,17 @@ class StreamSession:
     Per push input (n streams, c frames each): 'video' as stored uint8 crops [n, c, H, W, 3] or fp32
     [n, c, 3, 40, 40]; 'logmel' as VGGish examples [n, c, 96, 64]; a pre-extracted modality as [n, c, D_m].
     One push is one backbone pass over the n * c frames and one fixed sequence of head launches (captured as a
-    CUDA graph per (n, c), like LFAN.forward_features; eager when capture is off or fails)."""
+    CUDA graph per (n, c), like LFAN.forward_features; eager when capture is off or fails).
+
+    With ``wave_fps`` set (a model with 'logmel' and at least one other modality), a push carries 'wave' instead
+    of 'logmel': a sequence of n 1-D fp32 tensors on the session's device, each stream's next 16 kHz samples (any
+    number, 0 included).  The session computes the log-mel rows as their samples arrive (cer_stream_logmel) and
+    holds each frame back until its 0.96 s example is complete and it is ``lag`` frames old; ``push`` then returns
+    one [r_i, n_out] tensor per stream for the frames it released, and ``close`` flushes the rest with the
+    offline edge padding, so the examples are windowing.wave_to_examples' (DESIGN.md section 5.17)."""
 
     def __init__(self, model, max_streams: int = 256, max_chunk: int = 30, window_length: int = 300,
-                 hop_length: int = 200):
+                 hop_length: int = 200, wave_fps: float = None):
         from .modules import LFAN
         if not isinstance(model, LFAN):
             raise TypeError("StreamSession streams LFAN only: the CAN / JMT / MT heads are not streamed (JMT / MT attend "
@@ -123,10 +220,38 @@ class StreamSession:
         self.modalities = list(model.modality)
         self.device = model.regressor.weight.device
         self._len: Dict[int, int] = {}
+        self._emitted: Dict[int, int] = {}
         self._parity: Dict[int, int] = {}
         self._free = list(range(self.max_streams - 1, -1, -1))
         self._eng = None
         self._pack()
+        self.wave_fps = None if wave_fps is None else float(wave_fps)
+        self.example_hook = None       # called as hook([(sid, first frame, count)], examples) before each VGGish pass
+        if self.wave_fps is not None:
+            self._init_wave()
+
+    def _init_wave(self):
+        if "logmel" not in self.modalities or len(self.modalities) < 2:
+            raise ValueError("wave_fps needs a model with the 'logmel' modality and at least one other (which gives "
+                             f"the frame count of a push), got {self.modalities}")
+        if not self.wave_fps > 0:
+            raise ValueError(f"wave_fps must be positive, got {self.wave_fps}")
+        fps, S, dev = self.wave_fps, self.max_streams, self.device
+        self.lag = stream_lag(fps)
+        self.max_unreleased = self.lag + 2 * self.max_chunk
+        self.max_ahead = self.lag + self.max_chunk
+        self.example_rows = example_grid(fps)[0]
+        self.n_lm_rows = logmel_ring_rows(self.lag, self.max_chunk, fps)
+        self.n_hold = hold_rows(self.lag, self.max_chunk)
+        self.tail_len = LOGMEL["win"] - 1
+        self._samples: Dict[int, int] = {}
+        self._lm_tables = logmel_tables(LOGMEL).to(dev)
+        self._tails = torch.zeros(S, self.tail_len, dtype=torch.float32, device=dev)
+        self._lmring = torch.zeros(S, self.n_lm_rows, LOGMEL["n_mel"], dtype=torch.float32, device=dev)
+        self._atab = torch.zeros(S * np.dtype(list(_capi.STREAM_AUDIO_ENTRY_FIELDS)).itemsize, dtype=torch.uint8,
+                                 device=dev)
+        self._hold = {m: torch.zeros(S, self.n_hold, self._inring[m].shape[-1], dtype=torch.float32, device=dev)
+                      for m in self.modalities if m != "logmel"}
 
     # -- state ------------------------------------------------------------------------------
     def _check_model(self):
@@ -177,6 +302,8 @@ class StreamSession:
         for m in self.modalities:
             n += self.W * self._inring[m].shape[-1]
             n += sum(self.n_slots * 2 * r * b.c_in for b, r in zip(self._blocks[m], self._rows[m]))
+        if self.wave_fps is not None:
+            n += self.tail_len + self.n_lm_rows * LOGMEL["n_mel"] + sum(h.shape[1] * h.shape[2] for h in self._hold.values())
         return 4 * n
 
     def open(self) -> int:
@@ -184,19 +311,26 @@ class StreamSession:
         if not self._free:
             raise RuntimeError(f"all {self.max_streams} stream slots are open")
         sid = self._free.pop()
-        self._len[sid], self._parity[sid] = 0, 0
+        self._len[sid], self._emitted[sid], self._parity[sid] = 0, 0, 0
+        if self.wave_fps is not None:
+            self._samples[sid] = 0
         return sid
 
     def length(self, sid: int) -> int:
+        """Frames pushed to stream ``sid``."""
         return self._len[sid]
 
+    def emitted(self, sid: int) -> int:
+        """Frames of stream ``sid`` whose provisional logits were returned (== length without wave_fps)."""
+        return self._emitted[sid]
+
     # -- push -------------------------------------------------------------------------------
-    def _chunk_features(self, inputs: Dict[str, torch.Tensor], n: int) -> Tuple[int, Dict[str, torch.Tensor]]:
+    def _chunk_features(self, inputs: Dict[str, torch.Tensor], n: int, mods=None) -> Tuple[int, Dict[str, torch.Tensor]]:
         if "wave" in inputs:
             raise ValueError("'wave' cannot be streamed: the VGGish example of a frame needs 0.96 s of audio after it; "
-                             "push 'logmel' examples [n, c, 96, 64] instead")
+                             "push 'logmel' examples [n, c, 96, 64] instead, or open the session with wave_fps")
         chunk, out = None, {}
-        for m in self.modalities:
+        for m in mods or self.modalities:
             if m not in inputs:
                 raise KeyError(f"push needs the '{m}' input")
             x = inputs[m]
@@ -256,7 +390,10 @@ class StreamSession:
 
     @torch.no_grad()
     def push(self, ids: Sequence[int], inputs: Dict[str, torch.Tensor]) -> Tuple[torch.Tensor, List[int]]:
-        """Advance streams ``ids`` by c frames -> (provisional logits [n, c, n_out], final_upto per stream)."""
+        """Advance streams ``ids`` by c frames -> (provisional logits [n, c, n_out], final_upto per stream).
+
+        With wave_fps: -> (a list of n tensors [r_i, n_out], the provisional logits of the frames this push
+        released, continuing from emitted(i); final_upto = max(0, emitted(i) - W) per stream)."""
         self._check_model()
         ids = [int(i) for i in ids]
         n = len(ids)
@@ -265,36 +402,171 @@ class StreamSession:
         if len(set(ids)) != n or any(i not in self._len for i in ids):
             raise ValueError(f"stream ids must be distinct open streams, got {ids}")
         self._engines()
+        if self.wave_fps is not None:
+            return self._push_wave(ids, inputs)
         with torch.cuda.device(self.device):
             c, x = self._chunk_features(inputs, n)
             for m in self.modalities:
                 d = self._inring[m].shape[-1]
                 if x[m].shape[1] != d:
                     raise ValueError(f"'{m}': expected {d} features per frame, got {x[m].shape[1]}")
-                self._in[m][:n * c * d].view(n * c, d).copy_(x[m])
-            tab = step_table([(i, self._len[i], self._parity[i]) for i in ids], c, self.W, self.H, self.n_slots,
-                             self.n_lslots)
-            self._tab[:tab.shape[0]].copy_(torch.from_numpy(tab).pin_memory(), non_blocking=True)
-            g = self._graphs.get((n, c)) if self._use_graph() else False
-            if g:
-                g.replay()
-            else:
-                # capture records the launches without running them: the eager run is this step's
-                self._run_head(n, c)
-                if g is None:
-                    try:
-                        graph = torch.cuda.CUDAGraph()
-                        torch.cuda.synchronize(self.device)
-                        with torch.cuda.graph(graph):
-                            self._run_head(n, c)
-                        self._graphs[(n, c)] = graph
-                    except Exception:                     # capture not possible here: stay eager for this shape
-                        self._graphs[(n, c)] = False
-            out = self._out[:n * c * self.n_out].view(n, c, self.n_out).clone()
+            out = self._head_step(ids, c, x)
         for i in ids:
             self._len[i] += c
-            self._parity[i] ^= 1
         return out, [final_upto(self._len[i], self.W) for i in ids]
+
+    def _head_step(self, ids: List[int], c: int, x: Dict[str, torch.Tensor]) -> torch.Tensor:
+        """Frames emitted(i) .. emitted(i) + c - 1 of streams ``ids`` (features x[m] [n * c, D_m]) through the head
+        -> their provisional logits [n, c, n_out]; advances emitted and the TCN ring parity of those streams."""
+        n = len(ids)
+        for m in self.modalities:
+            d = self._inring[m].shape[-1]
+            self._in[m][:n * c * d].view(n * c, d).copy_(x[m])
+        tab = step_table([(i, self._emitted[i], self._parity[i]) for i in ids], c, self.W, self.H, self.n_slots,
+                         self.n_lslots)
+        self._tab[:tab.shape[0]].copy_(torch.from_numpy(tab).pin_memory(), non_blocking=True)
+        g = self._graphs.get((n, c)) if self._use_graph() else False
+        if g:
+            g.replay()
+        else:
+            # capture records the launches without running them: the eager run is this step's
+            self._run_head(n, c)
+            if g is None:
+                try:
+                    graph = torch.cuda.CUDAGraph()
+                    torch.cuda.synchronize(self.device)
+                    with torch.cuda.graph(graph):
+                        self._run_head(n, c)
+                    self._graphs[(n, c)] = graph
+                except Exception:                     # capture not possible here: stay eager for this shape
+                    self._graphs[(n, c)] = False
+        out = self._out[:n * c * self.n_out].view(n, c, self.n_out).clone()
+        for i in ids:
+            self._emitted[i] += c
+            self._parity[i] ^= 1
+        return out
+
+    # -- wave streams -------------------------------------------------------------------------
+    def _front_end(self, work: List[Tuple[int, int, torch.Tensor]]) -> None:
+        """Append samples to streams: work = (sid, samples received before, new fp32 samples on the device).
+        Computes every newly complete log-mel row into the ring and advances the tails (cer_stream_logmel)."""
+        work = [w for w in work if w[2].numel() > 0]
+        if not work:
+            return
+        tab = np.zeros(len(work), dtype=np.dtype(list(_capi.STREAM_AUDIO_ENTRY_FIELDS)))
+        off = 0
+        for k, (sid, a0, w) in enumerate(work):
+            r0, r1 = logmel_rows(a0), logmel_rows(a0 + w.numel())
+            tab[k] = (sid, r0, r1 - r0, 0, a0, off, w.numel())
+            off += w.numel()
+        samples = torch.cat([w for _, _, w in work]) if len(work) > 1 else work[0][2].contiguous()
+        raw = torch.from_numpy(tab.view(np.uint8)).pin_memory()
+        self._atab[:raw.numel()].copy_(raw, non_blocking=True)
+        c = LOGMEL
+        _capi.check(_capi.lib().cer_stream_logmel(
+            self._atab.data_ptr(), len(work), int(tab["n_rows"].max()), samples.data_ptr(), self._lm_tables.data_ptr(),
+            c["win"], c["hop"], c["fft"], c["n_mel"], c["log_offset"], self._tails.data_ptr(), self.tail_len,
+            self._lmring.data_ptr(), self.n_lm_rows, _capi.current_stream_ptr(self.device)), "cer_stream_logmel")
+
+    def _release(self, rel: List[Tuple[int, int, int, int]]) -> Dict[int, List[torch.Tensor]]:
+        """Release frames through the head: rel = (sid, first frame == emitted(sid), count, examples available or 0
+        for all).  One VGGish pass over every released example, then per group of streams with the same count one
+        head step per max_chunk frames.  Returns sid -> the provisional logits of its steps, in frame order."""
+        rel = [r for r in rel if r[2] > 0]
+        outs: Dict[int, List[torch.Tensor]] = {}
+        if not rel:
+            return outs
+        ex_rows, base, off = [], {}, 0
+        for sid, e0, r, n_ex in rel:
+            base[sid] = off
+            for t in range(e0, e0 + r):
+                ex_rows.append((sid, example_start(min(t, n_ex - 1) if n_ex else t, self.wave_fps), off))
+                off += 1
+        ent = torch.tensor(ex_rows, dtype=torch.int32).pin_memory().to(self.device, non_blocking=True)
+        ex = torch.empty(off, self.example_rows, LOGMEL["n_mel"], dtype=torch.float32, device=self.device)
+        _capi.check(_capi.lib().cer_stream_examples(self._lmring.data_ptr(), self.n_lm_rows, ent.data_ptr(), off,
+                                                    self.example_rows, LOGMEL["n_mel"], ex.data_ptr(),
+                                                    _capi.current_stream_ptr(self.device)), "cer_stream_examples")
+        if self.example_hook is not None:
+            self.example_hook([(sid, e0, r) for sid, e0, r, _ in rel], ex)
+        emb = self.model.spatial["audio"](ex)
+        groups: Dict[int, List[Tuple[int, int]]] = {}
+        for sid, e0, r, _ in rel:
+            groups.setdefault(r, []).append((sid, e0))
+        for r, members in groups.items():
+            ids = [sid for sid, _ in members]
+            for a, cc in flush_schedule(0, r, self.max_chunk):
+                rows = [(sid, e0 + a + k, base[sid] + a + k) for sid, e0 in members for k in range(cc)]
+                idx = torch.tensor([[sid * self.n_hold + f % self.n_hold, j] for sid, f, j in rows],
+                                   dtype=torch.int64).pin_memory().to(self.device, non_blocking=True)
+                x = {m: (emb.index_select(0, idx[:, 1]) if m == "logmel" else
+                         self._hold[m].view(-1, self._hold[m].shape[-1]).index_select(0, idx[:, 0]))
+                     for m in self.modalities}
+                out = self._head_step(ids, cc, x)
+                for j, sid in enumerate(ids):
+                    outs.setdefault(sid, []).append(out[j])
+        return outs
+
+    def _push_wave(self, ids: List[int], inputs) -> Tuple[List[torch.Tensor], List[int]]:
+        n, others = len(ids), [m for m in self.modalities if m != "logmel"]
+        if "logmel" in inputs:
+            raise ValueError("a session opened with wave_fps takes 'wave', not 'logmel': push one or the other")
+        if "wave" not in inputs:
+            raise KeyError("push needs the 'wave' input: a sequence of one 1-D fp32 tensor of new samples per stream")
+        waves = list(inputs["wave"])
+        if len(waves) != n:
+            raise ValueError(f"'wave': expected {n} tensors (one per stream), got {len(waves)}")
+        for w in waves:
+            if not isinstance(w, torch.Tensor) or w.dim() != 1 or w.dtype != torch.float32 or w.device != self.device:
+                raise ValueError(f"'wave': every stream's samples must be a 1-D fp32 tensor on {self.device}")
+        for m in others:
+            if m not in inputs:
+                raise KeyError(f"push needs the '{m}' input")
+        x0 = inputs[others[0]]
+        c = int(x0.shape[1]) if x0.dim() >= 2 else 0
+        if not 1 <= c <= self.max_chunk:
+            raise ValueError(f"chunk of {c} frames: need 1..{self.max_chunk}")
+        plan = []
+        for sid, w in zip(ids, waves):                    # the bounds, before any state changes
+            T1, A1 = self._len[sid] + c, self._samples[sid] + w.numel()
+            limit = synced_samples(T1 + self.max_ahead, self.wave_fps)
+            if A1 > limit:
+                raise ValueError(f"stream {sid}: audio may run ahead of the video by at most {self.max_ahead} frames "
+                                 f"(lag + max_chunk): {A1} samples after {T1} frames, at most {limit}")
+            E1 = released_upto(T1, A1, self._emitted[sid], self.lag, self.wave_fps)
+            if T1 - E1 > self.max_unreleased:
+                raise ValueError(f"stream {sid}: at most {self.max_unreleased} frames (lag + 2 * max_chunk) may wait "
+                                 f"for their audio, {T1 - E1} would: push more audio")
+            plan.append((sid, self._emitted[sid], E1 - self._emitted[sid]))
+        with torch.cuda.device(self.device):
+            _, x = self._chunk_features({m: inputs[m] for m in others}, n, others)
+            for m in others:
+                d = self._hold[m].shape[-1]
+                if x[m].shape[1] != d:
+                    raise ValueError(f"'{m}': expected {d} features per frame, got {x[m].shape[1]}")
+            self._front_end([(sid, self._samples[sid], w) for sid, w in zip(ids, waves)])
+            for sid, w in zip(ids, waves):
+                self._samples[sid] += w.numel()
+            idx = torch.tensor([sid * self.n_hold + (self._len[sid] + k) % self.n_hold for sid in ids for k in range(c)],
+                               dtype=torch.int64).pin_memory().to(self.device, non_blocking=True)
+            for m in others:
+                self._hold[m].view(-1, self._hold[m].shape[-1]).index_copy_(0, idx, x[m])
+            for sid in ids:
+                self._len[sid] += c
+            outs = self._release([(sid, e0, r, 0) for sid, e0, r in plan])
+            empty = torch.empty(0, self.n_out, dtype=torch.float32, device=self.device)
+            res = [torch.cat(outs[sid]) if sid in outs else empty for sid in ids]
+        return res, [final_upto(self._emitted[i], self.W) for i in ids]
+
+    def _flush_wave(self, sid: int) -> None:
+        """close: one second of the last sample (wave_to_examples' edge padding), the remaining log-mel rows, and the
+        held-back frames through the head; frames at or above the example count reuse the last example."""
+        A, T, E = self._samples[sid], self._len[sid], self._emitted[sid]
+        pad = self._tails[sid, -1:].expand(LOGMEL["sample_rate"]).contiguous()
+        self._front_end([(sid, A, pad)])
+        self._samples[sid] = A + pad.numel()
+        n_ex = n_examples_total(logmel_rows(A + pad.numel()), self.wave_fps)
+        self._release([(sid, E, T - E, n_ex)])
 
     # -- close ------------------------------------------------------------------------------
     @torch.no_grad()
@@ -306,8 +578,16 @@ class StreamSession:
             raise ValueError(f"stream {sid} is not open")
         self._check_model()
         self._engines()
+        if self.wave_fps is not None and self._len[sid] > 0:
+            if self._samples[sid] == 0:
+                raise ValueError(f"stream {sid} received no audio: its frames have no VGGish example (offline, "
+                                 "wave_to_examples fails on an empty waveform the same way)")
+            with torch.cuda.device(self.device):
+                self._flush_wave(sid)
         T, W = self._len.pop(sid), self.W
-        del self._parity[sid]
+        del self._parity[sid], self._emitted[sid]
+        if self.wave_fps is not None:
+            del self._samples[sid]
         self._free.append(sid)
         if T == 0:
             return torch.empty(0, self.n_out, dtype=torch.float32, device=self.device)

@@ -212,6 +212,32 @@ int cer_logmel_forward(const float* wave_dev, int64_t n_samples, const double* t
 int cer_frame_examples(const float* logmel_dev, const int32_t* starts_dev, int32_t n_examples, int32_t frames_per_example,
                        int32_t n_mel, float* out_dev, void* stream);
 
+/* Streaming form (streaming.StreamSession with wave_fps): the newly complete rows of n streams in one
+ * call, each computed by the body of cer_logmel_forward, so a row is bit-identical however the
+ * samples were split across calls.  One entry per stream with new samples or rows: */
+typedef struct {
+  int32_t slot;       /* stream slot: row of tails and ring */
+  int32_t first_row;  /* first new log-mel row (rows before it were computed by earlier calls) */
+  int32_t n_rows;     /* new rows: every row whose win samples are now all present */
+  int32_t reserved;
+  int64_t a0;         /* samples the stream received before this call */
+  int64_t src_off;    /* offset of its new samples in samples_dev */
+  int64_t n_new;      /* number of new samples (may be 0) */
+} cer_stream_audio_entry;
+/* table_dev [n_entries]; max_rows >= every n_rows.  tails_dev [streams][tail_len] holds each
+ * stream's samples a0 - tail_len .. a0 - 1 (tail_len >= win - 1: a call can end anywhere inside a
+ * hop) and is advanced by n_new; row f of a stream goes to ring_dev [streams][ring_rows][n_mel] at
+ * row f % ring_rows (of more new rows than ring_rows, only the last ring_rows are computed).
+ * tables_dev as for cer_logmel_forward. */
+int cer_stream_logmel(const cer_stream_audio_entry* table_dev, int32_t n_entries, int32_t max_rows, const float* samples_dev,
+                      const double* tables_dev, int32_t win, int32_t hop, int32_t fft, int32_t n_mel, double log_offset,
+                      float* tails_dev, int32_t tail_len, float* ring_dev, int32_t ring_rows, void* stream);
+/* entries_dev int32 [n_examples][3] = (slot, start_row, dst): out[dst][t][:] =
+ * ring[slot][(start_row + t) % ring_rows][:], t < frames_per_example (the ring form of
+ * cer_frame_examples). */
+int cer_stream_examples(const float* ring_dev, int32_t ring_rows, const int32_t* entries_dev, int32_t n_examples,
+                        int32_t frames_per_example, int32_t n_mel, float* out_dev, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * One TemporalBlock, fused.   Replaces TemporalBlock.forward
  * (models/temporal_convolutional_model.py:21-54): weight-normed dilated Conv1d + Chomp1d +

@@ -14,6 +14,15 @@ stream slots and chunks up to 30 frames.
 3. windowing.infer_videos on the same frames (n = 32 videos of the frames one stream would see), measured in the
    same run.
 Weights and inputs are synthetic and seeded; timing only (the numerics are tests/test_gpu_streaming.py's).
+
+    python tools/stream_bench.py --audio wave --out profiles/r05_stream_audio.json
+
+streams raw audio instead (DESIGN.md section 5.17): 'video' + 'logmel' computed from the waveform + 'bert', a session
+with wave_fps = 30 and every push carrying the samples in step with its frames, so each push releases c frames once
+warmed up.  The profiled run splits kernel time into IR-50 and preprocessing / VGGish / log-mel front end
+(cer_stream_logmel, cer_stream_examples) / head; VGGish is timed with CUDA events around its calls in that run (its
+convolutions are the IR-50 kernels, so kernel names cannot tell them apart) and IR-50 and preprocessing are the rest of
+the backbone kernel time.  infer_videos is not run in this mode.
 """
 from __future__ import annotations
 
@@ -31,6 +40,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from feature_vs_text_compound_emotion_b200 import streaming, synthetic, windowing  # noqa: E402
 
 HEAD_KERNELS = ("tcn_", "fusion_", "stream_")
+FRONT_END_KERNELS = ("stream_logmel", "stream_tail", "stream_examples")
 GC_RUNS = [0]
 gc.callbacks.append(lambda phase, info: GC_RUNS.__setitem__(0, GC_RUNS[0] + (phase == "start")))
 MODS = ["video", "vggish", "bert"]
@@ -48,21 +58,42 @@ def card():
     return info
 
 
-def lfan(dev):
+def lfan(dev, mods=MODS):
     from feature_vs_text_compound_emotion_b200.models.model import LFAN
     m = LFAN(backbone_settings={"visual_state_dict": "", "audio_state_dict": ""}, output_dim=7, task="CLASSIFICATION",
-             modality=MODS, kernel_size=5, example_length=300, tcn_channel=synthetic.TCN_CHANNELS, modal_dim=32,
+             modality=mods, kernel_size=5, example_length=300, tcn_channel=synthetic.TCN_CHANNELS, modal_dim=32,
              num_heads=2, root_dir="", device=dev)
-    m.init(visual_state_dict=synthetic.visual_backbone_state_dict(0))
-    m.load_state_dict(synthetic.lfan_state_dict(0, MODS), strict=True)
+    m.init(visual_state_dict=synthetic.visual_backbone_state_dict(0),
+           audio_state_dict=synthetic.vggish_state_dict(0) if "logmel" in mods else None)
+    m.load_state_dict(synthetic.lfan_state_dict(0, mods), strict=True)
     return m.to(dev).eval()
 
 
-def chunk_inputs(n, c, dev, seed):
+def chunk_inputs(n, c, dev, seed, wave=False):
     g = torch.Generator(device=dev).manual_seed(seed)
-    return {"video": torch.rand(n, c, 3, 40, 40, device=dev, generator=g) * 2 - 1,
-            "vggish": torch.randn(n, c, 128, device=dev, generator=g),
-            "bert": torch.randn(n, c, 768, device=dev, generator=g)}
+    x = {"video": torch.rand(n, c, 3, 40, 40, device=dev, generator=g) * 2 - 1,
+         "bert": torch.randn(n, c, 768, device=dev, generator=g)}
+    if wave:      # one 30-frame second of samples per stream; each push slices what is in step with its frames
+        x["_wave"] = torch.randn(n, 16000, device=dev, generator=g) * 0.3
+    else:
+        x["vggish"] = torch.randn(n, c, 128, device=dev, generator=g)
+    return x
+
+
+class Synced:
+    """Per push, the samples of every stream that keep its audio in step with its video (all streams of a config
+    are pushed together, so one count serves all)."""
+
+    def __init__(self, sess, fps):
+        self.sess, self.fps = sess, fps
+
+    def __call__(self, ids, x):
+        if "_wave" not in x:
+            return x
+        c = x["video"].shape[1]
+        t = self.sess.length(ids[0])
+        k = streaming.synced_samples(t + c, self.fps) - streaming.synced_samples(t, self.fps)
+        return {"video": x["video"], "bert": x["bert"], "wave": [w[:k] for w in x["_wave"]]}
 
 
 def recompute_rows(sess, c):
@@ -74,20 +105,41 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="profiles/r04_streaming.json")
     ap.add_argument("--window", type=float, default=2.0)
+    ap.add_argument("--audio", choices=("vggish", "wave"), default="vggish",
+                    help="wave: stream raw audio (logmel from the waveform) instead of pre-extracted vggish features")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     torch.set_grad_enabled(False)
-    rec = {"card": card(), "modalities": MODS, "window_length": 300, "hop_length": 200, "configs": []}
-    m = lfan(dev)
-    sess = streaming.StreamSession(m, max_streams=256, max_chunk=30)
+    wave = args.audio == "wave"
+    mods = ["video", "logmel", "bert"] if wave else MODS
+    fps = 30.0
+    rec = {"card": card(), "modalities": mods, "window_length": 300, "hop_length": 200, "configs": []}
+    m = lfan(dev, mods)
+    sess = streaming.StreamSession(m, max_streams=256, max_chunk=30, wave_fps=fps if wave else None)
     rec["state_bytes_per_stream"] = sess.state_bytes()
     rec["n_slots"], rec["n_logit_slots"] = sess.n_slots, sess.n_lslots
+    if wave:
+        rec.update({"wave_fps": fps, "lag_frames": sess.lag, "logmel_ring_rows": sess.n_lm_rows,
+                    "hold_rows": sess.n_hold})
+    synced = Synced(sess, fps)
+    vgg_ms = []
+    if wave:                            # device time of every VGGish call, read after the profiled run
+        aud = m.spatial["audio"]
+        aud_fwd = aud.forward
+
+        def timed(x, *a, **k):
+            s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            s.record()
+            y = aud_fwd(x, *a, **k)
+            e.record()
+            vgg_ms.append((s, e))
+            return y
     for n in (1, 32, 256):
         ids = [sess.open() for _ in range(n)]
         for c in (1, 8, 30):
-            pool = [chunk_inputs(n, c, dev, 10 * n + c + k) for k in range(4)]
-            for k in range(6):                                    # warm-up: every phase's first graph and plan setup
-                sess.push(ids, pool[k % 4])
+            pool = [chunk_inputs(n, c, dev, 10 * n + c + k, wave) for k in range(4)]
+            for k in range(6 + (-(-sess.lag // c) if wave else 0)):   # warm-up: past the lag, every graph and plan
+                sess.push(ids, synced(ids, pool[k % 4]))
             torch.cuda.synchronize()
             times, host, gcs, t0, k = [], [], [], time.perf_counter(), 0
             while time.perf_counter() - t0 < args.window or len(times) < 20:
@@ -95,7 +147,7 @@ def main():
                 g0 = GC_RUNS[0]
                 s.record()
                 h0 = time.perf_counter()
-                sess.push(ids, pool[k % 4])
+                sess.push(ids, synced(ids, pool[k % 4]))
                 host.append((time.perf_counter() - h0) * 1e3)     # the push call alone: enqueue + host work
                 e.record()
                 e.synchronize()
@@ -115,26 +167,45 @@ def main():
                                   for j in slow],
                    "recompute_rows_per_output_row": recompute_rows(sess, c)}
             from torch.profiler import ProfilerActivity, profile
+            if wave:
+                vgg_ms.clear()
+                aud.forward = timed
             with profile(activities=[ProfilerActivity.CUDA]) as prof:
                 for j in range(10):
-                    sess.push(ids, pool[j % 4])
+                    sess.push(ids, synced(ids, pool[j % 4]))
                 torch.cuda.synchronize()
-            head = back = 0.0
+            if wave:
+                del aud.forward
+            head = back = front = 0.0
             for ev in prof.key_averages():
                 t = ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
                 if ev.device_type is None or "Memcpy" in ev.key or "Memset" in ev.key:
                     continue
-                if any(ev.key.startswith("void cer::" + h) or ev.key.startswith(h) or ("cer::" + h) in ev.key
-                       for h in HEAD_KERNELS):
+                if any(("cer::" + h) in ev.key or ev.key.startswith(h) for h in FRONT_END_KERNELS):
+                    front += t
+                elif any(ev.key.startswith("void cer::" + h) or ev.key.startswith(h) or ("cer::" + h) in ev.key
+                         for h in HEAD_KERNELS):
                     head += t
                 else:
                     back += t
             cfg["profiled_kernel_us_per_step"] = {"backbone": back / 10, "head": head / 10,
-                                                  "head_share": head / max(head + back, 1e-9)}
+                                                  "head_share": head / max(head + back + front, 1e-9)}
+            if wave:
+                vgg = sum(s.elapsed_time(e) for s, e in vgg_ms) * 1e3
+                total = head + back + front
+                cfg["profiled_kernel_us_per_step"].update({
+                    "vggish_event_us": vgg / 10, "ir50_preproc": (back - vgg) / 10, "logmel_front_end": front / 10,
+                    "shares": {"ir50_preproc": (back - vgg) / total, "vggish": vgg / total,
+                               "logmel_front_end": front / total, "head": head / total}})
             rec["configs"].append(cfg)
             print(json.dumps(cfg), flush=True)
         for i in ids:
             sess.close(i)
+    if wave:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(rec, f, indent=1)
+        return
     # offline reference on the same kind of frames: 32 videos of 900 frames through infer_videos
     L, nv = 900, 32
     vids = [torch.rand(L, 3, 40, 40, device=dev, generator=torch.Generator(device=dev).manual_seed(i)) * 2 - 1
