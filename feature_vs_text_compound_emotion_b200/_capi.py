@@ -99,6 +99,13 @@ class FusionWeights(C.Structure):
                 ("wr", C.c_void_p), ("br", C.c_void_p)]
 
 
+class CanHeadWeights(C.Structure):
+    _fields_ = [("n_modals", C.c_int32), ("dim", C.c_int32 * CER_MAX_MODALS), ("n_out", C.c_int32),
+                ("attn_w", C.c_void_p * CER_MAX_MODALS), ("attn_b", C.c_void_p * CER_MAX_MODALS),
+                ("gate_w", C.c_void_p), ("gate_b", C.c_void_p), ("fc1_w", C.c_void_p), ("fc1_b", C.c_void_p),
+                ("fc2_w", C.c_void_p), ("fc2_b", C.c_void_p)]
+
+
 # name -> (restype, argtypes); mirrors include/cer_b200.h one to one
 SIGNATURES = {
     "cer_last_error": (C.c_char_p, []),
@@ -135,6 +142,8 @@ SIGNATURES = {
                                            C.c_void_p, C.c_size_t, C.c_void_p]),
     "cer_fusion_head_forward": (C.c_int, [C.POINTER(FusionWeights), C.POINTER(C.c_void_p), C.c_int64, C.c_void_p,
                                           C.c_void_p, C.c_void_p]),
+    "cer_can_head_forward": (C.c_int, [C.POINTER(CanHeadWeights), C.POINTER(C.c_void_p), C.POINTER(C.c_int32), C.c_int64,
+                                       C.c_int32, C.c_void_p, C.c_void_p]),
     "cer_head_last_variant": (C.c_char_p, []),
     "cer_head_train_workspace_bytes": (C.c_size_t, [C.POINTER(HeadTrainSpec), C.c_int64, C.c_int64]),
     "cer_head_train_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(HeadTrainSpec), C.c_int64, C.c_int64, C.c_void_p,

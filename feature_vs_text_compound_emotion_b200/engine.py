@@ -366,6 +366,55 @@ class FusionEngine:
         return (logits, fused) if want_fused else logits
 
 
+class CanHeadEngine:
+    """CAN's AttentionFusion + fc1 (bn1 folded) -> leaky_relu -> fc2 per frame in one launch (cer_can_head_forward).
+    A row's logits are the same bits at any row count, which the chained cer_linear_forward launches of CAN._fuse do
+    not promise (their row GEMM picks split-K from the grid size).  Weights in nn.Linear layouts, copied at packing."""
+
+    def __init__(self, attn: Sequence, gate, fc1, fc2, device: torch.device):
+        _capi.require_gpu()
+        self.device = torch.device(device)
+        self._keep: List[torch.Tensor] = []
+
+        def put(t):
+            d = t.detach().to(device=self.device, dtype=torch.float32, copy=True).contiguous()
+            self._keep.append(d)
+            return d.data_ptr()
+
+        w = _capi.CanHeadWeights()
+        w.n_modals = len(attn)
+        for i, (aw, ab) in enumerate(attn):
+            w.dim[i], w.attn_w[i], w.attn_b[i] = aw.shape[1], put(aw), put(ab)
+        w.gate_w, w.gate_b = put(gate[0]), put(gate[1])
+        w.fc1_w, w.fc1_b = put(fc1[0]), put(fc1[1])
+        w.fc2_w, w.fc2_b = put(fc2[0]), put(fc2[1])
+        w.n_out = fc2[0].shape[0]
+        self._w = w
+        self.dims = [a[0].shape[1] for a in attn]
+        self.n_out = w.n_out
+
+    def forward(self, feats: Sequence[torch.Tensor], apply_tanh: bool, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """feats[m]: [rows, D_m] fp32 (the row pitch may exceed D_m) -> logits [rows, n_out] (into ``out`` if given)."""
+        rows = feats[0].shape[0]
+        ptrs = (C.c_void_p * len(feats))()
+        ld = (C.c_int32 * len(feats))()
+        for i, f in enumerate(feats):
+            if f.dim() != 2 or f.shape[0] != rows or f.shape[1] != self.dims[i] or f.stride(1) != 1:
+                raise ValueError(f"modality {i}: expected [{rows},{self.dims[i]}] with unit feature stride, got "
+                                 f"{tuple(f.shape)}")
+            if f.device != self.device or f.dtype != torch.float32:
+                raise ValueError("inputs must be fp32 on the engine's CUDA device")
+            ptrs[i], ld[i] = f.data_ptr(), f.stride(0)
+        if out is None:
+            out = torch.empty(rows, self.n_out, dtype=torch.float32, device=self.device)
+        if not out.is_contiguous() or tuple(out.shape) != (rows, self.n_out):
+            raise ValueError(f"out: expected a contiguous [{rows},{self.n_out}] tensor")
+        with torch.cuda.device(self.device):
+            check(lib().cer_can_head_forward(C.byref(self._w), ptrs, ld, rows, int(apply_tanh), out.data_ptr(),
+                                             _capi.current_stream_ptr(self.device)), "cer_can_head_forward")
+        return out
+
+
 class PreprocEngine:
     """The reference's eval video transform on the device (cer_preproc_*): uint8 [N,H,W,3] stored
     crops -> fp32 [N,3,crop,crop] in [-1,1], bit-exact with PIL resize + crop + normalise."""

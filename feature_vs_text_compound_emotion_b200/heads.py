@@ -256,6 +256,19 @@ class CAN(_FeatureHead):
         gate = E.linear(cat, self.fuse.weights.weight, self.fuse.weights.bias)
         return self._tail(E.softmax_gate(gate, cat), B, T)
 
+    def frame_head(self) -> E.CanHeadEngine:
+        """AttentionFusion + tail as one row-invariant launch over the current weights (what streaming.StreamSession
+        runs; _fuse keeps its own launches).  A new engine whenever _engines() repacks."""
+        eng = self._engines()
+        cached = self.__dict__.get("_frame_head")
+        if cached is None or cached[0] is not eng:
+            _, w1, b1 = eng
+            f = self.fuse
+            head = E.CanHeadEngine([(a.weight, a.bias) for a in f.attn], (f.weights.weight, f.weights.bias), (w1, b1),
+                                   (self.fc2.weight, self.fc2.bias), w1.device)
+            cached = self.__dict__["_frame_head"] = (eng, head)
+        return cached[1]
+
 
 class JMT(_FeatureHead):
     """Drop-in for models/model.py:1051-1167 (``model_name`` 'JMT' or 'MT'); needs the 'video' and

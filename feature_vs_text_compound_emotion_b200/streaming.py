@@ -1,4 +1,4 @@
-"""Live-video inference: per-chunk logits for many concurrent streams of one LFAN (optional, not in the reference).
+"""Live-video inference: per-chunk logits for many concurrent streams of one LFAN or CAN (optional, not in the reference).
 
 :func:`windowing.infer_video` needs the whole video before it returns.  A :class:`StreamSession` serves up to
 ``max_streams`` live streams instead: ``push`` advances some of them by ``c`` frames and returns their
@@ -18,6 +18,13 @@ The provisional logits of frames ``< T - min(T, W)`` followed by ``close``'s res
 pre-extracted modalities; for 'video' / 'logmel' when the IR-50 / VGGish plan picks the same kernels at both
 pass sizes, the dependence ``infer_videos`` documents).  The TCN and fusion kernels are the offline ones,
 unchanged; csrc/stream.cu holds the per-stream state around them (DESIGN.md section 5.16).
+
+A CAN has no windows: the reference runs it over the whole video, its TemporalBlocks are causal and its fusion and
+tail are per frame, so a frame's logits are final as soon as it arrives.  Each stream is one TCN state slot that
+starts at frame 0 and never ends, ``push`` returns final logits (``final_upto`` is the stream's length) and ``close``
+returns only what was still held back.  The fusion head + tail run as one row-invariant kernel
+(cer_can_head_forward), so a stream's logits do not depend on the other streams of a push or on its chunk sizes
+(DESIGN.md section 5.18).
 """
 from __future__ import annotations
 
@@ -77,6 +84,15 @@ def close_windows(length: int, window_length: int, hop_length: int) -> List[Tupl
     first = length - window_length
     has_tail = first % hop_length != 0
     return [(s, has_tail and i == len(starts) - 1) for i, s in enumerate(starts) if s + window_length > first]
+
+
+def continuous_step_table(streams: Sequence[Tuple[int, int, int]]) -> np.ndarray:
+    """The cer_stream_entry table of one CAN step: streams = (sid, t_now, parity) per pushed stream -> int32
+    [len(streams), 8], one active entry per stream whose single state slot starts at frame 0 and never ends."""
+    tab = np.zeros((len(streams), len(_capi.STREAM_ENTRY_FIELDS)), dtype=np.int32)
+    for i, (sid, t_now, parity) in enumerate(streams):
+        tab[i, 0], tab[i, 4], tab[i, 5], tab[i, 6] = sid, t_now, parity, 1
+    return tab
 
 
 def step_table(streams: Sequence[Tuple[int, int, int]], chunk: int, window_length: int, hop_length: int,
@@ -186,7 +202,7 @@ def logmel_ring_rows(lag: int, max_chunk: int, fps: float) -> int:
 # Session
 # ----------------------------------------------------------------------------------------------
 class StreamSession:
-    """Up to ``max_streams`` live streams of one eval-mode LFAN, pushed ``<= max_chunk`` frames at a time.
+    """Up to ``max_streams`` live streams of one eval-mode LFAN or CAN, pushed ``<= max_chunk`` frames at a time.
 
     Per push input (n streams, c frames each): 'video' as stored uint8 crops [n, c, H, W, 3] or fp32
     [n, c, 3, 40, 40]; 'logmel' as VGGish examples [n, c, 96, 64]; a pre-extracted modality as [n, c, D_m].
@@ -198,14 +214,22 @@ class StreamSession:
     number, 0 included).  The session computes the log-mel rows as their samples arrive (cer_stream_logmel) and
     holds each frame back until its 0.96 s example is complete and it is ``lag`` frames old; ``push`` then returns
     one [r_i, n_out] tensor per stream for the frames it released, and ``close`` flushes the rest with the
-    offline edge padding, so the examples are windowing.wave_to_examples' (DESIGN.md section 5.17)."""
+    offline edge padding, so the examples are windowing.wave_to_examples' (DESIGN.md section 5.17).
+
+    With a CAN the logits ``push`` returns are final; ``window_length`` / ``hop_length`` do not apply and must stay
+    at their defaults (see the module docstring)."""
 
     def __init__(self, model, max_streams: int = 256, max_chunk: int = 30, window_length: int = 300,
                  hop_length: int = 200, wave_fps: float = None):
+        from .heads import CAN
         from .modules import LFAN
-        if not isinstance(model, LFAN):
-            raise TypeError("StreamSession streams LFAN only: the CAN / JMT / MT heads are not streamed (JMT / MT attend "
+        if not isinstance(model, (LFAN, CAN)):
+            raise TypeError("StreamSession streams LFAN and CAN only: the JMT / MT heads are not streamed (JMT / MT attend "
                             "over the whole window, so a frame's logits depend on later frames)")
+        self.continuous = isinstance(model, CAN)          # no windows: one never-ending TCN slot per stream
+        if self.continuous and (window_length, hop_length) != (300, 200):
+            raise ValueError("a CAN stream has no windows: window_length / hop_length do not apply, got "
+                             f"{window_length}, {hop_length}")
         if not (1 <= hop_length <= window_length):
             raise ValueError(f"need 1 <= hop_length <= window_length, got {hop_length}, {window_length}")
         if max_streams < 1 or max_chunk < 1:
@@ -214,11 +238,16 @@ class StreamSession:
         self.model = model
         self._check_model()
         self.max_streams, self.max_chunk = int(max_streams), int(max_chunk)
-        self.W, self.H = int(window_length), int(hop_length)
-        self.n_slots = n_window_slots(self.W, self.H, self.max_chunk)
-        self.n_lslots = n_logit_slots(self.W, self.H, self.max_chunk)
-        self.modalities = list(model.modality)
-        self.device = model.regressor.weight.device
+        if self.continuous:
+            self.W = self.H = None
+            self.n_slots, self.n_lslots = 1, 0
+            self._model_engines, mods, self.device = model._engines, model.modalities, model.fc2.weight.device
+        else:
+            self.W, self.H = int(window_length), int(hop_length)
+            self.n_slots = n_window_slots(self.W, self.H, self.max_chunk)
+            self.n_lslots = n_logit_slots(self.W, self.H, self.max_chunk)
+            self._model_engines, mods, self.device = model._head_engines, model.modality, model.regressor.weight.device
+        self.modalities = list(mods)
         self._len: Dict[int, int] = {}
         self._emitted: Dict[int, int] = {}
         self._parity: Dict[int, int] = {}
@@ -250,7 +279,7 @@ class StreamSession:
         self._lmring = torch.zeros(S, self.n_lm_rows, LOGMEL["n_mel"], dtype=torch.float32, device=dev)
         self._atab = torch.zeros(S * np.dtype(list(_capi.STREAM_AUDIO_ENTRY_FIELDS)).itemsize, dtype=torch.uint8,
                                  device=dev)
-        self._hold = {m: torch.zeros(S, self.n_hold, self._inring[m].shape[-1], dtype=torch.float32, device=dev)
+        self._hold = {m: torch.zeros(S, self.n_hold, self._dims[m], dtype=torch.float32, device=dev)
                       for m in self.modalities if m != "logmel"}
 
     # -- state ------------------------------------------------------------------------------
@@ -259,21 +288,26 @@ class StreamSession:
             raise RuntimeError("StreamSession runs the inference kernels: call model.eval() first")
 
     def _pack(self):
-        """(Re)bind the model's packed head; allocate the rings and step buffers on first use."""
-        tcn, fus = self.model._head_engines()
-        self._eng, self._graphs = (tcn, fus), {}
+        """(Re)bind the model's packed head (LFAN: its FusionEngine; CAN: CAN.frame_head); allocate the rings and step
+        buffers on first use."""
+        self._eng, self._graphs = self._model_engines(), {}
+        tcn = self._eng[0]
+        self._head = self.model.frame_head() if self.continuous else self._eng[1]
+        self._tanh = self.continuous and self.model.task == "REGRESSION"
         dev, S, ne, cm = self.device, self.max_streams, self.max_streams * self.n_slots, self.max_chunk
         f32 = dict(dtype=torch.float32, device=dev)
-        self.n_out = fus.n_out
+        self.n_out = self._head.n_out
         fresh = not hasattr(self, "_tab")
         if fresh:
             self._tab = torch.zeros(ne, len(_capi.STREAM_ENTRY_FIELDS), dtype=torch.int32, device=dev)
-            self._lring = torch.zeros(S, self.n_lslots, self.W, self.n_out, **f32)
+            if not self.continuous:
+                self._lring = torch.zeros(S, self.n_lslots, self.W, self.n_out, **f32)
             self._out = torch.empty(S * cm * self.n_out, **f32)
             self._in, self._inring, self._rings, self._staged, self._outs, self._ws, self._gath = {}, {}, {}, {}, {}, {}, {}
-        self._blocks, self._rows = {}, {}
+        self._blocks, self._rows, self._dims = {}, {}, {}
         for m in self.modalities:
             eng = tcn[m]
+            self._dims[m] = eng.c_in
             if eng.precision != "tf32":      # LFAN packs its TCNs for the tensor-core kernel; the staging assumes its padding
                 raise NotImplementedError(f"'{m}': StreamSession runs the tensor-core TCN kernel only")
             blocks = eng.blocks
@@ -282,7 +316,8 @@ class StreamSession:
             if not fresh:
                 continue
             self._in[m] = torch.empty(S * cm * eng.c_in, **f32)
-            self._inring[m] = torch.zeros(S, self.W, eng.c_in, **f32)
+            if not self.continuous:
+                self._inring[m] = torch.zeros(S, self.W, eng.c_in, **f32)
             self._rings[m] = [torch.zeros(S * self.n_slots * 2 * max(r, 1) * b.c_in, **f32) for b, r in zip(blocks, rows)]
             self._staged[m] = [torch.empty(ne * (r + cm) * b.c_in, **f32) for b, r in zip(blocks, rows)]
             self._outs[m] = [torch.empty(ne * (r + cm) * b.c_out, **f32) for b, r in zip(blocks, rows)]
@@ -291,16 +326,20 @@ class StreamSession:
             self._gath[m] = torch.empty(ne * cm * eng.c_out, **f32)
 
     def _engines(self):
-        eng = self.model._head_engines()
+        eng = self._model_engines()
         if eng is not self._eng:                    # weights changed: the captured graphs hold the old packing
             self._pack()
         return self._eng
 
+    def _final_upto(self, emitted: int) -> int:
+        return emitted if self.continuous else final_upto(emitted, self.W)
+
     def state_bytes(self) -> int:
         """Device memory one stream slot holds across steps (rings), in bytes."""
-        n = self.n_lslots * self.W * self.n_out
+        n = 0 if self.continuous else self.n_lslots * self.W * self.n_out
         for m in self.modalities:
-            n += self.W * self._inring[m].shape[-1]
+            if not self.continuous:
+                n += self.W * self._dims[m]
             n += sum(self.n_slots * 2 * r * b.c_in for b, r in zip(self._blocks[m], self._rows[m]))
         if self.wave_fps is not None:
             n += self.tail_len + self.n_lm_rows * LOGMEL["n_mel"] + sum(h.shape[1] * h.shape[2] for h in self._hold.values())
@@ -321,7 +360,7 @@ class StreamSession:
         return self._len[sid]
 
     def emitted(self, sid: int) -> int:
-        """Frames of stream ``sid`` whose provisional logits were returned (== length without wave_fps)."""
+        """Frames of stream ``sid`` whose logits were returned (== length without wave_fps)."""
         return self._emitted[sid]
 
     # -- push -------------------------------------------------------------------------------
@@ -359,14 +398,15 @@ class StreamSession:
         """The fixed launch sequence of one step over the session's buffers (captured per (n, c))."""
         lib, chk = _capi.lib(), _capi.check
         st = _capi.current_stream_ptr(self.device)
-        tcn, fus = self._eng
+        tcn = self._eng[0]
         ne, tab = n * self.n_slots, self._tab.data_ptr()
         feats = []
         for m in self.modalities:
             eng = tcn[m]
             d_in = eng.c_in
-            chk(lib.cer_stream_retain(tab, n, self.n_slots, c, self._in[m].data_ptr(), d_in, self.W,
-                                      self._inring[m].data_ptr(), st), "cer_stream_retain")
+            if not self.continuous:
+                chk(lib.cer_stream_retain(tab, n, self.n_slots, c, self._in[m].data_ptr(), d_in, self.W,
+                                          self._inring[m].data_ptr(), st), "cer_stream_retain")
             src, src_dim, src_len, src_rows = self._in[m], d_in, 0, 0
             for b, (blk, rows) in enumerate(zip(self._blocks[m], self._rows[m])):
                 L = rows + c
@@ -380,12 +420,15 @@ class StreamSession:
             g = self._gath[m]
             chk(lib.cer_stream_gather(tab, ne, c, src.data_ptr(), src_rows, src_dim, g.data_ptr(), st), "cer_stream_gather")
             feats.append(g[:ne * c * src_dim].view(ne * c, src_dim))
-        logits = fus.forward(feats)
+        if self.continuous:                         # per-frame and final: straight into the output buffer
+            self._head.forward(feats, self._tanh, out=self._out[:n * c * self.n_out].view(n * c, self.n_out))
+            return
+        logits = self._head.forward(feats)
         chk(lib.cer_stream_average(tab, n, self.n_slots, c, self.W, self.n_out, logits.data_ptr(), self._out.data_ptr(),
                                    self._lring.data_ptr(), self.n_lslots, st), "cer_stream_average")
 
     def _use_graph(self) -> bool:
-        return (self.model.head_cuda_graph and os.environ.get("CER_HEAD_GRAPH", "1") != "0"
+        return (getattr(self.model, "head_cuda_graph", True) and os.environ.get("CER_HEAD_GRAPH", "1") != "0"
                 and not torch.cuda.is_current_stream_capturing())
 
     @torch.no_grad()
@@ -393,7 +436,9 @@ class StreamSession:
         """Advance streams ``ids`` by c frames -> (provisional logits [n, c, n_out], final_upto per stream).
 
         With wave_fps: -> (a list of n tensors [r_i, n_out], the provisional logits of the frames this push
-        released, continuing from emitted(i); final_upto = max(0, emitted(i) - W) per stream)."""
+        released, continuing from emitted(i); final_upto = max(0, emitted(i) - W) per stream).
+
+        With a CAN every returned logit is final: final_upto = emitted(i)."""
         self._check_model()
         ids = [int(i) for i in ids]
         n = len(ids)
@@ -407,23 +452,24 @@ class StreamSession:
         with torch.cuda.device(self.device):
             c, x = self._chunk_features(inputs, n)
             for m in self.modalities:
-                d = self._inring[m].shape[-1]
+                d = self._dims[m]
                 if x[m].shape[1] != d:
                     raise ValueError(f"'{m}': expected {d} features per frame, got {x[m].shape[1]}")
             out = self._head_step(ids, c, x)
         for i in ids:
             self._len[i] += c
-        return out, [final_upto(self._len[i], self.W) for i in ids]
+        return out, [self._final_upto(self._len[i]) for i in ids]
 
     def _head_step(self, ids: List[int], c: int, x: Dict[str, torch.Tensor]) -> torch.Tensor:
         """Frames emitted(i) .. emitted(i) + c - 1 of streams ``ids`` (features x[m] [n * c, D_m]) through the head
         -> their provisional logits [n, c, n_out]; advances emitted and the TCN ring parity of those streams."""
         n = len(ids)
         for m in self.modalities:
-            d = self._inring[m].shape[-1]
+            d = self._dims[m]
             self._in[m][:n * c * d].view(n * c, d).copy_(x[m])
-        tab = step_table([(i, self._emitted[i], self._parity[i]) for i in ids], c, self.W, self.H, self.n_slots,
-                         self.n_lslots)
+        streams = [(i, self._emitted[i], self._parity[i]) for i in ids]
+        tab = (continuous_step_table(streams) if self.continuous else
+               step_table(streams, c, self.W, self.H, self.n_slots, self.n_lslots))
         self._tab[:tab.shape[0]].copy_(torch.from_numpy(tab).pin_memory(), non_blocking=True)
         g = self._graphs.get((n, c)) if self._use_graph() else False
         if g:
@@ -556,40 +602,45 @@ class StreamSession:
             outs = self._release([(sid, e0, r, 0) for sid, e0, r in plan])
             empty = torch.empty(0, self.n_out, dtype=torch.float32, device=self.device)
             res = [torch.cat(outs[sid]) if sid in outs else empty for sid in ids]
-        return res, [final_upto(self._emitted[i], self.W) for i in ids]
+        return res, [self._final_upto(self._emitted[i]) for i in ids]
 
-    def _flush_wave(self, sid: int) -> None:
+    def _flush_wave(self, sid: int) -> List[torch.Tensor]:
         """close: one second of the last sample (wave_to_examples' edge padding), the remaining log-mel rows, and the
-        held-back frames through the head; frames at or above the example count reuse the last example."""
+        held-back frames through the head; frames at or above the example count reuse the last example.  Returns the
+        logits of those head steps, in frame order."""
         A, T, E = self._samples[sid], self._len[sid], self._emitted[sid]
         pad = self._tails[sid, -1:].expand(LOGMEL["sample_rate"]).contiguous()
         self._front_end([(sid, A, pad)])
         self._samples[sid] = A + pad.numel()
         n_ex = n_examples_total(logmel_rows(A + pad.numel()), self.wave_fps)
-        self._release([(sid, E, T - E, n_ex)])
+        return self._release([(sid, E, T - E, n_ex)]).get(sid, [])
 
     # -- close ------------------------------------------------------------------------------
     @torch.no_grad()
     def close(self, sid: int) -> torch.Tensor:
         """End stream ``sid`` -> the final logits [min(T, W), n_out] of its frames T - min(T, W) .. T - 1, and free
-        its slot."""
+        its slot.  With a CAN: the logits of the frames not returned yet ([0, n_out] without wave_fps; the
+        held-back frames with it)."""
         from .engine import stitch_windows
         if sid not in self._len:
             raise ValueError(f"stream {sid} is not open")
         self._check_model()
         self._engines()
+        flushed = []
         if self.wave_fps is not None and self._len[sid] > 0:
             if self._samples[sid] == 0:
                 raise ValueError(f"stream {sid} received no audio: its frames have no VGGish example (offline, "
                                  "wave_to_examples fails on an empty waveform the same way)")
             with torch.cuda.device(self.device):
-                self._flush_wave(sid)
+                flushed = self._flush_wave(sid)
         T, W = self._len.pop(sid), self.W
         del self._parity[sid], self._emitted[sid]
         if self.wave_fps is not None:
             del self._samples[sid]
         self._free.append(sid)
-        if T == 0:
+        if self.continuous and flushed:
+            return torch.cat(flushed)
+        if T == 0 or self.continuous:
             return torch.empty(0, self.n_out, dtype=torch.float32, device=self.device)
         first, _ = close_range(T, W)
         wins = close_windows(T, W, self.H)

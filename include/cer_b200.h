@@ -308,10 +308,41 @@ int cer_modal_attention_forward(const float* const* qkv_dev, int64_t rows, int32
 int cer_fusion_head_forward(const cer_fusion_weights* w, const float* const* feats_dev, int64_t rows,
                             float* logits_dev, float* fused_out_dev /* [rows][E] or NULL */, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * CAN fusion head + tail, fused.   Replaces AttentionFusion.forward (models/model.py:552-568) and
+ * fc1 -> bn1 -> leaky_relu -> fc2 (-> tanh) of CAN.forward (:678-682) per frame:
+ *   cat = [attn_0(z_0) | ... | attn_{M-1}(z_{M-1})]  (Linear(C_i -> 128) each, D = 128 * M)
+ *   h   = leaky_relu(fc1'(softmax(weights(cat)) * cat), 0.01)   (softmax over all D entries)
+ *   out = fc2(h), tanh(out) if apply_tanh (task == REGRESSION).
+ * Exact fp32 on the CUDA cores.  Every output element is summed over k in one fixed order and the
+ * softmax reductions run in one fixed order, so a row's logits are the same bits whatever `rows`
+ * is and wherever the row lies in the call (a live stream does not change with the other streams
+ * sharing its push; streaming.StreamSession with a CAN).  Limits: 1 <= M <= 4, C_i <= 512,
+ * n_out <= 64.  Weight layouts are nn.Linear's ([out][in], row-major).
+ * ------------------------------------------------------------------------------------------ */
+typedef struct cer_can_head_weights {
+  int32_t n_modals;                    /* M                                                       */
+  int32_t dim[CER_MAX_MODALS];         /* C_i: last TemporalBlock channels of modality i          */
+  int32_t n_out;                       /* fc2 outputs                                             */
+  const float* attn_w[CER_MAX_MODALS]; /* fp32 [128][C_i]  fuse.attn.<i>.weight                    */
+  const float* attn_b[CER_MAX_MODALS]; /* fp32 [128]       fuse.attn.<i>.bias                      */
+  const float* gate_w;                 /* fp32 [D][D]      fuse.weights.weight                     */
+  const float* gate_b;                 /* fp32 [D]                                                 */
+  const float* fc1_w;                  /* fp32 [D][D]      fc1.weight * bn1 scale (per output row) */
+  const float* fc1_b;                  /* fp32 [D]         fc1.bias * bn1 scale + bn1 shift        */
+  const float* fc2_w;                  /* fp32 [n_out][D]  fc2.weight                              */
+  const float* fc2_b;                  /* fp32 [n_out]                                             */
+} cer_can_head_weights;
+
+/* feats_dev: HOST array of M device pointers, modality i fp32 [rows][ld[i]] (its first C_i columns are
+ * read; ld: HOST int32 [M], ld[i] >= C_i); out_dev: fp32 [rows][n_out]. */
+int cer_can_head_forward(const cer_can_head_weights* w, const float* const* feats_dev, const int32_t* ld, int64_t rows,
+                         int32_t apply_tanh, float* out_dev, void* stream);
+
 /* Name of the kernel instantiation the last head launch on this thread ran: one conv launch of
- * cer_tcn_block_tc_forward (e.g. "tcn_igemm_kernel<64,8>"), cer_tcn_block_forward ("tcn_block_kernel<128,4,5>")
- * or cer_fusion_head_forward ("fusion_head_kernel<5>").  "none" before the first launch; a call refused
- * before launching leaves it unchanged. */
+ * cer_tcn_block_tc_forward (e.g. "tcn_igemm_kernel<64,8>"), cer_tcn_block_forward ("tcn_block_kernel<128,4,5>"),
+ * cer_fusion_head_forward ("fusion_head_kernel<5>") or cer_can_head_forward ("can_head_kernel").  "none" before
+ * the first launch; a call refused before launching leaves it unchanged. */
 const char* cer_head_last_variant(void);
 
 /* ------------------------------------------------------------------------------------------

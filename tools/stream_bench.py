@@ -23,6 +23,14 @@ warmed up.  The profiled run splits kernel time into IR-50 and preprocessing / V
 (cer_stream_logmel, cer_stream_examples) / head; VGGish is timed with CUDA events around its calls in that run (its
 convolutions are the IR-50 kernels, so kernel names cannot tell them apart) and IR-50 and preprocessing are the rest of
 the backbone kernel time.  infer_videos is not run in this mode.
+
+    python tools/stream_bench.py --head can --out profiles/r06_stream_can.json
+
+streams a CAN instead (DESIGN.md section 5.18): 'video' + 'vggish' + 'bert' with synthetic.TCN_SETTINGS, final per-frame
+logits, at (n, c) in {1x1, 1x30, 32x8, 32x30, 256x1, 256x8, 256x30}; head kernels are the TCN, stream.cu and
+can_head_kernel.  The same run times can_head_kernel alone at 7 680 rows (CUDA events over repeated launches on one
+set of inputs, so its 1.4 MB of weights are L2-resident as in a step) and reports GFLOP/s from the shape-derived
+FLOP count.  infer_videos is not run in this mode.
 """
 from __future__ import annotations
 
@@ -39,7 +47,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from feature_vs_text_compound_emotion_b200 import streaming, synthetic, windowing  # noqa: E402
 
-HEAD_KERNELS = ("tcn_", "fusion_", "stream_")
+HEAD_KERNELS = ("tcn_", "fusion_", "stream_", "can_head")
 FRONT_END_KERNELS = ("stream_logmel", "stream_tail", "stream_examples")
 GC_RUNS = [0]
 gc.callbacks.append(lambda phase, info: GC_RUNS.__setitem__(0, GC_RUNS[0] + (phase == "start")))
@@ -67,6 +75,41 @@ def lfan(dev, mods=MODS):
            audio_state_dict=synthetic.vggish_state_dict(0) if "logmel" in mods else None)
     m.load_state_dict(synthetic.lfan_state_dict(0, mods), strict=True)
     return m.to(dev).eval()
+
+
+def can(dev, mods=MODS):
+    from feature_vs_text_compound_emotion_b200.models.model import CAN
+    m = CAN(task="CLASSIFICATION", modalities=mods, tcn_settings=synthetic.TCN_SETTINGS,
+            backbone_settings={"visual_state_dict": "", "audio_state_dict": ""}, output_dim=7, root_dir="", device=dev,
+            visual_state_dict=synthetic.visual_backbone_state_dict(0))
+    m.load_state_dict(synthetic.can_state_dict(0, mods), strict=True)
+    return m.to(dev).eval()
+
+
+def can_head_flop(m) -> int:
+    """FLOPs of one frame through cer_can_head_forward: the four GEMVs (softmax, activation and bias not counted)."""
+    D = 128 * len(m.modalities)
+    cs = sum(synthetic.TCN_SETTINGS[k]["channel"][-1] for k in m.modalities)
+    return 2 * 128 * cs + 2 * 2 * D * D + 2 * D * m.fc2.weight.shape[0]
+
+
+def time_can_head(m, dev, rows=7680, reps=200):
+    head = m.frame_head()
+    g = torch.Generator(device=dev).manual_seed(7)
+    z = [torch.randn(rows, synthetic.TCN_SETTINGS[k]["channel"][-1], device=dev, generator=g) for k in m.modalities]
+    out = torch.empty(rows, head.n_out, device=dev)
+    for _ in range(10):
+        head.forward(z, False, out=out)
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record()
+    for _ in range(reps):
+        head.forward(z, False, out=out)
+    e.record()
+    e.synchronize()
+    us = s.elapsed_time(e) * 1e3 / reps
+    flop = can_head_flop(m) * rows
+    return {"rows": rows, "reps": reps, "us_per_launch": us, "flop_per_frame": can_head_flop(m),
+            "gflop_per_s": flop / (us * 1e-6) / 1e9}
 
 
 def chunk_inputs(n, c, dev, seed, wave=False):
@@ -107,14 +150,24 @@ def main():
     ap.add_argument("--window", type=float, default=2.0)
     ap.add_argument("--audio", choices=("vggish", "wave"), default="vggish",
                     help="wave: stream raw audio (logmel from the waveform) instead of pre-extracted vggish features")
+    ap.add_argument("--head", choices=("lfan", "can"), default="lfan")
     args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("stream_bench measures the B200 kernels: no CUDA device")
     dev = torch.device("cuda:0")
     torch.set_grad_enabled(False)
     wave = args.audio == "wave"
+    is_can = args.head == "can"
+    if wave and is_can:
+        raise SystemExit("--head can streams pre-extracted vggish features")
     mods = ["video", "logmel", "bert"] if wave else MODS
     fps = 30.0
-    rec = {"card": card(), "modalities": mods, "window_length": 300, "hop_length": 200, "configs": []}
-    m = lfan(dev, mods)
+    rec = {"card": card(), "head": args.head, "modalities": mods, "configs": []}
+    if is_can:
+        rec["tcn_settings"] = {k: synthetic.TCN_SETTINGS[k] for k in mods}
+    else:
+        rec.update({"window_length": 300, "hop_length": 200})
+    m = can(dev, mods) if is_can else lfan(dev, mods)
     sess = streaming.StreamSession(m, max_streams=256, max_chunk=30, wave_fps=fps if wave else None)
     rec["state_bytes_per_stream"] = sess.state_bytes()
     rec["n_slots"], rec["n_logit_slots"] = sess.n_slots, sess.n_lslots
@@ -134,9 +187,10 @@ def main():
             e.record()
             vgg_ms.append((s, e))
             return y
-    for n in (1, 32, 256):
+    grid = {1: (1, 30), 32: (8, 30), 256: (1, 8, 30)} if is_can else {n: (1, 8, 30) for n in (1, 32, 256)}
+    for n, chunks in grid.items():
         ids = [sess.open() for _ in range(n)]
-        for c in (1, 8, 30):
+        for c in chunks:
             pool = [chunk_inputs(n, c, dev, 10 * n + c + k, wave) for k in range(4)]
             for k in range(6 + (-(-sess.lag // c) if wave else 0)):   # warm-up: past the lag, every graph and plan
                 sess.push(ids, synced(ids, pool[k % 4]))
@@ -201,7 +255,10 @@ def main():
             print(json.dumps(cfg), flush=True)
         for i in ids:
             sess.close(i)
-    if wave:
+    if is_can:
+        rec["can_head_kernel"] = time_can_head(m, dev)
+        print(json.dumps(rec["can_head_kernel"]), flush=True)
+    if wave or is_can:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
             json.dump(rec, f, indent=1)
