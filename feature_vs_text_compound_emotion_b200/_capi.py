@@ -191,6 +191,8 @@ SIGNATURES = {
                                    C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_sdpa_tc_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                       C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "cer_sdpa_tc_seg_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                          C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_add_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float,
                                     C.c_void_p, C.c_void_p]),
     "cer_modal_attention_maps": (C.c_int, [C.POINTER(C.c_void_p), C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),

@@ -105,10 +105,14 @@ __device__ __forceinline__ void mma_tf32(float (&d)[4], uint32_t a0, uint32_t a1
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-template <int E>
+//   kSeg: blockIdx.y is a segment s; q, k, v and out rows are [seg_off[s], seg_off[s+1]) of their buffers and
+//   len_q = len_k = that length (self- or cross-attention inside one video of a concatenated batch).  A CTA past
+//   its segment's end returns before any load or barrier; every other instruction is the uniform kernel's, so a
+//   segment gives the same bits as a batch-1 launch on it alone.
+template <int E, bool kSeg>
 __global__ void __launch_bounds__(128) sdpa_tc_kernel(const float* __restrict__ q, int ldq, const float* __restrict__ k, int ldk,
                                                       const float* __restrict__ v, int ldv, int len_q, int len_k,
-                                                      float* __restrict__ out, int ldo) {
+                                                      float* __restrict__ out, int ldo, const int* __restrict__ seg_off) {
   constexpr int LD = E + 4;
   extern __shared__ float sm_f[];
   uint32_t* sQ = reinterpret_cast<uint32_t*>(sm_f);            // [64][LD] tf32 bits
@@ -118,9 +122,18 @@ __global__ void __launch_bounds__(128) sdpa_tc_kernel(const float* __restrict__ 
   const int g = lane >> 2, t = lane & 3;
   const int b = blockIdx.y;
   const int q0 = blockIdx.x * kSdpaQ;
-  const float* qb = q + (long long)b * len_q * ldq;
-  const float* kb = k + (long long)b * len_k * ldk;
-  const float* vb = v + (long long)b * len_k * ldv;
+  long long row_q, row_k;
+  if constexpr (kSeg) {
+    row_q = row_k = seg_off[b];
+    len_q = len_k = seg_off[b + 1] - seg_off[b];
+    if (q0 >= len_q) return;                                    // uniform per CTA: no barrier is reached by part of it
+  } else {
+    row_q = (long long)b * len_q;
+    row_k = (long long)b * len_k;
+  }
+  const float* qb = q + row_q * ldq;
+  const float* kb = k + row_k * ldk;
+  const float* vb = v + row_k * ldv;
   const float scale = rsqrtf((float)E);
 
   for (int i = threadIdx.x; i < kSdpaQ * (E / 4); i += 128) {
@@ -214,7 +227,7 @@ __global__ void __launch_bounds__(128) sdpa_tc_kernel(const float* __restrict__ 
   }
   const float inv0 = 1.f / lrow[0], inv1 = 1.f / lrow[1];
   const int r0 = q0 + warp * 16 + g, r1 = r0 + 8;
-  float* ob = out + (long long)b * len_q * ldo;
+  float* ob = out + row_q * ldo;
 #pragma unroll
   for (int n = 0; n < E / 8; ++n) {
     if (r0 < len_q) *reinterpret_cast<float2*>(ob + (long long)r0 * ldo + n * 8 + 2 * t) = make_float2(o[n][0] * inv0, o[n][1] * inv0);
@@ -309,17 +322,30 @@ extern "C" int cer_sdpa_forward(const float* q_dev, int32_t ldq, const float* k_
   return CER_OK;
 }
 
-template <int E>
+// Uniform: grid (ceil(len_q / 64), batch).  Segmented (seg_off != null): grid (ceil(len_q / 64), n_seg), len_q the
+// longest segment.
+template <int E, bool kSeg>
 static int launch_sdpa_tc(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, int batch, int len_q, int len_k,
-                          float* out, int ldo, cudaStream_t st) {
+                          float* out, int ldo, const int* seg_off, cudaStream_t st) {
   const size_t smem = (size_t)(kSdpaQ + 2 * kSdpaK) * (E + 4) * sizeof(float);
   static unsigned long long configured = 0;
   if (first_use_on_device(&configured))
-    CER_CUDA(cudaFuncSetAttribute(sdpa_tc_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CER_CUDA(cudaFuncSetAttribute(sdpa_tc_kernel<E, kSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((len_q + kSdpaQ - 1) / kSdpaQ, batch);
-  sdpa_tc_kernel<E><<<grid, 128, smem, st>>>(q, ldq, k, ldk, v, ldv, len_q, len_k, out, ldo);
+  sdpa_tc_kernel<E, kSeg><<<grid, 128, smem, st>>>(q, ldq, k, ldk, v, ldv, len_q, len_k, out, ldo, seg_off);
   CER_CUDA(cudaGetLastError());
   return CER_OK;
+}
+
+// dim / pitch / alignment conditions shared by both entry points
+static int check_sdpa_tc(const char* what, const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev,
+                         int32_t ldv, int32_t dim, const float* out_dev, int32_t ldo) {
+  if ((dim != 64 && dim != 128) || ldq % 4 || ldk % 4 || ldv % 4 || ldo % 2)
+    return set_error(CER_ERR_INVALID, std::string(what) + ": dim must be 64 or 128, row pitches multiples of 4 floats");
+  if ((reinterpret_cast<uintptr_t>(q_dev) | reinterpret_cast<uintptr_t>(k_dev) | reinterpret_cast<uintptr_t>(v_dev)) & 15 ||
+      reinterpret_cast<uintptr_t>(out_dev) & 7)
+    return set_error(CER_ERR_INVALID, std::string(what) + ": q / k / v must be 16-byte aligned, out 8-byte aligned");
+  return cer_check_device();
 }
 
 extern "C" int cer_sdpa_tc_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev,
@@ -328,16 +354,26 @@ extern "C" int cer_sdpa_tc_forward(const float* q_dev, int32_t ldq, const float*
   if (!q_dev || !k_dev || !v_dev || !out_dev || batch <= 0 || len_q <= 0 || len_k <= 0 || ldq < dim || ldk < dim || ldv < dim ||
       ldo < dim || batch > 65535)
     return set_error(CER_ERR_INVALID, "cer_sdpa_tc_forward: bad argument");
-  if ((dim != 64 && dim != 128) || ldq % 4 || ldk % 4 || ldv % 4 || ldo % 2)
-    return set_error(CER_ERR_INVALID, "cer_sdpa_tc_forward: dim must be 64 or 128, row pitches multiples of 4 floats");
-  if ((reinterpret_cast<uintptr_t>(q_dev) | reinterpret_cast<uintptr_t>(k_dev) | reinterpret_cast<uintptr_t>(v_dev)) & 15 ||
-      reinterpret_cast<uintptr_t>(out_dev) & 7)
-    return set_error(CER_ERR_INVALID, "cer_sdpa_tc_forward: q / k / v must be 16-byte aligned, out 8-byte aligned");
-  int rc = cer_check_device();
+  int rc = check_sdpa_tc("cer_sdpa_tc_forward", q_dev, ldq, k_dev, ldk, v_dev, ldv, dim, out_dev, ldo);
   if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  return dim == 128 ? launch_sdpa_tc<128>(q_dev, ldq, k_dev, ldk, v_dev, ldv, batch, len_q, len_k, out_dev, ldo, st)
-                    : launch_sdpa_tc<64>(q_dev, ldq, k_dev, ldk, v_dev, ldv, batch, len_q, len_k, out_dev, ldo, st);
+  return dim == 128 ? launch_sdpa_tc<128, false>(q_dev, ldq, k_dev, ldk, v_dev, ldv, batch, len_q, len_k, out_dev, ldo, nullptr, st)
+                    : launch_sdpa_tc<64, false>(q_dev, ldq, k_dev, ldk, v_dev, ldv, batch, len_q, len_k, out_dev, ldo, nullptr, st);
+}
+
+extern "C" int cer_sdpa_tc_seg_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev,
+                                       int32_t ldv, const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len, int32_t dim,
+                                       float* out_dev, int32_t ldo, void* stream) {
+  if (!q_dev || !k_dev || !v_dev || !out_dev || !seg_off_dev || n_seg < 0 || max_len < 0 || ldq < dim || ldk < dim ||
+      ldv < dim || ldo < dim)
+    return set_error(CER_ERR_INVALID, "cer_sdpa_tc_seg_forward: bad argument");
+  if (n_seg > 65535) return set_error(CER_ERR_INVALID, "cer_sdpa_tc_seg_forward: more than 65535 segments (the grid's y limit)");
+  int rc = check_sdpa_tc("cer_sdpa_tc_seg_forward", q_dev, ldq, k_dev, ldk, v_dev, ldv, dim, out_dev, ldo);
+  if (rc) return rc;
+  if (n_seg == 0 || max_len == 0) return CER_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return dim == 128 ? launch_sdpa_tc<128, true>(q_dev, ldq, k_dev, ldk, v_dev, ldv, n_seg, max_len, max_len, out_dev, ldo, seg_off_dev, st)
+                    : launch_sdpa_tc<64, true>(q_dev, ldq, k_dev, ldk, v_dev, ldv, n_seg, max_len, max_len, out_dev, ldo, seg_off_dev, st);
 }
 
 extern "C" int cer_add_layernorm(const float* x_dev, const float* res_dev, int64_t rows, int32_t dim, const float* gamma_dev,

@@ -596,6 +596,46 @@ def sdpa(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, batch: int, len_q: i
     return out
 
 
+class Segments:
+    """Row segmentation of videos laid end to end in one buffer: segment s is rows [off[s], off[s+1]).  Built once per
+    call from host-side lengths (all positive), so the offsets are ascending from 0 and ``max_len`` bounds every
+    segment, as cer_sdpa_tc_seg_forward requires."""
+
+    def __init__(self, lengths: Sequence[int], device):
+        self.lengths = [int(t) for t in lengths]
+        if any(t <= 0 for t in self.lengths):
+            raise ValueError(f"segments need positive lengths, got {self.lengths}")
+        off = [0]
+        for t in self.lengths:
+            off.append(off[-1] + t)
+        self.offsets = off
+        self.n_seg = len(self.lengths)
+        self.max_len = max(self.lengths, default=0)
+        self.rows = off[-1]
+        self.off = torch.tensor(off, dtype=torch.int32).to(device)
+
+
+def sdpa_segments(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, seg: Segments) -> torch.Tensor:
+    """Single-head attention inside each segment (cer_sdpa_tc_seg_forward, TF32 tensor cores): rows of segment s of q
+    attend over rows of segment s of k / v only.  q / k / v [seg.rows, E] (column slices of a packed projection are
+    fine) -> [seg.rows, E].  There is no other kernel behind it: inputs the tensor-core kernel cannot take raise."""
+    e = q.shape[1]
+    if e not in (64, 128) or any(t.dim() != 2 or t.shape != (seg.rows, e) for t in (k, v)) or q.shape[0] != seg.rows:
+        raise ValueError(f"sdpa_segments: q / k / v must be [{seg.rows}, E] with E 64 or 128, got "
+                         f"{[tuple(t.shape) for t in (q, k, v)]}")
+    if any(t.stride(1) != 1 or t.stride(0) % 4 or t.data_ptr() % 16 or t.dtype != torch.float32 for t in (q, k, v)):
+        raise ValueError("sdpa_segments: q / k / v must be fp32 with unit feature stride, row pitches that are multiples "
+                         "of 4 floats and 16-byte aligned rows")
+    if seg.off.device != q.device:
+        raise ValueError("sdpa_segments: the segment offsets are on another device")
+    out = torch.empty(seg.rows, e, dtype=torch.float32, device=q.device)
+    with torch.cuda.device(q.device):
+        check(lib().cer_sdpa_tc_seg_forward(q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0),
+                                            seg.off.data_ptr(), seg.n_seg, seg.max_len, e, out.data_ptr(), e,
+                                            _capi.current_stream_ptr()), "cer_sdpa_tc_seg_forward")
+    return out
+
+
 def add_layernorm(x: torch.Tensor, res: Optional[torch.Tensor], gamma: torch.Tensor, beta: torch.Tensor,
                   eps: float = 1e-5) -> torch.Tensor:
     out = torch.empty_like(x)

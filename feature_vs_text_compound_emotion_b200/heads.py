@@ -62,8 +62,9 @@ class TransformerEncoderBlock(nn.Module):
         self.layers = SequentialEncoder(*[TransformerEncoderLayer(input_dim, num_heads, hidden_dim) for _ in range(num_layers)])
 
 
-def _mha(mod: nn.MultiheadAttention, q_in, kv_in, batch, len_q, len_k):
-    """nn.MultiheadAttention(E, 1)(q_in, kv_in, kv_in) on batch-major rows [batch*len, E]."""
+def _mha(mod: nn.MultiheadAttention, q_in, kv_in, layout):
+    """nn.MultiheadAttention(E, 1)(q_in, kv_in, kv_in) on rows [R, E].  ``layout``: (batch, len_q, len_k) for batch-major
+    sequences of equal length, or an engine.Segments (one sequence per video, queries and keys segmented alike)."""
     e = mod.embed_dim
     W, b = mod.in_proj_weight, mod.in_proj_bias
     if q_in is kv_in:
@@ -73,14 +74,14 @@ def _mha(mod: nn.MultiheadAttention, q_in, kv_in, batch, len_q, len_k):
         q = E.linear(q_in, W[:e], b[:e])
         kv = E.linear(kv_in, W[e:], b[e:])
         k, v = kv[:, :e], kv[:, e:]
-    att = E.sdpa(q, k, v, batch, len_q, len_k)
+    att = E.sdpa_segments(q, k, v, layout) if isinstance(layout, E.Segments) else E.sdpa(q, k, v, *layout)
     return E.linear(att, mod.out_proj.weight, mod.out_proj.bias)
 
 
-def _encoder(block: TransformerEncoderBlock, x, batch, length):
-    """TransformerEncoderBlock.forward (model.py:723-750) on batch-major rows."""
+def _encoder(block: TransformerEncoderBlock, x, layout):
+    """TransformerEncoderBlock.forward (model.py:723-750) on rows; ``layout`` as for _mha."""
     for layer in block.layers:
-        a = _mha(layer.attention, x, x, batch, length, length)
+        a = _mha(layer.attention, x, x, layout)
         x = E.add_layernorm(x, a, layer.layer_norm1.weight, layer.layer_norm1.bias, layer.layer_norm1.eps)
         ff = E.linear(E.linear(x, layer.feed_forward[0].weight, layer.feed_forward[0].bias, "relu"),
                       layer.feed_forward[2].weight, layer.feed_forward[2].bias)
@@ -217,6 +218,29 @@ class _FeatureHead(_PackedModule):
         _capi.require_gpu()
         return self._fuse(self._encode_features(feats))
 
+    def forward_videos(self, feats, lengths) -> torch.Tensor:
+        """Whole videos laid end to end, each run as the reference runs these heads (batch 1, the whole video):
+        feats[m] [sum(lengths), D_m] (visual = 512-d IR-50 embeddings) -> per-frame logits [sum(lengths), n_out].
+
+        The TCN runs on one right-padded [n_videos, T_max, D_m] batch: its blocks are causal, so rows past a video's
+        end never reach the video's frames, and the tensor-core kernel's per-row arithmetic does not depend on B or
+        T, so each video's rows are those of a TCN run on that video alone.  The valid rows are then gathered back
+        into the concatenated layout for the fusion head (see _fuse_videos)."""
+        from . import _capi, windowing
+        _capi.require_gpu()
+        tcn, _, _ = self._engines()
+        dev = self.fc2.weight.device
+        n = len(lengths)
+        t_max, idx = windowing.padded_row_index(lengths)
+        idx = idx.to(dev, non_blocking=True)
+        z = {}
+        for m in self.modalities:
+            x = feats[m].float()
+            pad = torch.zeros(n * t_max, x.shape[1], dtype=torch.float32, device=dev)
+            pad[idx] = x
+            z[m] = tcn[m].forward(pad.view(n, t_max, -1)).view(n * t_max, -1)[idx]
+        return self._fuse_videos(z, lengths)
+
     def _tail(self, c2d: torch.Tensor, B: int, T: int) -> torch.Tensor:
         _, w1, b1 = self._engines()
         h = E.linear(c2d, w1, b1, "leaky_relu")
@@ -255,6 +279,11 @@ class CAN(_FeatureHead):
             E.linear(z[m].view(B * T, -1), self.fuse.attn[i].weight, self.fuse.attn[i].bias, out=cat[:, 128 * i:128 * (i + 1)])
         gate = E.linear(cat, self.fuse.weights.weight, self.fuse.weights.bias)
         return self._tail(E.softmax_gate(gate, cat), B, T)
+
+    def _fuse_videos(self, z, lengths):
+        """AttentionFusion + tail row by row (frame_head(): one result per frame whatever else is in the call, so a
+        video's logits equal a StreamSession's for the same frames)."""
+        return self.frame_head().forward([z[m] for m in self.modalities], self.task == "REGRESSION")
 
     def frame_head(self) -> E.CanHeadEngine:
         """AttentionFusion + tail as one row-invariant launch over the current weights (what streaming.StreamSession
@@ -297,19 +326,30 @@ class JMT(_FeatureHead):
         return self._fuse(self._encode(X))
 
     def _fuse(self, z):
-        f = self.fuse
         B, T, _ = z['video'].shape
         R = B * T
-        vis = z['video'].view(R, -1)
-        aud = E.linear(z['vggish'].view(R, -1), f.augment_audio_feats_dim.weight, f.augment_audio_feats_dim.bias)
-        ea = _encoder(f.audio_encoder, aud, B, T)
+        # the final encoder attends over all L*B positions (see module docstring)
+        out = self._fuse_rows(z['video'].view(R, -1), z['vggish'].view(R, -1), (B, T, T), (1, R, R))
+        return self._tail(out, B, T)
+
+    def _fuse_videos(self, z, lengths):
+        """With batch 1 per video, the reference's "all L*B positions" are the video's own frames: every attention
+        runs inside each video's segment of the concatenated rows."""
+        seg = E.Segments(lengths, z['video'].device)
+        return self._tail(self._fuse_rows(z['video'], z['vggish'], seg, seg), 1, seg.rows)[0]
+
+    def _fuse_rows(self, vis, vggish, seq, final):
+        """JMTFusion / MTFusion on rows [R, C]: ``seq`` lays out the sequences of the modality encoders and the
+        cross-attention, ``final`` those of the final encoder and self-attention (each as _mha's layout)."""
+        f = self.fuse
+        aud = E.linear(vggish, f.augment_audio_feats_dim.weight, f.augment_audio_feats_dim.bias)
+        ea = _encoder(f.audio_encoder, aud, seq)
         if self.model_name == "JMT":
             jr = E.linear(torch.cat((vis, aud), dim=1), f.reduce_feats_dim.weight, f.reduce_feats_dim.bias)
-            ej = _encoder(f.jr_encoder, jr, B, T)
-            last = _mha(f.CA_ajr, ea, ej, B, T, T)            # the only stack slot the output reads
+            ej = _encoder(f.jr_encoder, jr, seq)
+            last = _mha(f.CA_ajr, ea, ej, seq)                # the only stack slot the output reads
         else:
-            ev = _encoder(f.visual_encoder, vis, B, T)
-            last = _mha(f.CA_av, ea, ev, B, T, T)
-        enc = _encoder(f.final_encoder, last, 1, R)           # attention over all L*B positions (see module docstring)
-        out = _mha(f.final_self_attention, enc, enc, 1, R, R)
-        return self._tail(out, B, T)
+            ev = _encoder(f.visual_encoder, vis, seq)
+            last = _mha(f.CA_av, ea, ev, seq)
+        enc = _encoder(f.final_encoder, last, final)
+        return _mha(f.final_self_attention, enc, enc, final)

@@ -6,6 +6,9 @@ table (SURVEY.md section 8 f1):
   * IR-50 is per-frame in eval mode, so every *unique* frame is encoded once and the 512-d
     embeddings are windowed, instead of re-encoding the 100-frame overlaps (33-50 % less conv work);
   * all windows of a video go through the head as one batch (the reference loops with bsz 1).
+
+The alternative heads CAN / JMT / MT have no windows: the reference runs them over the whole video with batch size
+1 (trainer.py:480-485).  ``infer_video`` / ``infer_videos`` give them those semantics (see :func:`infer_videos`).
 """
 from __future__ import annotations
 
@@ -86,7 +89,7 @@ def video_level_prediction(frame_logits: torch.Tensor, ignore_last_class: bool =
 @torch.no_grad()
 def infer_video(model, video: torch.Tensor, feats: Dict[str, torch.Tensor], window_length: int = 300,
                 hop_length: int = 200, fps: float = 30.0) -> torch.Tensor:
-    """One whole video through the LFAN mirror.
+    """One whole video through the LFAN mirror (or a CAN / JMT / MT: :func:`infer_videos` on this one video).
 
     video: [T,3,40,40] fp32 on the GPU (post eval-transform) or the stored uint8 [T,H,W,3] crops
     (then base/dataset.py:503-510 runs on the device, engine.PreprocEngine); feats[m]: [T, D_m] for
@@ -94,6 +97,8 @@ def infer_video(model, video: torch.Tensor, feats: Dict[str, torch.Tensor], wind
     'wave': the mono 16 kHz waveform, turned into one example per frame at ``fps`` on the device).  Returns per-frame logits [T, n_out] = the reference's stitched output.
     """
     from .engine import stitch_windows
+    if _is_feature_head(model):
+        return infer_videos(model, [video], [feats], window_length, hop_length, fps)[0]
     T = video.shape[0]
     if video.dtype == torch.uint8:                             # stored crops: the eval transform runs on the device
         video = preprocess_frames(model, video)
@@ -128,6 +133,58 @@ def window_index_table(lengths: Sequence[int], window_length: int = 300, hop_len
     return starts, torch.cat(rows)
 
 
+def padded_row_index(lengths: Sequence[int]):
+    """Videos laid end to end -> (T_max, int64 [sum(lengths)]): the row of each frame in a right-padded
+    [n_videos, T_max] batch (video i, frame t -> i * T_max + t), in concatenated order.  Scattering the concatenated
+    rows through it fills the padded batch; gathering through it takes the valid rows back."""
+    t_max = max((int(t) for t in lengths), default=0)
+    idx = [i * t_max + torch.arange(int(t)) for i, t in enumerate(lengths)]
+    return t_max, (torch.cat(idx) if idx else torch.empty(0, dtype=torch.int64))
+
+
+def _is_feature_head(model) -> bool:
+    from .heads import _FeatureHead
+    return isinstance(model, _FeatureHead)
+
+
+def _check_whole_videos(model, videos, feats, window_length: int, hop_length: int) -> List[int]:
+    """The inputs of CAN / JMT / MT whole-video inference, checked before any device work -> the video lengths."""
+    if (window_length, hop_length) != (300, 200):
+        raise ValueError(f"{type(model).__name__} runs over the whole video, it has no windows: window_length / "
+                         f"hop_length do not apply, got {window_length}, {hop_length}")
+    lengths = []
+    for i, (v, f) in enumerate(zip(videos, feats)):
+        T = int(v.shape[0])
+        if T == 0:
+            raise ValueError(f"video {i} is empty")
+        for m in model.modalities:
+            if m == "video":
+                continue
+            key = "wave" if m == "logmel" and m not in f and "wave" in f else m
+            if key not in f:
+                raise ValueError(f"video {i}: the head needs modality '{m}'" + (" (or 'wave')" if m == "logmel" else ""))
+            if key != "wave" and int(f[key].shape[0]) != T:
+                raise ValueError(f"video {i}: '{key}' has {int(f[key].shape[0])} rows for {T} frames")
+        lengths.append(T)
+    return lengths
+
+
+def _backbone_rows(model, videos, feats, lengths, modalities, fps: float) -> Dict[str, torch.Tensor]:
+    """The frames of all videos through the eval transform and IR-50 / VGGish back to back in full passes ->
+    src[m] [sum(lengths), D_m] in concatenated order (the non-visual feature rows concatenated as given)."""
+    src = {}
+    for m in modalities:
+        if m == "video":
+            frames = torch.cat([preprocess_frames(model, v) if v.dtype == torch.uint8 else v for v in videos])
+            src[m] = model.spatial["visual"](frames)                # every unique frame of every video once
+        elif m == "logmel":
+            ex = torch.cat([f[m] if m in f else wave_to_examples(model, f["wave"], t, fps) for f, t in zip(feats, lengths)])
+            src[m] = model.spatial["audio"](ex)
+        else:
+            src[m] = torch.cat([f[m] for f in feats])
+    return src
+
+
 @torch.no_grad()
 def infer_videos(model, videos: Sequence[torch.Tensor], feats: Sequence[Dict[str, torch.Tensor]], window_length: int = 300,
                  hop_length: int = 200, fps: float = 30.0, windows_per_pass: int = 16) -> List[torch.Tensor]:
@@ -137,25 +194,29 @@ def infer_videos(model, videos: Sequence[torch.Tensor], feats: Sequence[Dict[str
     the frames of all videos go through IR-50 / VGGish back to back in full passes, the windows of all
     videos go through the head in groups of ``windows_per_pass`` (one CUDA graph, the last group padded by
     repeating its last window) and only the stitch is per video.  Short videos stop paying for
-    partly-filled launches.  Returns one [T_i, n_out] tensor per video."""
+    partly-filled launches.  Returns one [T_i, n_out] tensor per video.
+
+    A CAN / JMT / MT runs over each whole video as the reference does (batch 1, no windows; ``window_length`` /
+    ``hop_length`` must stay at their defaults and ``windows_per_pass`` does not apply).  The backbone passes are
+    shared as above, the TCN runs on one right-padded batch, and the fusion head on the frames of all videos laid end
+    to end: CAN frame by frame, JMT / MT with every attention kept inside its video (engine.sdpa_segments).  A CAN's
+    result per video does not depend on the other videos in the call; a JMT / MT's agrees to fp32 reordering (its
+    row GEMMs pick split-K from the row count).  Every modality the head was built with is needed per video, with T
+    rows ('logmel' may come as 'wave'); an empty video is refused."""
     from .engine import stitch_windows
     if len(videos) != len(feats):
         raise ValueError("one feature dict per video")
+    whole = _is_feature_head(model)
+    if whole:
+        lengths = _check_whole_videos(model, videos, feats, window_length, hop_length)
     if not videos:
         return []
     dev = videos[0].device
+    if whole:
+        src = _backbone_rows(model, videos, feats, lengths, model.modalities, fps)
+        return list(model.forward_videos(src, lengths).split(lengths))
     lengths = [int(v.shape[0]) for v in videos]
-    frames = torch.cat([preprocess_frames(model, v) if v.dtype == torch.uint8 else v for v in videos])
-    src = {}
-    for m in model.modality:
-        if m == "video":
-            src[m] = model.spatial["visual"](frames)                # every unique frame of every video once
-        elif m == "logmel":
-            ex = torch.cat([f[m] if m in f else wave_to_examples(model, f["wave"], t, fps) for f, t in zip(feats, lengths)])
-            src[m] = model.spatial["audio"](ex)
-        else:
-            src[m] = torch.cat([f[m] for f in feats])
-    del frames
+    src = _backbone_rows(model, videos, feats, lengths, model.modality, fps)
     starts, idx = window_index_table(lengths, window_length, hop_length)
     idx = idx.to(dev, non_blocking=True)                            # [n_windows_total, window_length]
     n_win = idx.shape[0]

@@ -496,6 +496,15 @@ int cer_sdpa_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_
  * Any len_q / len_k (ragged tiles are masked).  Result within ~1e-3 of cer_sdpa_forward. */
 int cer_sdpa_tc_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev, int32_t ldv,
                         int32_t batch, int32_t len_q, int32_t len_k, int32_t dim, float* out_dev, int32_t ldo, void* stream);
+/* The same attention over the segments of one row buffer (the videos of a concatenated batch): for every s < n_seg,
+ * rows [seg_off[s], seg_off[s+1]) of out attend over rows [seg_off[s], seg_off[s+1]) of k / v only.  seg_off_dev:
+ * int32 [n_seg + 1] on the device, ascending from 0; no segment is longer than max_len (the caller's contract, not
+ * checked: the grid covers max_len query rows per segment).  Same dim / pitch / alignment conditions as
+ * cer_sdpa_tc_forward; n_seg <= 65535; n_seg == 0 is a no-op.  Segment s gives the same bits as
+ * cer_sdpa_tc_forward(batch 1, len_q = len_k = its length) on its rows alone. */
+int cer_sdpa_tc_seg_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev, int32_t ldv,
+                            const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len, int32_t dim, float* out_dev,
+                            int32_t ldo, void* stream);
 /* y = tanh(y) in place: the output squashing of task == REGRESSION (models/model.py:523, :682, :1165). */
 /* a += b over n contiguous fp32 values (where the gradients of two branches meet) */
 int cer_add_inplace(float* a_dev, const float* b_dev, int64_t n, void* stream);
