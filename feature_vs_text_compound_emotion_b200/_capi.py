@@ -211,6 +211,8 @@ SIGNATURES = {
                                      C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_stream_retain": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
                                     C.c_void_p, C.c_void_p]),
+    "cer_stream_append": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                    C.c_void_p, C.c_void_p]),
 }
 
 # int32 fields of cer_stream_entry, in order

@@ -129,6 +129,26 @@ __global__ void __launch_bounds__(kStreamThreads) stream_retain_kernel(
   }
 }
 
+// A JMT / MT stream's history: the chunk rows of each entry (src [n_entries][chunk][dim], a gather's output) go to
+// history [n_streams][max_frames][dim] at rows t_now .. t_now + chunk - 1.  Rows past max_frames and entries with a
+// sid outside [0, n_streams) are dropped (the host refuses such pushes), so nothing outside the range is written.
+__global__ void __launch_bounds__(kStreamThreads) stream_append_kernel(
+    const cer_stream_entry* __restrict__ tab, int n_entries, int chunk, const float* __restrict__ src, int dim,
+    int n_streams, int max_frames, float* __restrict__ history) {
+  const long long total = (long long)n_entries * chunk * dim;
+  for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)(idx % dim);
+    const long long er = idx / dim;
+    const int r = (int)(er % chunk);
+    const int ei = (int)(er / chunk);
+    const cer_stream_entry e = tab[ei];
+    const int f = e.t_now + r;
+    if (e.active && e.sid >= 0 && e.sid < n_streams && f >= 0 && f < max_frames)
+      history[((size_t)e.sid * max_frames + f) * dim + c] = src[idx];
+  }
+}
+
 static int grid_for(long long total) {
   const long long blocks = (total + kStreamThreads - 1) / kStreamThreads;
   return (int)(blocks < 148LL * 16 ? (blocks > 0 ? blocks : 1) : 148LL * 16);
@@ -187,6 +207,19 @@ extern "C" int cer_stream_retain(const cer_stream_entry* table_dev, int32_t n_st
   const long long total = (long long)n_streams * chunk * dim;
   stream_retain_kernel<<<grid_for(total), kStreamThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       table_dev, n_streams, n_slots, chunk, src_dev, dim, window_length, ring_dev);
+  CER_CUDA(cudaGetLastError());
+  return CER_OK;
+}
+
+extern "C" int cer_stream_append(const cer_stream_entry* table_dev, int32_t n_entries, int32_t chunk, const float* src_dev,
+                                 int32_t dim, int32_t n_streams, int32_t max_frames, float* history_dev, void* stream) {
+  using namespace cer;
+  if (!table_dev || !src_dev || !history_dev || n_entries <= 0 || chunk <= 0 || dim <= 0 || n_streams <= 0 ||
+      max_frames <= 0)
+    return set_error(CER_ERR_INVALID, "cer_stream_append: bad argument");
+  const long long total = (long long)n_entries * chunk * dim;
+  stream_append_kernel<<<grid_for(total), kStreamThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      table_dev, n_entries, chunk, src_dev, dim, n_streams, max_frames, history_dev);
   CER_CUDA(cudaGetLastError());
   return CER_OK;
 }

@@ -25,6 +25,12 @@ starts at frame 0 and never ends, ``push`` returns final logits (``final_upto`` 
 returns only what was still held back.  The fusion head + tail run as one row-invariant kernel
 (cer_can_head_forward), so a stream's logits do not depend on the other streams of a push or on its chunk sizes
 (DESIGN.md section 5.18).
+
+A JMT / MT (opened with ``max_frames``) attends over the whole sequence, so no logit is final before the stream ends.
+Its backbones and causal TCN + BatchNorm1d still run as frames arrive, through CAN's continuous step, and each
+stream keeps the TCN output rows on the device (its history).  ``push`` returns no logits; ``peek`` runs the fusion
+over the history of the listed streams as if they ended now, and ``close`` does so for one stream and frees it
+(DESIGN.md section 5.20).
 """
 from __future__ import annotations
 
@@ -93,6 +99,23 @@ def continuous_step_table(streams: Sequence[Tuple[int, int, int]]) -> np.ndarray
     for i, (sid, t_now, parity) in enumerate(streams):
         tab[i, 0], tab[i, 4], tab[i, 5], tab[i, 6] = sid, t_now, parity, 1
     return tab
+
+
+def history_overflow(lengths: Sequence[int], chunk: int, max_frames: int) -> List[int]:
+    """Positions in ``lengths`` of the streams that a push of ``chunk`` frames would take past ``max_frames``."""
+    return [i for i, t in enumerate(lengths) if int(t) + chunk > max_frames]
+
+
+def history_row_index(sids: Sequence[int], lengths: Sequence[int], max_frames: int) -> torch.Tensor:
+    """Rows of the [streams * max_frames] history view holding the first lengths[i] frames of stream sids[i], laid
+    end to end in list order (stream sid, frame t -> sid * max_frames + t): int64 [sum(lengths)]."""
+    idx = [int(s) * max_frames + torch.arange(int(t)) for s, t in zip(sids, lengths)]
+    return torch.cat(idx) if idx else torch.empty(0, dtype=torch.int64)
+
+
+def history_bytes(channels: Sequence[int], max_frames: int) -> int:
+    """Device bytes of one JMT / MT stream's history: max_frames fp32 rows of each modality's last TCN channel count."""
+    return 4 * max_frames * sum(int(c) for c in channels)
 
 
 def step_table(streams: Sequence[Tuple[int, int, int]], chunk: int, window_length: int, hop_length: int,
@@ -217,23 +240,46 @@ class StreamSession:
     offline edge padding, so the examples are windowing.wave_to_examples' (DESIGN.md section 5.17).
 
     With a CAN the logits ``push`` returns are final; ``window_length`` / ``hop_length`` do not apply and must stay
-    at their defaults (see the module docstring)."""
+    at their defaults (see the module docstring).
+
+    A JMT / MT needs ``max_frames``, the most frames any stream of the session will carry: each stream keeps the
+    [max_frames, C_m] TCN + BatchNorm1d output rows of every modality on the device (``state_bytes()`` counts them).
+    Inputs are the model's modalities: 'video' as above and 'vggish' rows [n, c, 128] ('logmel' / ``wave_fps`` do
+    not apply).  No frame is final before the stream ends, so ``push`` returns (logits [n, 0, n_out], [0] * n);
+    ``peek(ids)`` returns per stream the whole-video logits [T_i, n_out] of the frames pushed so far, as if the
+    stream ended now, from one fusion pass over all listed streams (JMT._fuse_videos, every attention inside its
+    stream); ``close(sid)`` returns the same for one stream and frees it.  With equal backbone embeddings (always for
+    'vggish' rows; for 'video' when the IR-50 plan picks the same kernels at both pass sizes, e.g. CER_RASTER=0),
+    ``close`` and a one-stream ``peek`` equal ``windowing.infer_video`` on the same frames bit for bit: the
+    continuous TCN rows are the offline rows, and the fusion on one stream of T rows is the launch sequence
+    infer_videos runs for one video.  A peek of several streams agrees with per-stream peeks to fp32 reordering (the
+    fusion's row GEMMs pick split-K from the total row count).  A push that would take a stream past ``max_frames``
+    is refused before any state changes (DESIGN.md section 5.20)."""
 
     def __init__(self, model, max_streams: int = 256, max_chunk: int = 30, window_length: int = 300,
-                 hop_length: int = 200, wave_fps: float = None):
-        from .heads import CAN
+                 hop_length: int = 200, wave_fps: float = None, max_frames: int = None):
+        from .heads import CAN, JMT
         from .modules import LFAN
-        if not isinstance(model, (LFAN, CAN)):
-            raise TypeError("StreamSession streams LFAN and CAN only: the JMT / MT heads are not streamed (JMT / MT attend "
-                            "over the whole window, so a frame's logits depend on later frames)")
-        self.continuous = isinstance(model, CAN)          # no windows: one never-ending TCN slot per stream
+        self.whole = isinstance(model, JMT)                # JMT / MT: TCN rows kept, fusion over them at peek / close
+        if not (isinstance(model, (LFAN, CAN)) or (self.whole and max_frames is not None)):
+            raise TypeError("StreamSession streams LFAN and CAN as they arrive, and JMT / MT only with max_frames (JMT / MT "
+                            "attend over the whole window, so a frame's logits depend on later frames): open a JMT / MT "
+                            "session as StreamSession(model, max_streams, max_chunk, max_frames=F), F the longest "
+                            "stream, and read whole-stream logits with peek / close")
+        if max_frames is not None and not self.whole:
+            raise ValueError("max_frames applies to JMT / MT sessions only (an LFAN / CAN stream keeps no history)")
+        if self.whole and int(max_frames) < 1:
+            raise ValueError(f"max_frames must be positive, got {max_frames}")
+        self.continuous = isinstance(model, (CAN, JMT))   # no windows: one never-ending TCN slot per stream
         if self.continuous and (window_length, hop_length) != (300, 200):
-            raise ValueError("a CAN stream has no windows: window_length / hop_length do not apply, got "
+            name = getattr(model, "model_name", type(model).__name__)
+            raise ValueError(f"a {name} stream has no windows: window_length / hop_length do not apply, got "
                              f"{window_length}, {hop_length}")
         if not (1 <= hop_length <= window_length):
             raise ValueError(f"need 1 <= hop_length <= window_length, got {hop_length}, {window_length}")
         if max_streams < 1 or max_chunk < 1:
             raise ValueError("max_streams and max_chunk must be positive")
+        self.max_frames = int(max_frames) if self.whole else None
         _capi.require_gpu()
         self.model = model
         self._check_model()
@@ -288,22 +334,23 @@ class StreamSession:
             raise RuntimeError("StreamSession runs the inference kernels: call model.eval() first")
 
     def _pack(self):
-        """(Re)bind the model's packed head (LFAN: its FusionEngine; CAN: CAN.frame_head); allocate the rings and step
-        buffers on first use."""
+        """(Re)bind the model's packed head (LFAN: its FusionEngine; CAN: CAN.frame_head; JMT / MT: none, the fusion
+        runs at peek / close); allocate the rings, histories and step buffers on first use."""
         self._eng, self._graphs = self._model_engines(), {}
         tcn = self._eng[0]
-        self._head = self.model.frame_head() if self.continuous else self._eng[1]
+        self._head = None if self.whole else self.model.frame_head() if self.continuous else self._eng[1]
         self._tanh = self.continuous and self.model.task == "REGRESSION"
         dev, S, ne, cm = self.device, self.max_streams, self.max_streams * self.n_slots, self.max_chunk
         f32 = dict(dtype=torch.float32, device=dev)
-        self.n_out = self._head.n_out
+        self.n_out = self.model.fc2.out_features if self.whole else self._head.n_out
         fresh = not hasattr(self, "_tab")
         if fresh:
             self._tab = torch.zeros(ne, len(_capi.STREAM_ENTRY_FIELDS), dtype=torch.int32, device=dev)
             if not self.continuous:
                 self._lring = torch.zeros(S, self.n_lslots, self.W, self.n_out, **f32)
-            self._out = torch.empty(S * cm * self.n_out, **f32)
+            self._out = torch.empty(0 if self.whole else S * cm * self.n_out, **f32)
             self._in, self._inring, self._rings, self._staged, self._outs, self._ws, self._gath = {}, {}, {}, {}, {}, {}, {}
+            self._hist = {}
         self._blocks, self._rows, self._dims = {}, {}, {}
         for m in self.modalities:
             eng = tcn[m]
@@ -324,6 +371,8 @@ class StreamSession:
             self._ws[m] = torch.empty(max(ne * (r + cm) * b.c_out for b, r in zip(blocks, rows)) * 4, dtype=torch.uint8,
                                       device=dev)
             self._gath[m] = torch.empty(ne * cm * eng.c_out, **f32)
+            if self.whole:
+                self._hist[m] = torch.zeros(S, self.max_frames, blocks[-1].c_out, **f32)
 
     def _engines(self):
         eng = self._model_engines()
@@ -332,6 +381,8 @@ class StreamSession:
         return self._eng
 
     def _final_upto(self, emitted: int) -> int:
+        if self.whole:
+            return 0
         return emitted if self.continuous else final_upto(emitted, self.W)
 
     def state_bytes(self) -> int:
@@ -343,6 +394,8 @@ class StreamSession:
             n += sum(self.n_slots * 2 * r * b.c_in for b, r in zip(self._blocks[m], self._rows[m]))
         if self.wave_fps is not None:
             n += self.tail_len + self.n_lm_rows * LOGMEL["n_mel"] + sum(h.shape[1] * h.shape[2] for h in self._hold.values())
+        if self.whole:
+            return 4 * n + history_bytes([self._blocks[m][-1].c_out for m in self.modalities], self.max_frames)
         return 4 * n
 
     def open(self) -> int:
@@ -420,6 +473,11 @@ class StreamSession:
             g = self._gath[m]
             chk(lib.cer_stream_gather(tab, ne, c, src.data_ptr(), src_rows, src_dim, g.data_ptr(), st), "cer_stream_gather")
             feats.append(g[:ne * c * src_dim].view(ne * c, src_dim))
+        if self.whole:                              # JMT / MT: the rows join each stream's history (peek / close fuse it)
+            for m, f in zip(self.modalities, feats):
+                chk(lib.cer_stream_append(tab, ne, c, f.data_ptr(), f.shape[1], self.max_streams, self.max_frames,
+                                          self._hist[m].data_ptr(), st), "cer_stream_append")
+            return
         if self.continuous:                         # per-frame and final: straight into the output buffer
             self._head.forward(feats, self._tanh, out=self._out[:n * c * self.n_out].view(n * c, self.n_out))
             return
@@ -438,7 +496,10 @@ class StreamSession:
         With wave_fps: -> (a list of n tensors [r_i, n_out], the provisional logits of the frames this push
         released, continuing from emitted(i); final_upto = max(0, emitted(i) - W) per stream).
 
-        With a CAN every returned logit is final: final_upto = emitted(i)."""
+        With a CAN every returned logit is final: final_upto = emitted(i).
+
+        With a JMT / MT no logit is final before close: -> (logits [n, 0, n_out], [0] * n); the frames' TCN rows join
+        the streams' histories (read them through peek / close)."""
         self._check_model()
         ids = [int(i) for i in ids]
         n = len(ids)
@@ -446,6 +507,13 @@ class StreamSession:
             raise ValueError("push needs at least one stream")
         if len(set(ids)) != n or any(i not in self._len for i in ids):
             raise ValueError(f"stream ids must be distinct open streams, got {ids}")
+        if self.whole:                              # every stream's bound, before any state changes
+            x0 = inputs.get(self.modalities[0])
+            c = int(x0.shape[1]) if isinstance(x0, torch.Tensor) and x0.dim() >= 2 else 0
+            over = [ids[j] for j in history_overflow([self._len[i] for i in ids], c, self.max_frames)]
+            if over:
+                raise ValueError(f"streams {over}: a push of {c} frames would take them past max_frames = "
+                                 f"{self.max_frames} (lengths {[self._len[i] for i in over]})")
         self._engines()
         if self.wave_fps is not None:
             return self._push_wave(ids, inputs)
@@ -486,7 +554,8 @@ class StreamSession:
                     self._graphs[(n, c)] = graph
                 except Exception:                     # capture not possible here: stay eager for this shape
                     self._graphs[(n, c)] = False
-        out = self._out[:n * c * self.n_out].view(n, c, self.n_out).clone()
+        out = (self._out.new_empty(n, 0, self.n_out) if self.whole else
+               self._out[:n * c * self.n_out].view(n, c, self.n_out).clone())
         for i in ids:
             self._emitted[i] += c
             self._parity[i] ^= 1
@@ -615,17 +684,54 @@ class StreamSession:
         n_ex = n_examples_total(logmel_rows(A + pad.numel()), self.wave_fps)
         return self._release([(sid, E, T - E, n_ex)]).get(sid, [])
 
+    # -- JMT / MT: whole-stream logits -----------------------------------------------------------
+    @torch.no_grad()
+    def peek(self, ids: Sequence[int]) -> List[torch.Tensor]:
+        """JMT / MT sessions: per listed open stream the whole-video logits [T_i, n_out] of the frames pushed so far,
+        as if the stream ended now ([0, n_out] for a stream with no frames).  One fusion pass over all listed streams;
+        the streams stay open."""
+        if not self.whole:
+            raise TypeError("peek reads the whole-stream logits of a JMT / MT session; an LFAN / CAN session returns "
+                            "its logits from push and close")
+        ids = [int(i) for i in ids]
+        if len(set(ids)) != len(ids) or any(i not in self._len for i in ids):
+            raise ValueError(f"stream ids must be distinct open streams, got {ids}")
+        self._check_model()
+        self._engines()
+        return self._whole_logits(ids)
+
+    def _whole_logits(self, ids: List[int]) -> List[torch.Tensor]:
+        """The history rows of streams ``ids`` laid end to end through JMT._fuse_videos (the function infer_videos
+        runs), so every attention stays inside its stream."""
+        lengths = [self._len[i] for i in ids]
+        live = [(i, t) for i, t in zip(ids, lengths) if t > 0]
+        out = iter([])
+        if live:
+            sids, lens = [i for i, _ in live], [t for _, t in live]
+            with torch.cuda.device(self.device):
+                idx = history_row_index(sids, lens, self.max_frames).to(self.device, non_blocking=True)
+                z = {m: self._hist[m].view(-1, self._hist[m].shape[-1]).index_select(0, idx) for m in self.modalities}
+                out = iter(self.model._fuse_videos(z, lens).split(lens))
+        return [next(out) if t > 0 else torch.empty(0, self.n_out, dtype=torch.float32, device=self.device)
+                for t in lengths]
+
     # -- close ------------------------------------------------------------------------------
     @torch.no_grad()
     def close(self, sid: int) -> torch.Tensor:
         """End stream ``sid`` -> the final logits [min(T, W), n_out] of its frames T - min(T, W) .. T - 1, and free
         its slot.  With a CAN: the logits of the frames not returned yet ([0, n_out] without wave_fps; the
-        held-back frames with it)."""
+        held-back frames with it).  With a JMT / MT: the whole-video logits [T, n_out] of every frame, as
+        ``peek([sid])`` computes them."""
         from .engine import stitch_windows
         if sid not in self._len:
             raise ValueError(f"stream {sid} is not open")
         self._check_model()
         self._engines()
+        if self.whole:
+            out = self._whole_logits([sid])[0]
+            del self._len[sid], self._parity[sid], self._emitted[sid]
+            self._free.append(sid)
+            return out
         flushed = []
         if self.wave_fps is not None and self._len[sid] > 0:
             if self._samples[sid] == 0:

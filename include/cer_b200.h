@@ -578,6 +578,12 @@ int cer_stream_average(const cer_stream_entry* table_dev, int32_t n_streams, int
  * frame mod window_length. */
 int cer_stream_retain(const cer_stream_entry* table_dev, int32_t n_streams, int32_t n_slots, int32_t chunk,
                       const float* src_dev, int32_t dim, int32_t window_length, float* ring_dev, void* stream);
+/* A JMT / MT stream's history: the chunk rows src [n_entries][chunk][dim] (a gather's output) ->
+ * history [n_streams][max_frames][dim] at rows t_now .. t_now + chunk - 1 of each active entry's
+ * sid.  Nothing else is written: rows at or past max_frames and sids outside [0, n_streams) are
+ * dropped. */
+int cer_stream_append(const cer_stream_entry* table_dev, int32_t n_entries, int32_t chunk, const float* src_dev,
+                      int32_t dim, int32_t n_streams, int32_t max_frames, float* history_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -31,6 +31,17 @@ logits, at (n, c) in {1x1, 1x30, 32x8, 32x30, 256x1, 256x8, 256x30}; head kernel
 can_head_kernel.  The same run times can_head_kernel alone at 7 680 rows (CUDA events over repeated launches on one
 set of inputs, so its 1.4 MB of weights are L2-resident as in a step) and reports GFLOP/s from the shape-derived
 FLOP count.  infer_videos is not run in this mode.
+
+    python tools/stream_bench.py --head jmt --out profiles/r07_stream_jmt.json
+
+streams a JMT (or MT, --head mt) instead (DESIGN.md section 5.20): 'video' (fp32 40 px crops) + 'vggish' rows with
+synthetic.TCN_SETTINGS, one session of 256 slots, chunks up to 30 and max_frames 6000.
+1. The push step (backbones + continuous TCN + cer_stream_append) at 1x1, 32x8 and 256x30, timed as above.
+2. peek over all open streams at 300, 1000 and 3000 frames per stream, for 1, 32 and 256 streams (host clock around
+   the call, which ends in a device synchronise: its logits are read); the attention FLOPs of one peek (5 attentions
+   per stream, 4 T^2 E each, E = 128) beside it.
+3. close of one 3000-frame stream against windowing.infer_video on the same whole video started at end of stream,
+   alternated, with the largest difference between their logits.
 """
 from __future__ import annotations
 
@@ -86,6 +97,108 @@ def can(dev, mods=MODS):
     return m.to(dev).eval()
 
 
+def jmt(dev, name):
+    from feature_vs_text_compound_emotion_b200.models.model import JMT
+    mods = ["video", "vggish"]
+    m = JMT(task="CLASSIFICATION", modalities=mods, tcn_settings=synthetic.TCN_SETTINGS,
+            backbone_settings={"visual_state_dict": "", "audio_state_dict": ""}, output_dim=7, root_dir="", device=dev,
+            model_name=name, visual_state_dict=synthetic.visual_backbone_state_dict(0))
+    m.load_state_dict(synthetic.jmt_state_dict(0, mods, model_name=name), strict=True)
+    return m.to(dev).eval()
+
+
+def timed_call(fn, reps):
+    """Median and all wall times (ms) of fn() over reps calls, each ending in a device synchronise."""
+    ts = []
+    for _ in range(reps):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        fn()
+        torch.cuda.synchronize()
+        ts.append((time.perf_counter() - t0) * 1e3)
+    return sorted(ts)[len(ts) // 2], ts
+
+
+def whole_stream_bench(args, m, dev, rec):
+    """--head jmt / mt: push step, peek and close against infer_video (see the module docstring)."""
+    max_frames, E = 6000, 128
+    sess = streaming.StreamSession(m, max_streams=256, max_chunk=30, max_frames=max_frames)
+    rec.update({"max_frames": max_frames, "state_bytes_per_stream": sess.state_bytes(),
+                "tcn_settings": {k: synthetic.TCN_SETTINGS[k] for k in m.modalities}, "configs": [], "peek": [],
+                "close_vs_infer_video": {}})
+    for n, c in ((1, 1), (32, 8), (256, 30)):
+        ids = [sess.open() for _ in range(n)]
+        pool = [chunk_inputs(n, c, dev, 10 * n + c + k, bert=False) for k in range(4)]
+        for k in range(6):
+            sess.push(ids, pool[k % 4])
+        torch.cuda.synchronize()
+        times, t0, k = [], time.perf_counter(), 0
+        while ((time.perf_counter() - t0 < args.window or len(times) < 20)
+               and sess.length(ids[0]) + c <= max_frames):
+            s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            s.record()
+            sess.push(ids, pool[k % 4])
+            e.record()
+            e.synchronize()
+            times.append(s.elapsed_time(e))
+            k += 1
+        ts = sorted(times)
+        mean, med = sum(ts) / len(ts), ts[len(ts) // 2]
+        cfg = {"streams": n, "chunk": c, "steps": len(ts), "median_ms": med,
+               "p99_ms": ts[min(len(ts) - 1, int(0.99 * len(ts)))],
+               "frames_per_s_median": n * c / (med / 1e3), "frames_per_s_mean": n * c / (mean / 1e3)}
+        rec["configs"].append(cfg)
+        print(json.dumps(cfg), flush=True)
+        for i in ids:
+            sess.close(i)
+    for n in (1, 32, 256):
+        ids = [sess.open() for _ in range(n)]
+        pool = [chunk_inputs(n, 30, dev, 1000 + n + k, bert=False) for k in range(4)]
+        k = 0
+        for T in (300, 1000, 3000):
+            while sess.length(ids[0]) < T:
+                sess.push(ids, pool[k % 4])
+                k += 1
+            sess.peek(ids)                                        # warm-up at this shape
+            med, ts = timed_call(lambda: sess.peek(ids), 5 if n * T < 100000 else 3)
+            flop = 5 * 4 * n * T * T * E
+            cfg = {"streams": n, "frames_per_stream": T, "median_ms": med, "times_ms": [round(t, 3) for t in ts],
+                   "attention_gflop": flop / 1e9, "attention_tflop_per_s": flop / (med / 1e3) / 1e12}
+            rec["peek"].append(cfg)
+            print(json.dumps(cfg), flush=True)
+        for i in ids:
+            sess.close(i)
+    T = 3000
+    g = torch.Generator(device=dev).manual_seed(5)
+    video = torch.rand(T, 3, 40, 40, device=dev, generator=g) * 2 - 1
+    vgg = torch.randn(T, 128, device=dev, generator=g)
+    windowing.infer_video(m, video, {"vggish": vgg})              # warm-up: plans for the 3000-frame passes
+    close_ms, infer_ms, diff = [], [], 0.0
+    for _ in range(4):
+        sid = sess.open()
+        for a in range(0, T, 30):
+            sess.push([sid], {"video": video[None, a:a + 30], "vggish": vgg[None, a:a + 30]})
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        got = sess.close(sid)
+        torch.cuda.synchronize()
+        close_ms.append((time.perf_counter() - t0) * 1e3)
+        t0 = time.perf_counter()
+        want = windowing.infer_video(m, video, {"vggish": vgg})
+        torch.cuda.synchronize()
+        infer_ms.append((time.perf_counter() - t0) * 1e3)
+        diff = max(diff, (got - want).abs().max().item())
+    rec["close_vs_infer_video"] = {
+        "frames": T, "reps": len(close_ms), "close_ms": [round(t, 3) for t in close_ms],
+        "infer_video_ms": [round(t, 3) for t in infer_ms], "close_median_ms": sorted(close_ms)[len(close_ms) // 2],
+        "infer_video_median_ms": sorted(infer_ms)[len(infer_ms) // 2], "max_abs_diff": diff,
+        "note": "default IR-50 plan (CER_RASTER unset): the push passes and the 3000-frame pass may pick other kernels"}
+    print(json.dumps(rec["close_vs_infer_video"]), flush=True)
+    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+    with open(args.out, "w") as f:
+        json.dump(rec, f, indent=1)
+
+
 def can_head_flop(m) -> int:
     """FLOPs of one frame through cer_can_head_forward: the four GEMVs (softmax, activation and bias not counted)."""
     D = 128 * len(m.modalities)
@@ -112,10 +225,11 @@ def time_can_head(m, dev, rows=7680, reps=200):
             "gflop_per_s": flop / (us * 1e-6) / 1e9}
 
 
-def chunk_inputs(n, c, dev, seed, wave=False):
+def chunk_inputs(n, c, dev, seed, wave=False, bert=True):
     g = torch.Generator(device=dev).manual_seed(seed)
-    x = {"video": torch.rand(n, c, 3, 40, 40, device=dev, generator=g) * 2 - 1,
-         "bert": torch.randn(n, c, 768, device=dev, generator=g)}
+    x = {"video": torch.rand(n, c, 3, 40, 40, device=dev, generator=g) * 2 - 1}
+    if bert:
+        x["bert"] = torch.randn(n, c, 768, device=dev, generator=g)
     if wave:      # one 30-frame second of samples per stream; each push slices what is in step with its frames
         x["_wave"] = torch.randn(n, 16000, device=dev, generator=g) * 0.3
     else:
@@ -150,13 +264,19 @@ def main():
     ap.add_argument("--window", type=float, default=2.0)
     ap.add_argument("--audio", choices=("vggish", "wave"), default="vggish",
                     help="wave: stream raw audio (logmel from the waveform) instead of pre-extracted vggish features")
-    ap.add_argument("--head", choices=("lfan", "can"), default="lfan")
+    ap.add_argument("--head", choices=("lfan", "can", "jmt", "mt"), default="lfan")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("stream_bench measures the B200 kernels: no CUDA device")
     dev = torch.device("cuda:0")
     torch.set_grad_enabled(False)
     wave = args.audio == "wave"
+    if args.head in ("jmt", "mt"):
+        if wave:
+            raise SystemExit("--head jmt / mt streams pre-extracted vggish features")
+        m = jmt(dev, args.head.upper())
+        whole_stream_bench(args, m, dev, {"card": card(), "head": args.head, "modalities": m.modalities})
+        return
     is_can = args.head == "can"
     if wave and is_can:
         raise SystemExit("--head can streams pre-extracted vggish features")
