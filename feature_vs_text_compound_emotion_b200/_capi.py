@@ -106,6 +106,18 @@ class CanHeadWeights(C.Structure):
                 ("fc2_w", C.c_void_p), ("fc2_b", C.c_void_p)]
 
 
+class BertLayer(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("wqkv", "bqkv", "wo", "bo", "ln1_g", "ln1_b", "w1", "b1", "w2", "b2", "ln2_g",
+                                          "ln2_b")]
+
+
+class BertWeights(C.Structure):
+    _fields_ = [("hidden", C.c_int32), ("intermediate", C.c_int32), ("n_heads", C.c_int32), ("n_layers", C.c_int32),
+                ("vocab", C.c_int32), ("max_pos", C.c_int32), ("type_vocab", C.c_int32), ("ln_eps", C.c_float),
+                ("word_emb", C.c_void_p), ("pos_emb", C.c_void_p), ("type_emb", C.c_void_p), ("emb_ln_g", C.c_void_p),
+                ("emb_ln_b", C.c_void_p), ("layers", C.POINTER(BertLayer))]
+
+
 # name -> (restype, argtypes); mirrors include/cer_b200.h one to one
 SIGNATURES = {
     "cer_last_error": (C.c_char_p, []),
@@ -193,6 +205,18 @@ SIGNATURES = {
                                       C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_sdpa_tc_seg_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
                                           C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "cer_sdpa_tc_seg_heads_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                                C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "cer_bert_workspace_bytes": (C.c_size_t, [C.POINTER(BertWeights), C.c_int64]),
+    "cer_bert_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(BertWeights), C.c_int64, C.c_void_p, C.c_size_t]),
+    "cer_bert_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p,
+                                   C.c_void_p]),
+    "cer_bert_destroy": (None, [C.c_void_p]),
+    "cer_bert_embed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "cer_bert_linear": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                  C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cer_text_frames": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
+                                  C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_add_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float,
                                     C.c_void_p, C.c_void_p]),
     "cer_modal_attention_maps": (C.c_int, [C.POINTER(C.c_void_p), C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),

@@ -11,7 +11,7 @@ void set_head_variant(const char* name) { g_head_variant = name; }
 }  // namespace cer
 
 extern "C" const char* cer_last_error(void) { return cer::g_last_error.c_str(); }
-extern "C" int cer_version(void) { return 108; }
+extern "C" int cer_version(void) { return 109; }
 extern "C" const char* cer_head_last_variant(void) { return cer::g_head_variant; }
 
 extern "C" int cer_check_device(void) {

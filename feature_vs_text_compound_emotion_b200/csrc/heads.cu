@@ -109,7 +109,9 @@ __device__ __forceinline__ void mma_tf32(float (&d)[4], uint32_t a0, uint32_t a1
 //   len_q = len_k = that length (self- or cross-attention inside one video of a concatenated batch).  A CTA past
 //   its segment's end returns before any load or barrier; every other instruction is the uniform kernel's, so a
 //   segment gives the same bits as a batch-1 launch on it alone.
-template <int E, bool kSeg>
+//   kHeads (segmented only): blockIdx.z is a head h; q, k, v and out start E * h columns further into their rows
+//   (head h of a multi-head projection through the same row pitches).  Otherwise the code is kSeg's.
+template <int E, bool kSeg, bool kHeads = false>
 __global__ void __launch_bounds__(128) sdpa_tc_kernel(const float* __restrict__ q, int ldq, const float* __restrict__ k, int ldk,
                                                       const float* __restrict__ v, int ldv, int len_q, int len_k,
                                                       float* __restrict__ out, int ldo, const int* __restrict__ seg_off) {
@@ -130,6 +132,11 @@ __global__ void __launch_bounds__(128) sdpa_tc_kernel(const float* __restrict__ 
   } else {
     row_q = (long long)b * len_q;
     row_k = (long long)b * len_k;
+  }
+  if constexpr (kHeads) {
+    static_assert(kSeg, "head batching is a form of the segmented kernel");
+    const int col = E * blockIdx.z;
+    q += col; k += col; v += col; out += col;
   }
   const float* qb = q + row_q * ldq;
   const float* kb = k + row_k * ldk;
@@ -322,17 +329,17 @@ extern "C" int cer_sdpa_forward(const float* q_dev, int32_t ldq, const float* k_
   return CER_OK;
 }
 
-// Uniform: grid (ceil(len_q / 64), batch).  Segmented (seg_off != null): grid (ceil(len_q / 64), n_seg), len_q the
-// longest segment.
-template <int E, bool kSeg>
+// Uniform: grid (ceil(len_q / 64), batch).  Segmented (seg_off != null): grid (ceil(len_q / 64), n_seg, heads), len_q
+// the longest segment.
+template <int E, bool kSeg, bool kHeads = false>
 static int launch_sdpa_tc(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, int batch, int len_q, int len_k,
-                          float* out, int ldo, const int* seg_off, cudaStream_t st) {
+                          float* out, int ldo, const int* seg_off, cudaStream_t st, int heads = 1) {
   const size_t smem = (size_t)(kSdpaQ + 2 * kSdpaK) * (E + 4) * sizeof(float);
   static unsigned long long configured = 0;
   if (first_use_on_device(&configured))
-    CER_CUDA(cudaFuncSetAttribute(sdpa_tc_kernel<E, kSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  dim3 grid((len_q + kSdpaQ - 1) / kSdpaQ, batch);
-  sdpa_tc_kernel<E, kSeg><<<grid, 128, smem, st>>>(q, ldq, k, ldk, v, ldv, len_q, len_k, out, ldo, seg_off);
+    CER_CUDA(cudaFuncSetAttribute(sdpa_tc_kernel<E, kSeg, kHeads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  dim3 grid((len_q + kSdpaQ - 1) / kSdpaQ, batch, heads);
+  sdpa_tc_kernel<E, kSeg, kHeads><<<grid, 128, smem, st>>>(q, ldq, k, ldk, v, ldv, len_q, len_k, out, ldo, seg_off);
   CER_CUDA(cudaGetLastError());
   return CER_OK;
 }
@@ -374,6 +381,21 @@ extern "C" int cer_sdpa_tc_seg_forward(const float* q_dev, int32_t ldq, const fl
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   return dim == 128 ? launch_sdpa_tc<128, true>(q_dev, ldq, k_dev, ldk, v_dev, ldv, n_seg, max_len, max_len, out_dev, ldo, seg_off_dev, st)
                     : launch_sdpa_tc<64, true>(q_dev, ldq, k_dev, ldk, v_dev, ldv, n_seg, max_len, max_len, out_dev, ldo, seg_off_dev, st);
+}
+
+extern "C" int cer_sdpa_tc_seg_heads_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev,
+                                             int32_t ldv, const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len, int32_t dim,
+                                             int32_t heads, float* out_dev, int32_t ldo, void* stream) {
+  if (!q_dev || !k_dev || !v_dev || !out_dev || !seg_off_dev || n_seg < 0 || max_len < 0 || heads <= 0 || heads > 64 ||
+      ldq < dim * heads || ldk < dim * heads || ldv < dim * heads || ldo < dim * heads)
+    return set_error(CER_ERR_INVALID, "cer_sdpa_tc_seg_heads_forward: bad argument (1 <= heads <= 64, pitches >= dim * heads)");
+  if (n_seg > 65535) return set_error(CER_ERR_INVALID, "cer_sdpa_tc_seg_heads_forward: more than 65535 segments (the grid's y limit)");
+  if (dim != 64) return set_error(CER_ERR_INVALID, "cer_sdpa_tc_seg_heads_forward: dim must be 64");
+  int rc = check_sdpa_tc("cer_sdpa_tc_seg_heads_forward", q_dev, ldq, k_dev, ldk, v_dev, ldv, dim, out_dev, ldo);
+  if (rc) return rc;
+  if (n_seg == 0 || max_len == 0) return CER_OK;
+  return launch_sdpa_tc<64, true, true>(q_dev, ldq, k_dev, ldk, v_dev, ldv, n_seg, max_len, max_len, out_dev, ldo, seg_off_dev,
+                                        static_cast<cudaStream_t>(stream), heads);
 }
 
 extern "C" int cer_add_layernorm(const float* x_dev, const float* res_dev, int64_t rows, int32_t dim, const float* gamma_dev,

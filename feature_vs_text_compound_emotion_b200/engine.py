@@ -415,6 +415,131 @@ class CanHeadEngine:
         return out
 
 
+class BertEngine:
+    """BERT text encoder plan (cer_bert_*): transcripts of WordPiece ids -> per token the sum of the last four hidden
+    states, [n_tokens, hidden] fp32.  ``packed`` is packing.pack_bert's output; ``cfg`` holds hidden, intermediate,
+    n_heads, vocab, max_pos, type_vocab and ln_eps.  The workspace grows with the largest call seen (max_tokens)."""
+
+    def __init__(self, packed: dict, cfg: dict, device: torch.device):
+        _capi.require_gpu()
+        self.device = torch.device(device)
+        self._keep: List[torch.Tensor] = []
+
+        def put(t):
+            d = t.to(self.device).contiguous()
+            self._keep.append(d)
+            return d.data_ptr()
+
+        layers = packed["layers"]
+        self._layers = (_capi.BertLayer * len(layers))()
+        for i, l in enumerate(layers):
+            self._layers[i] = _capi.BertLayer(*[put(l[n]) for n in ("wqkv", "bqkv", "wo", "bo", "ln1_g", "ln1_b", "w1", "b1",
+                                                                     "w2", "b2", "ln2_g", "ln2_b")])
+        self._w = _capi.BertWeights(cfg["hidden"], cfg["intermediate"], cfg["n_heads"], len(layers), cfg["vocab"],
+                                    cfg["max_pos"], cfg["type_vocab"], cfg["ln_eps"], put(packed["word_emb"]),
+                                    put(packed["pos_emb"]), put(packed["type_emb"]), put(packed["emb_ln_g"]),
+                                    put(packed["emb_ln_b"]), self._layers)
+        self.hidden = cfg["hidden"]
+        self.max_tokens = 0
+        self._h = None
+        self._ws = None
+
+    def _plan(self, n_tokens: int):
+        if n_tokens <= self.max_tokens:
+            return self._h
+        self._destroy()
+        n = max(n_tokens, 2 * self.max_tokens, 1024)
+        with torch.cuda.device(self.device):
+            nbytes = lib().cer_bert_workspace_bytes(C.byref(self._w), n)
+            self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+            h = C.c_void_p()
+            check(lib().cer_bert_create(C.byref(h), C.byref(self._w), n, self._ws.data_ptr(), nbytes), "cer_bert_create")
+        self._h, self.max_tokens = h, n
+        return h
+
+    def forward(self, ids: torch.Tensor, seg: "Segments", out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """ids: int64 [seg.rows] on the engine's device, the transcripts end to end -> [seg.rows, hidden] fp32."""
+        if ids.dim() != 1 or ids.dtype != torch.int64 or ids.device != self.device or ids.shape[0] != seg.rows:
+            raise ValueError(f"ids: expected int64 [{seg.rows}] on {self.device}")
+        ids = ids.contiguous()
+        if out is None:
+            out = torch.empty(seg.rows, self.hidden, dtype=torch.float32, device=self.device)
+        h = self._plan(seg.rows)
+        with torch.cuda.device(self.device):
+            check(lib().cer_bert_forward(h, ids.data_ptr(), seg.off.data_ptr(), seg.n_seg, seg.max_len, seg.rows,
+                                         out.data_ptr(), _capi.current_stream_ptr(self.device)), "cer_bert_forward")
+        return out
+
+    def embed(self, ids: torch.Tensor, seg: "Segments") -> torch.Tensor:
+        """The embedding kernel alone: hidden_states[0], [seg.rows, hidden]."""
+        ids = ids.contiguous()
+        out = torch.empty(seg.rows, self.hidden, dtype=torch.float32, device=self.device)
+        h = self._plan(seg.rows)
+        with torch.cuda.device(self.device):
+            check(lib().cer_bert_embed(h, ids.data_ptr(), seg.off.data_ptr(), seg.n_seg, seg.max_len, out.data_ptr(),
+                                       _capi.current_stream_ptr(self.device)), "cer_bert_embed")
+        return out
+
+    def _destroy(self):
+        h = getattr(self, "_h", None)
+        if h:
+            try:
+                lib().cer_bert_destroy(h)
+            except Exception:
+                pass
+            self._h = None
+
+    def __del__(self):
+        self._destroy()
+
+
+BERT_EPI = {"bias": 0, "gelu": 1, "residual": 2}
+
+
+def bert_linear(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor, epi: str = "bias",
+                res: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The BERT plan's tcgen05 TF32 linear kernel alone (cer_bert_linear): x [rows, in] W^T + b, then erf-GELU
+    (epi="gelu") or + res (epi="residual").  Contiguous fp32 CUDA tensors; in and out multiples of 64."""
+    rows, k = x.shape
+    n = w.shape[0]
+    if any(not t.is_contiguous() or t.dtype != torch.float32 for t in (x, w, b) + ((res,) if res is not None else ())):
+        raise ValueError("bert_linear: contiguous fp32 tensors expected")
+    y = torch.empty(rows, n, dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        check(lib().cer_bert_linear(x.data_ptr(), rows, k, w.data_ptr(), b.data_ptr(), n, BERT_EPI[epi], _ptr(res),
+                                    y.data_ptr(), _capi.current_stream_ptr()), "cer_bert_linear")
+    return y
+
+
+def sdpa_segments_heads(qkv: torch.Tensor, seg: "Segments", heads: int, head_dim: int = 64) -> torch.Tensor:
+    """Multi-head attention inside each segment in one launch (cer_sdpa_tc_seg_heads_forward): qkv [seg.rows, 3 * E]
+    with E = heads * head_dim laid out as q | k | v, head h in columns [h * head_dim, (h + 1) * head_dim) of each
+    -> [seg.rows, E]."""
+    e = heads * head_dim
+    if qkv.dim() != 2 or qkv.shape != (seg.rows, 3 * e) or not qkv.is_contiguous() or qkv.dtype != torch.float32:
+        raise ValueError(f"sdpa_segments_heads: qkv must be contiguous fp32 [{seg.rows}, {3 * e}]")
+    out = torch.empty(seg.rows, e, dtype=torch.float32, device=qkv.device)
+    with torch.cuda.device(qkv.device):
+        check(lib().cer_sdpa_tc_seg_heads_forward(qkv.data_ptr(), 3 * e, qkv.data_ptr() + 4 * e, 3 * e,
+                                                  qkv.data_ptr() + 8 * e, 3 * e, seg.off.data_ptr(), seg.n_seg, seg.max_len,
+                                                  head_dim, heads, out.data_ptr(), e, _capi.current_stream_ptr()),
+              "cer_sdpa_tc_seg_heads_forward")
+    return out
+
+
+def text_frames(rows: torch.Tensor, tok: torch.Tensor, mean: Optional[torch.Tensor] = None,
+                std: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """out[f] = (rows[tok[f]] - mean) / std (or rows[tok[f]]) on the device (cer_text_frames).  rows [n, D] fp32,
+    tok int32 [F] -> [F, D]."""
+    n_frames, dim = tok.shape[0], rows.shape[1]
+    if out is None:
+        out = torch.empty(n_frames, dim, dtype=torch.float32, device=rows.device)
+    with torch.cuda.device(rows.device):
+        check(lib().cer_text_frames(rows.data_ptr(), rows.stride(0), tok.data_ptr(), n_frames, dim, _ptr(mean), _ptr(std),
+                                    out.data_ptr(), out.stride(0), _capi.current_stream_ptr()), "cer_text_frames")
+    return out
+
+
 class PreprocEngine:
     """The reference's eval video transform on the device (cer_preproc_*): uint8 [N,H,W,3] stored
     crops -> fp32 [N,3,crop,crop] in [-1,1], bit-exact with PIL resize + crop + normalise."""

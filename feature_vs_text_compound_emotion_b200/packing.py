@@ -222,6 +222,33 @@ def pack_fusion(sd: Dict[str, torch.Tensor], modalities: Sequence[str], modal_di
     return out
 
 
+def pack_bert(sd: Dict[str, torch.Tensor], n_layers: int = None) -> dict:
+    """HF BertModel state_dict -> the cer_bert_weights layout (include/cer_b200.h): fp32, nn.Linear / nn.Embedding
+    layouts as they are, except that each layer's query / key / value weights and biases are stacked into one [3H, H]
+    projection (wqkv) and one [3H] bias (bqkv).  The pooler is not used."""
+    if n_layers is None:
+        n_layers = 0
+        while f"encoder.layer.{n_layers}.attention.self.query.weight" in sd:
+            n_layers += 1
+    f = lambda k: sd[k].detach().float().contiguous()
+    e = "embeddings."
+    out = {"word_emb": f(e + "word_embeddings.weight"), "pos_emb": f(e + "position_embeddings.weight"),
+           "type_emb": f(e + "token_type_embeddings.weight"), "emb_ln_g": f(e + "LayerNorm.weight"),
+           "emb_ln_b": f(e + "LayerNorm.bias"), "layers": []}
+    for i in range(n_layers):
+        p = f"encoder.layer.{i}."
+        a = p + "attention.self."
+        out["layers"].append({
+            "wqkv": torch.cat([f(a + n + ".weight") for n in ("query", "key", "value")]).contiguous(),
+            "bqkv": torch.cat([f(a + n + ".bias") for n in ("query", "key", "value")]).contiguous(),
+            "wo": f(p + "attention.output.dense.weight"), "bo": f(p + "attention.output.dense.bias"),
+            "ln1_g": f(p + "attention.output.LayerNorm.weight"), "ln1_b": f(p + "attention.output.LayerNorm.bias"),
+            "w1": f(p + "intermediate.dense.weight"), "b1": f(p + "intermediate.dense.bias"),
+            "w2": f(p + "output.dense.weight"), "b2": f(p + "output.dense.bias"),
+            "ln2_g": f(p + "output.LayerNorm.weight"), "ln2_b": f(p + "output.LayerNorm.bias")})
+    return out
+
+
 VGGISH_CFG = (64, "M", 128, "M", 256, 256, "M", 512, 512, "M")     # make_layers(), models/backbone.py:43-53
 
 

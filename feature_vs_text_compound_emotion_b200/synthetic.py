@@ -373,3 +373,32 @@ def jmt_state_dict(seed: int = 0, modalities: Sequence[str] = ("video", "vggish"
     _linear(sd, "fc1", 128, 128, g)
     _linear(sd, "fc2", output_dim, 128, g)
     return sd
+
+
+def bert_state_dict(seed: int = 0, std: float = 0.02, **config) -> "OrderedDict[str, torch.Tensor]":
+    """HF ``BertModel(BertConfig(**config)).state_dict()`` layout (bert-base-uncased sizes by default; the keyword
+    names are those of text.BertTextEncoder), in HF's key order.  Every weight, embedding and bias is N(0, std^2), every
+    LayerNorm weight 1 + N(0, std^2): std 0.02 is HF's initializer range, std 0.1 makes attention peaky."""
+    from .text import BertTextEncoder
+    with torch.device("meta"):
+        shapes = [(k, tuple(v.shape)) for k, v in BertTextEncoder(**config).state_dict().items()]
+    g = torch.Generator().manual_seed(seed + 15485863)
+    sd: "OrderedDict[str, torch.Tensor]" = OrderedDict()
+    for k, shape in shapes:
+        t = std * torch.randn(shape, generator=g)
+        sd[k] = 1.0 + t if k.endswith("LayerNorm.weight") else t
+    return sd
+
+
+def transcript_ids(lengths: Sequence[int], seed: int = 0, vocab: int = 30522) -> List[torch.Tensor]:
+    """Seeded int64 WordPiece ids, one transcript per length: [CLS] (101) first and [SEP] (102) last when there is
+    room, ids from [999, vocab) between them."""
+    g = torch.Generator().manual_seed(seed + 32452843)
+    out = []
+    for n in lengths:
+        t = torch.randint(999, vocab, (int(n),), generator=g, dtype=torch.int64)
+        t[0] = 101
+        if n > 1:
+            t[-1] = 102
+        out.append(t)
+    return out

@@ -505,12 +505,87 @@ int cer_sdpa_tc_forward(const float* q_dev, int32_t ldq, const float* k_dev, int
 int cer_sdpa_tc_seg_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev, int32_t ldv,
                             const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len, int32_t dim, float* out_dev,
                             int32_t ldo, void* stream);
+/* The segmented attention for every head of a multi-head projection in one launch: head h < heads reads columns
+ * [dim * h, dim * h + dim) of the q / k / v rows and writes the same columns of out (pitches >= dim * heads).  dim is
+ * 64, 1 <= heads <= 64, otherwise the conditions of cer_sdpa_tc_seg_forward.  Head h gives the same bits as
+ * cer_sdpa_tc_seg_forward on the column slices q_dev + dim * h, ... with the same pitches. */
+int cer_sdpa_tc_seg_heads_forward(const float* q_dev, int32_t ldq, const float* k_dev, int32_t ldk, const float* v_dev,
+                                  int32_t ldv, const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len, int32_t dim,
+                                  int32_t heads, float* out_dev, int32_t ldo, void* stream);
 /* y = tanh(y) in place: the output squashing of task == REGRESSION (models/model.py:523, :682, :1165). */
 /* a += b over n contiguous fp32 values (where the gradients of two branches meet) */
 int cer_add_inplace(float* a_dev, const float* b_dev, int64_t n, void* stream);
 int cer_tanh_inplace(float* y_dev, int64_t n, void* stream);
 int cer_add_layernorm(const float* x_dev, const float* res_dev, int64_t rows, int32_t dim, const float* gamma_dev,
                       const float* beta_dev, float eps, float* out_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * BERT text encoder (the `bert` feature stream).   Computes what HF BertModel(input_ids) computes in
+ * eval mode for unpadded transcripts (token_type_ids 0, positions 0..n-1) and returns per token the
+ * sum of the last four hidden states (the outputs of the last four layers), fp32.  The transcripts of
+ * one call are segments of one token buffer: segment s is rows [seg_off[s], seg_off[s+1]) and attends
+ * only over itself.  Every kernel is row-invariant: a token's row does not depend on the other
+ * segments of the call.  Linear layers run on tcgen05 kind::tf32 (fp32 operands, fp32 accumulate).
+ * Weights arrive pre-packed by packing.pack_bert, all fp32 device arrays in nn.Linear / nn.Embedding
+ * layouts (H = hidden, I = intermediate):
+ * ------------------------------------------------------------------------------------------ */
+typedef struct cer_bert_layer {
+  const float* wqkv;    /* [3H][H]  rows 0..H-1 attention.self.query.weight, H..2H-1 key.weight, 2H..3H-1 value.weight */
+  const float* bqkv;    /* [3H]     query.bias | key.bias | value.bias                                                */
+  const float* wo;      /* [H][H]   attention.output.dense.weight                                                     */
+  const float* bo;      /* [H]      attention.output.dense.bias                                                       */
+  const float* ln1_g;   /* [H]      attention.output.LayerNorm.weight                                                 */
+  const float* ln1_b;   /* [H]      attention.output.LayerNorm.bias                                                   */
+  const float* w1;      /* [I][H]   intermediate.dense.weight                                                         */
+  const float* b1;      /* [I]      intermediate.dense.bias                                                           */
+  const float* w2;      /* [H][I]   output.dense.weight                                                               */
+  const float* b2;      /* [H]      output.dense.bias                                                                 */
+  const float* ln2_g;   /* [H]      output.LayerNorm.weight                                                           */
+  const float* ln2_b;   /* [H]      output.LayerNorm.bias                                                             */
+} cer_bert_layer;
+
+typedef struct cer_bert_weights {
+  int32_t hidden;           /* H: 64 * n_heads (head_dim 64)                                               */
+  int32_t intermediate;     /* I: a multiple of 64; the activation is exact erf-GELU                       */
+  int32_t n_heads, n_layers;
+  int32_t vocab;            /* rows of word_emb; an id outside [0, vocab) gives a NaN row                  */
+  int32_t max_pos;          /* rows of pos_emb, <= 512: the longest segment                                */
+  int32_t type_vocab;       /* rows of type_emb; only row 0 is read (token_type_ids are 0)                 */
+  float ln_eps;             /* every LayerNorm's eps (1e-12 for bert-base-uncased)                          */
+  const float* word_emb;    /* [vocab][H]       embeddings.word_embeddings.weight                          */
+  const float* pos_emb;     /* [max_pos][H]     embeddings.position_embeddings.weight                      */
+  const float* type_emb;    /* [type_vocab][H]  embeddings.token_type_embeddings.weight                    */
+  const float* emb_ln_g;    /* [H]              embeddings.LayerNorm.weight                                */
+  const float* emb_ln_b;    /* [H]              embeddings.LayerNorm.bias                                  */
+  const cer_bert_layer* layers;  /* HOST array [n_layers]: encoder.layer.{i}; copied by cer_bert_create     */
+} cer_bert_weights;
+
+typedef struct cer_bert cer_bert;
+
+/* Workspace of a plan for up to max_tokens tokens per call: max_tokens * (7 H + I) floats. */
+size_t cer_bert_workspace_bytes(const cer_bert_weights* w, int64_t max_tokens);
+/* Checks the configuration (CER_ERR_INVALID otherwise) and encodes the TMA maps of the weights and the workspace. */
+int cer_bert_create(cer_bert** out, const cer_bert_weights* w, int64_t max_tokens, void* workspace_dev, size_t workspace_bytes);
+/* ids_dev: int64 [n_tokens] WordPiece ids, the segments end to end; seg_off_dev: int32 [n_seg + 1] on the device,
+ * ascending from 0 to n_tokens, no segment longer than max_len (the caller's contract, not checked on the device);
+ * max_len <= max_pos, n_tokens <= max_tokens, n_seg <= 65535.  out_dev: fp32 [n_tokens][H], 16 B aligned.  No
+ * allocation and no synchronisation: everything is enqueued on `stream`. */
+int cer_bert_forward(cer_bert* plan, const int64_t* ids_dev, const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len,
+                     int64_t n_tokens, float* out_dev, void* stream);
+void cer_bert_destroy(cer_bert* plan);
+/* The plan's embedding kernel alone (tests): out_dev fp32 [n_tokens][H] = hidden_states[0]. */
+int cer_bert_embed(const cer_bert* plan, const int64_t* ids_dev, const int32_t* seg_off_dev, int32_t n_seg, int32_t max_len,
+                   float* out_dev, void* stream);
+/* The plan's linear kernel alone: y [rows][out_dim] = epi(x [rows][in_dim] w^T + bias), w [out_dim][in_dim];
+ * epi 0: + bias, 1: + bias then erf-GELU, 2: + bias + res [rows][out_dim].  in_dim and out_dim multiples of 64,
+ * every pointer 16 B aligned, all rows contiguous. */
+int cer_bert_linear(const float* x_dev, int64_t rows, int32_t in_dim, const float* w_dev, const float* bias_dev,
+                    int32_t out_dim, int32_t epi, const float* res_dev, float* y_dev, void* stream);
+/* Token rows -> frame rows: out[f] = (rows[tok[f]] - mean) / std per feature (the dataset's z-score), or rows[tok[f]]
+ * when mean_dev and std_dev are both NULL.  rows_dev fp32 [*][ldr], tok_dev int32 [n_frames] row indices, out_dev
+ * fp32 [n_frames][ldo]; dim and pitches multiples of 4, pointers 16 B aligned. */
+int cer_text_frames(const float* rows_dev, int32_t ldr, const int32_t* tok_dev, int64_t n_frames, int32_t dim,
+                    const float* mean_dev, const float* std_dev, float* out_dev, int32_t ldo, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Window stitching.   Replaces the sum / overlap-count / divide of
