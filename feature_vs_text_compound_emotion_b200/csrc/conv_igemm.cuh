@@ -92,6 +92,21 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&h);
 }
 
+// One 256-bit global store (STG.256, sm_100): `p` must be 32-byte aligned.  The epilogue stores one pixel row per
+// lane, so a 128-bit store covers only half of a 32 B sector in each of 32 rows; a 256-bit store writes whole
+// sectors with half the instructions and no lane exchange (tools/epilogue_probe.cu, DESIGN.md section 5.12).
+__device__ __forceinline__ void st_global_256(void* p, uint4 a, uint4 b) {
+  asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
+               ::"l"(p), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
+               : "memory");
+}
+__device__ __forceinline__ uint4 pack_bf16x8(const float* f) {
+  return make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
+}
+__device__ __forceinline__ uint4 f32x4_bits(const float* f) {
+  return make_uint4(__float_as_uint(f[0]), __float_as_uint(f[1]), __float_as_uint(f[2]), __float_as_uint(f[3]));
+}
+
 // One output tile of the fused epilogue, for one epilogue thread (warp 0-7):
 //   + bias[class(pixel)][co] -> PReLU(alpha[co]) -> + residual[m][co] -> bf16 | fp32.
 // `tmem_acc` is the accumulator's TMEM base column; `tfull` the barrier that says it is complete.
@@ -248,27 +263,26 @@ __device__ __forceinline__ void conv_epilogue_core(const ConvKernelParams& p, co
         h[j] = *reinterpret_cast<uint32_t*>(&mx);
       }
       if (pool_store) {
-        uint4* op = reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + pool_off + c0);
+        __nv_bfloat16* op = static_cast<__nv_bfloat16*>(p.out) + pool_off + c0;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) op[j] = make_uint4(h[4 * j], h[4 * j + 1], h[4 * j + 2], h[4 * j + 3]);
+        for (int j = 0; j < 2; ++j)
+          st_global_256(op + 16 * j, make_uint4(h[8 * j], h[8 * j + 1], h[8 * j + 2], h[8 * j + 3]),
+                        make_uint4(h[8 * j + 4], h[8 * j + 5], h[8 * j + 6], h[8 * j + 7]));
       }
     } else if (valid) {
       if (p.out_fp32) {
-        float4* op = reinterpret_cast<float4*>(static_cast<float*>(p.out) + out_off + c0);
+        float* op = static_cast<float*>(p.out) + out_off + c0;
 #pragma unroll
-        for (int j = 0; j < 8; ++j) op[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
+        for (int j = 0; j < 4; ++j) st_global_256(op + 8 * j, f32x4_bits(f + 8 * j), f32x4_bits(f + 8 * j + 4));
       } else {
-        uint4* op = reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + out_off + c0);
+        __nv_bfloat16* op = static_cast<__nv_bfloat16*>(p.out) + out_off + c0;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          op[j] = make_uint4(pack_bf16x2(f[8 * j + 0], f[8 * j + 1]), pack_bf16x2(f[8 * j + 2], f[8 * j + 3]),
-                             pack_bf16x2(f[8 * j + 4], f[8 * j + 5]), pack_bf16x2(f[8 * j + 6], f[8 * j + 7]));
-        }
+        for (int j = 0; j < 2; ++j) st_global_256(op + 16 * j, pack_bf16x8(f + 16 * j), pack_bf16x8(f + 16 * j + 8));
       }
     } else if (zero_store) {                 // pad position of a padded-raster output (bf16): must read as the conv's zero padding
-      uint4* op = reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + out_off + c0);
+      __nv_bfloat16* op = static_cast<__nv_bfloat16*>(p.out) + out_off + c0;
 #pragma unroll
-      for (int j = 0; j < 4; ++j) op[j] = make_uint4(0u, 0u, 0u, 0u);
+      for (int j = 0; j < 2; ++j) st_global_256(op + 16 * j, make_uint4(0u, 0u, 0u, 0u), make_uint4(0u, 0u, 0u, 0u));
     }
   }
 }

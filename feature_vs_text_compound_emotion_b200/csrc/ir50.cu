@@ -1118,6 +1118,8 @@ extern "C" int cer_conv_forward(const void* src_nhwc, int32_t n_frames, int32_t 
   if (!src_nhwc || !weight || !bias || !dst || n_frames <= 0 || n_alloc < n_frames || (ksize != 1 && ksize != 3) ||
       (bias_classes != 1 && bias_classes != 9))
     return set_error(CER_ERR_INVALID, "cer_conv_forward: bad argument");
+  if (reinterpret_cast<uintptr_t>(dst) % 32)          // the epilogue stores 32-byte vectors
+    return set_error(CER_ERR_INVALID, "cer_conv_forward: dst must be 32B aligned");
   int rc = cer_check_device();
   if (rc) return rc;
   rc = load_driver_entry_points();

@@ -284,8 +284,9 @@ static int run_pass(cer_vggish* p, const float* x, int n, int last_step, float* 
 extern "C" int cer_vggish_forward(cer_vggish* p, const float* x, int64_t n_patches, float* emb_out, void* stream) {
   if (!p || n_patches < 0 || (n_patches > 0 && (!x || !emb_out)))
     return set_error(CER_ERR_INVALID, "cer_vggish_forward: bad argument");
-  if (reinterpret_cast<uintptr_t>(x) % 4 || reinterpret_cast<uintptr_t>(emb_out) % 16)
-    return set_error(CER_ERR_INVALID, "cer_vggish_forward: emb_out must be 16B aligned");
+  // the last FC's epilogue stores 32-byte vectors straight into emb_out
+  if (reinterpret_cast<uintptr_t>(x) % 4 || reinterpret_cast<uintptr_t>(emb_out) % 32)
+    return set_error(CER_ERR_INVALID, "cer_vggish_forward: emb_out must be 32B aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int H = p->w.in_h, W = p->w.in_w;
   for (int64_t f0 = 0; f0 < n_patches; f0 += p->cap) {
@@ -306,8 +307,8 @@ extern "C" int64_t cer_vggish_debug_activation(cer_vggish* p, const float* x, in
                                                void* stream) {
   if (!p || !x || !dst_dev || n_patches <= 0 || n_patches > p->cap || step < -1 || step >= (int)p->steps.size())
     return set_error(CER_ERR_INVALID, "cer_vggish_debug_activation: bad argument");
-  if (reinterpret_cast<uintptr_t>(x) % 4 || reinterpret_cast<uintptr_t>(dst_dev) % 16)
-    return set_error(CER_ERR_INVALID, "cer_vggish_debug_activation: dst must be 16B aligned");
+  if (reinterpret_cast<uintptr_t>(x) % 4 || reinterpret_cast<uintptr_t>(dst_dev) % 32)   // the last FC stores into it
+    return set_error(CER_ERR_INVALID, "cer_vggish_debug_activation: dst must be 32B aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const bool last = step + 1 == (int)p->steps.size();
   int rc = run_pass(p, x, (int)n_patches, step, last ? static_cast<float*>(dst_dev) : nullptr, st);

@@ -126,7 +126,7 @@ void cer_ir50_destroy(cer_ir50* plan);
  * weight: bf16 [cout][ksize*ksize*cin] with K = (r,s,ci); bias: fp32 [bias_classes][cout]
  * (bias_classes 9 = border-class table, stride-1 pad-1 3x3 only); alpha: PReLU slopes or NULL;
  * res: bf16 [M][cout] residual or NULL; dst: bf16 (or fp32 if out_fp32) [M][cout],
- * M = n_frames*hout*wout.  cin, cout multiples of 64. */
+ * M = n_frames*hout*wout, 32 B aligned.  cin, cout multiples of 64. */
 int cer_conv_forward(const void* src_nhwc_dev, int32_t n_frames, int32_t n_alloc, int32_t h, int32_t w, int32_t cin,
                      const void* weight_dev, int32_t cout, int32_t ksize, int32_t stride, int32_t pad,
                      const float* bias_dev, int32_t bias_classes, const float* alpha_dev, const void* res_dev,
@@ -169,7 +169,7 @@ typedef struct cer_vggish cer_vggish;
 size_t cer_vggish_workspace_bytes(const cer_vggish_weights* w, int64_t patches_per_pass);
 int cer_vggish_create(cer_vggish** out, const cer_vggish_weights* w, int64_t patches_per_pass, void* workspace_dev,
                       size_t workspace_bytes);
-/* x_dev: fp32 [n_patches][in_h][in_w] log-mel examples; emb_out_dev: fp32 [n_patches][128]. */
+/* x_dev: fp32 [n_patches][in_h][in_w] log-mel examples; emb_out_dev: fp32 [n_patches][128], 32 B aligned. */
 int cer_vggish_forward(cer_vggish* plan, const float* x_dev, int64_t n_patches, float* emb_out_dev, void* stream);
 int64_t cer_vggish_launches(const cer_vggish* plan, int64_t n_patches);
 void cer_vggish_destroy(cer_vggish* plan);
@@ -185,7 +185,7 @@ typedef struct cer_vggish_step {
 /* Copies the first min(max_steps, n) step descriptors to `out` and returns n, the number of steps. */
 int32_t cer_vggish_steps(const cer_vggish* plan, cer_vggish_step* out, int32_t max_steps);
 /* Debug/inspection: one pass over `n_patches` (<= patches_per_pass) patches -- the stem, then steps 0 .. step --
- * and a copy of that step's output to dst_dev (16 B aligned).  step = -1 is the stem's pooled bf16
+ * and a copy of that step's output to dst_dev (32 B aligned).  step = -1 is the stem's pooled bf16
  * [n][in_h/2][in_w/2][c1]; the last step (the fp32 FC) writes dst_dev directly.  At n_patches = patches_per_pass
  * the launches are exactly those of that cer_vggish_forward pass.  Returns the element count or a negative status. */
 int64_t cer_vggish_debug_activation(cer_vggish* plan, const float* x_dev, int64_t n_patches, int32_t step, void* dst_dev,
