@@ -215,6 +215,9 @@ SIGNATURES = {
     "cer_bert_embed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "cer_bert_linear": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                   C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cer_face_fit": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_double), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cer_face_warp": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
+                                C.c_void_p, C.c_void_p]),
     "cer_text_frames": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_int32, C.c_void_p]),
     "cer_add_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float,

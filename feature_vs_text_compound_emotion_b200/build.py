@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libcer_b200.so")
 STAMP = os.path.join(HERE, ".libcer_b200.stamp")
-SOURCES = ["common.cu", "ir50.cu", "vggish.cu", "tcn.cu", "tcn_tc.cu", "fusion.cu", "train.cu", "preproc.cu", "logmel.cu", "heads.cu", "se.cu", "stream.cu", "can_head.cu", "bert.cu"]
+SOURCES = ["common.cu", "ir50.cu", "vggish.cu", "tcn.cu", "tcn_tc.cu", "fusion.cu", "train.cu", "preproc.cu", "logmel.cu", "heads.cu", "se.cu", "stream.cu", "can_head.cu", "bert.cu", "align.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-O2"]
 

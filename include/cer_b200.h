@@ -588,6 +588,29 @@ int cer_text_frames(const float* rows_dev, int32_t ldr, const int32_t* tok_dev, 
                     const float* mean_dev, const float* std_dev, float* out_dev, int32_t ldo, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Five-point face alignment (faces.align): full uint8 frames + detector landmarks -> the aligned
+ * uint8 face crops the `video` stream takes.  Restates face.evoLVe's warp_and_crop_face with
+ * reflective=True: get_similarity_transform_for_cv2 then cv2.warpAffine(img, M, (crop, crop))
+ * (INTER_LINEAR, BORDER_CONSTANT 0), bit-exact with OpenCV's fixed-point arithmetic for the same M.
+ * Not in the reference's inference path: its offline pipeline stores the crops (SURVEY §2.1 row 19).
+ * ------------------------------------------------------------------------------------------ */
+/* landmarks_dev: fp32 [n][5][2] (x, y) pixel coordinates, in the order left eye, right eye, nose,
+ * left mouth corner, right mouth corner; reference_host: HOST fp64 [5][2], the same points in the
+ * crop (CER_ERR_INVALID if not finite or all coincident).  Per face, in fp64: the least-squares
+ * similarity onto the reference and onto the mirrored reference composed with the reflection, the
+ * one with the smaller residual norm kept (the non-reflective one on a tie).  fwd_dev: fp64 [n][2][3],
+ * the source -> crop matrix cv2 is given; inv_dev: fp64 [n][2][3], its inverse exactly as
+ * cv::warpAffine computes it.  Landmarks whose five points coincide give a non-finite matrix. */
+int cer_face_fit(const float* landmarks_dev, int64_t n, const double* reference_host, double* fwd_dev, double* inv_dev,
+                 void* stream);
+/* frames_dev: uint8 [n_frames][h][w][3], h and w <= 32767; frame_index_dev: int64 [n], face i is cut
+ * from frame frame_index[i] (an index outside [0, n_frames) gives a zero crop, nothing is read);
+ * inv_dev: fp64 [n][2][3] crop -> source matrices (cer_face_fit's inv_dev); out_dev: uint8
+ * [n][crop][crop][3], 1 <= crop <= 1024, any alignment.  Channels are carried as given. */
+int cer_face_warp(const uint8_t* frames_dev, int64_t n_frames, int32_t h, int32_t w, const int64_t* frame_index_dev,
+                  const double* inv_dev, int64_t n, int32_t crop, uint8_t* out_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Window stitching.   Replaces the sum / overlap-count / divide of
  * Trainer.inference_forward_windows (trainer.py:864-890) on device.
  * win_logits: fp32 [n_windows][win_len][n_out]; win_start: int32 [n_windows] first frame of each
